@@ -1,6 +1,6 @@
 """bench.py -- env-steps/s of the Ofighters hot path on B200 (contract: see README / DESIGN.md section 6).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 A *step* is one lockstep frame of every arena in the batch: scripted-bot actions -> fused arena
 step (K1) -> observation raster (K2) [-> policy forward for the policy workloads], with the
@@ -23,7 +23,11 @@ Timing: CUDA events on the launching stream around every step, L2 flushed (256 M
 between steps when the working set is smaller than L2, barrier + synchronize on both sides of the
 timed region, max over ranks.  `--impl reference` times the CPU restatement of the reference
 (oracle/step_c.c, OpenMP over all host cores) on the same workload; the reference itself is pure
-Python under /root/reference and cannot travel to the GPU box.
+Python and is not part of this repository.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step computed (observation heads, arena state,
+the policy ships' played actions, bit maps) as DIR/<name>.npy in float32 / float64, for a fixed seeded sample of arenas
+(rank 0's when several GPUs run), so that two builds can be compared output for output on identical inputs.
 """
 import argparse
 import json
@@ -252,6 +256,47 @@ def wants_learning(args, name, wl):
     return bool(wl["policy"]) and (args.learn == "on" or (args.learn == "auto" and name == "sharded1m"))
 
 
+# --dump-outputs: 512 sampled arenas, the bit maps of the first 128 of them.  At the largest laser list of any workload
+# (stress: 2048 slots x 32 ships) that is 54 MB, under the 64 MB the dump may take.
+DUMP_ARENAS, DUMP_MAP_ARENAS, DUMP_MAX_BYTES = 512, 128, 64 * 2 ** 20
+
+
+def dump_outputs(out_dir, bg, maps, played):
+    """Writes the outputs of the last step as out_dir/<name>.npy: `arena_ids` (global ids of a sample of DUMP_ARENAS arenas
+    drawn with SEED), for those arenas the observation heads `obs_vec`, every field of `bg.state()` (laser slots past an
+    arena's live count are zeroed, the laser columns cut at the sample's largest live count), the batch's action buffer
+    `actions` (the rows the policy wrote; scripted bots draw their actions inside the frame kernel and leave their rows
+    zero), the policy ships' played `policy_iaction` / `policy_xy` (policy workloads), the bit maps `maps` (u32 words, first
+    DUMP_MAP_ARENAS sampled arenas); and the batch's episode statistics `stats`.  Integers become float64 (float32 when
+    16 bits or fewer), so every value is exact."""
+    import numpy as np
+    import torch
+    N = bg.n_arenas
+    ids = np.sort(np.random.Generator(np.random.PCG64(SEED)).choice(N, size=min(N, DUMP_ARENAS), replace=False))
+    sel = torch.from_numpy(ids).to(bg.device)
+    pick = lambda t: t.index_select(0, sel).cpu().numpy()
+    st = {k: pick(v) for k, v in bg.state().items()}
+    width = max(1, int(st["n_lasers"].max()))
+    live = np.arange(width)[None, :] < st["n_lasers"][:, None]
+    for k in st:
+        if k.startswith("laser_"):
+            st[k] = np.where(live, st[k][:, :width], 0).astype(st[k].dtype)
+    out = {"arena_ids": ids + bg.arena0, "obs_vec": pick(bg.obs_vec), **st, "actions": pick(bg.actions),
+           "maps": maps.index_select(0, sel[:DUMP_MAP_ARENAS]).cpu().numpy().view(np.uint32), "stats": bg.stats.cpu().numpy()}
+    if played is not None:
+        iact, xy = played
+        out["policy_iaction"] = pick(iact.reshape(N, -1))
+        out["policy_xy"] = pick(xy.reshape(N, -1, 2))
+    for k, v in out.items():
+        out[k] = v.astype(np.float32 if v.dtype == np.float32 or (v.dtype.kind in "iub" and v.dtype.itemsize <= 2) else np.float64)
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_MAX_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 # ----------------------------------------------------------------------------- GPU arm
 def gpu_arm(args, name, wl):
     import torch
@@ -307,6 +352,7 @@ def gpu_arm(args, name, wl):
     coll = {"all_reduce": 0, "broadcast": 0, "restarts": 0, "replays": 0}
     frame_no = [0]                                        # frames since construction (identical on every rank)
     weights_dirty = [False]
+    played = [None]                                       # (iaction, xy) the policy ships played in the last step
 
     def n_launched():
         return bg.launch_count + (policy.launch_count if policy is not None else 0) + \
@@ -353,17 +399,18 @@ def gpu_arm(args, name, wl):
                 sched = learner.trainer.epsilon if learner is not None else schedule
                 collecting = frame_no[0] + 1 < 20
                 if learner is not None:
-                    _, _, replayed = learner.act(bg, maps)     # choose (collecting / eps-greedy), write rows, remember / replay
+                    iact, xy, replayed = learner.act(bg, maps)     # choose (collecting / eps-greedy), write rows, remember / replay
+                    played[0] = (iact, xy)
                     coll["replays"] += 1 if replayed else 0
                     weights_dirty[0] |= replayed
                 else:                                          # the other ranks follow the shared schedule between broadcasts
-                    policy.act(bg, maps, epsilon=sched, collecting=collecting)
+                    played[0] = policy.act(bg, maps, epsilon=sched, collecting=collecting)
                     if not collecting:
                         sched.next()
                 if (frame_no[0] + 1) % 50 == 0:
                     sync_actor_weights()
             else:
-                policy.act(bg, maps)               # forward on the current maps -> the policy ship's ("external") action row
+                played[0] = policy.act(bg, maps)   # forward on the current maps -> the policy ship's ("external") action row
         bg.frame(maps=maps)                        # scripted bots + step + observation maps: one fused launch (ofb_frame_bots)
         frame_no[0] += 1
         launches[0] += n_launched() - n0
@@ -419,6 +466,8 @@ def gpu_arm(args, name, wl):
     bg.check_overflow()
     value = N * world * steps / (total_ms * 1e-3)
     episode_stats = sharding.stats_dict(bg.stats)
+    if args.dump_outputs and rank == 0:                   # before the measurements below restart and step the batch
+        dump_outputs(args.dump_outputs, bg, maps, played[0])
 
     # ---- dominant kernel alone, same events + flush
     roof = kernel_roofline(bg, maps, flush_buf, wl, dev, policy)
@@ -935,12 +984,19 @@ def main():
                          "frames), weights broadcast, loss in the per-episode reduction (auto = on for sharded1m)")
     ap.add_argument("--flush", default="write+read", choices=["write", "write+read"],
                     help="L2 flush between timed steps when the working set is L2-sized")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "a seeded sample of arenas, at most 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     name, wl = resolve_workload(args)
     if args.impl == "reference":
         if int(os.environ.get("RANK", "0")) != 0:
             return
-        steps = min(args.steps, 400)
+        steps = args.steps
         v, ms, cores, sample, fwd = cpu_arm_with_policy(wl, steps, min(max(args.warmup, 3), 10))
         emit(({
             "impl": "reference", "metric": METRIC % (" + policy fwd" if wl["policy"] else ""),
@@ -951,7 +1007,7 @@ def main():
             "config": workload_config(name, wl, max(1, args.gpus), wants_learning(args, name, wl)),
             "reference_class": "cpu-port",
             "note": "CPU restatement of the reference's algorithm on a bounded sample of the workload (the reference is pure "
-                    "Python under /root/reference and is absent on the GPU box)" +
+                    "Python and is not part of this repository)" +
                     ("; policy forward = torch-fp32 restatement of the Keras model; learning is not part of the CPU sample"
                      if wl["policy"] else ""),
             "cpu_baseline": {"value": v, "unit": "env-steps/s", "cores": cores, "kind": "port", "sample": sample},

@@ -1,13 +1,15 @@
-"""Loader for the UNMODIFIED reference (build-container only) -- test infrastructure.
+"""Loader for the UNMODIFIED reference -- test infrastructure.
 
-Imports ``ofighters.lib.battleground`` & friends from /root/reference after
+Imports ``ofighters.lib.battleground`` & friends from the original Ofighters
+source tree named by the environment variable OFB_REFERENCE_ROOT after
 injecting ``sys.modules`` shims for the third-party packages that are absent
 here (matplotlib, keras, tensorflow, tkinter, pandas = mocks; skimage.draw.disk
 = the restatement in oracle/disk.py).  Nothing of the reference is copied or
 edited; see SURVEY.md Appendix C.
 
-/root/reference does not exist on the GPU box: only ``oracle/gen_golden.py``
-and the container-only tests (skipped when the path is missing) use this.
+The reference is not part of this repository: only ``oracle/gen_golden.py``
+and the tests marked ``reference`` (skipped when OFB_REFERENCE_ROOT is unset)
+use this.
 """
 import contextlib
 import io
@@ -16,7 +18,7 @@ import sys
 import types
 from unittest.mock import MagicMock
 
-REFERENCE_ROOT = os.environ.get("OFB_REFERENCE_ROOT", "/root/reference")
+REFERENCE_ROOT = os.environ.get("OFB_REFERENCE_ROOT", "")
 
 _MOCKED = [
     "matplotlib", "matplotlib.pyplot", "matplotlib.cm", "matplotlib.figure",
@@ -30,7 +32,7 @@ _loaded = None
 
 
 def available():
-    return os.path.isdir(os.path.join(REFERENCE_ROOT, "ofighters", "lib"))
+    return bool(REFERENCE_ROOT) and os.path.isdir(os.path.join(REFERENCE_ROOT, "ofighters", "lib"))
 
 
 def load():
@@ -39,7 +41,7 @@ def load():
     if _loaded is not None:
         return _loaded
     if not available():
-        raise RuntimeError("reference tree not present at %s" % REFERENCE_ROOT)
+        raise RuntimeError("reference tree not present: set OFB_REFERENCE_ROOT to the original Ofighters source tree")
     from oracle.disk import disk
     for m in _MOCKED:
         if m not in sys.modules:

@@ -10,13 +10,13 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
+    config.addinivalue_line("markers", "reference: needs the original Ofighters source tree (OFB_REFERENCE_ROOT)")
 
 
 def pytest_collection_modifyitems(config, items):
     from oracle import ref_shim
     if not ref_shim.available():
-        skip = pytest.mark.skip(reason="/root/reference not present")
+        skip = pytest.mark.skip(reason="OFB_REFERENCE_ROOT does not name the original Ofighters source tree")
         for it in items:
             if "reference" in it.keywords:
                 it.add_marker(skip)

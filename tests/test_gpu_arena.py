@@ -383,3 +383,57 @@ def test_host_wait_covers_the_action_copy_without_observation_buffer():
         buf.fill_(-1)                                    # scribble over the tape: the frame must already have its copy
     want, got = src.state(("ship_x", "ship_y", "ship_score", "n_lasers")), rep.state(("ship_x", "ship_y", "ship_score", "n_lasers"))
     assert all(torch.equal(want[k], got[k]) for k in want)
+
+
+def _bench_dump(out_dir, workload, steps):
+    """Runs bench.py --dump-outputs (3 warm-up steps, without the extra measurements) and loads what it wrote."""
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", workload, "--steps", str(steps), "--warmup", "3",
+                    "--dump-outputs", str(out_dir)], check=True, timeout=900, stdout=subprocess.DEVNULL,
+                   env=dict(os.environ, OFB_BENCH_NO_EXTRA="1"))
+    d = {f[:-4]: np.load(os.path.join(str(out_dir), f)) for f in os.listdir(str(out_dir))}
+    assert all(v.dtype in (np.float32, np.float64) for v in d.values())
+    assert sum(v.nbytes for v in d.values()) <= 64 * 2 ** 20
+    return d
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs on arena4096 with 4 timed steps: the pre-roll puts the episode restart inside them, so the last
+    step is frame 2 of episode 1 (202 frames in all).  The sampled arenas' state, observation heads and maps equal the C
+    restatement's after the same 202 seeded frames, and every file is float32 / float64, 64 MB at most in all."""
+    from oracle.step_c import ArenasC
+    d = _bench_dump(tmp_path, "arena4096", 4)
+    ids = d["arena_ids"].astype(np.int64)
+    assert len(ids) == 512 and np.all(np.diff(ids) > 0) and ids[-1] < 4096
+    assert np.all(d["time"] == 2)
+    N, S, seed = 4096, 7, 0x0F16
+    c = ArenasC(ArenasC(np.zeros((N, S, 2), np.int32)).random_spawn(seed, 0))
+    for it in range(202):
+        if it == 200:
+            c.reset(c.random_spawn(seed, 1))
+        c.step(c.bot_actions("random", seed, it))
+    for k in ("time", "ship_x", "ship_y", "ship_px", "ship_py", "ship_alive", "ship_hull", "ship_score", "n_lasers", "kills", "deaths"):
+        assert np.array_equal(d[k], c.arr[k][ids]), k
+    n = int(d["n_lasers"].max())
+    live = np.arange(n)[None, :] < d["n_lasers"][:, None]
+    assert np.array_equal(d["laser_x"][:, :n], np.where(live, c.arr["laser_x"][ids, :n], 0))
+    assert np.array_equal(d["obs_vec"], c.obs_vec()[ids])
+    assert np.array_equal(d["maps"], c.raster_bits()[ids[:128]])
+    assert np.array_equal(d["stats"], c.arr["stats"])
+    assert d["actions"].shape == (512, S, 4) and not d["actions"].any()     # scripted bots draw their actions in the frame kernel
+    assert "policy_iaction" not in d
+
+
+def test_bench_dump_outputs_carry_the_played_policy_actions(tmp_path):
+    """bench.py --dump-outputs on policy7 (all 7 ships driven by the policy forward): policy_iaction / policy_xy hold one
+    played action per sampled arena and ship, and the dumped action rows are exactly those actions, [iaction == 0 (shoot),
+    iaction == 1 (thrust), x, y] (QlearnIA.play's action vector)."""
+    d = _bench_dump(tmp_path, "policy7", 2)
+    ia, xy, act = d["policy_iaction"], d["policy_xy"], d["actions"]
+    assert ia.shape == (512, 7) and xy.shape == (512, 7, 2) and act.shape == (512, 7, 4)
+    assert np.isin(ia, (0, 1)).all() and ((xy >= 0) & (xy < 400)).all()
+    assert np.array_equal(act[..., 0], ia == 0) and np.array_equal(act[..., 1], ia == 1) and np.array_equal(act[..., 2:], xy)
+    assert xy.any()                                      # rows were really written (a zero buffer would agree with zeros)

@@ -82,9 +82,23 @@ def test_golden_files_cover_quirks():
     assert s["n_lasers"].max() > 200 and s["ship_alive"][0, -1].sum() == 0
 
 
-# ---- live reference (build container only) ------------------------------------------------
+LIVE_CASES = [("random", 7, 120, 11), ("stress", 16, 40, 12), ("lattice", 9, 80, 13)]
+
+
+@pytest.mark.parametrize("kind,S,T,seed", LIVE_CASES)
+def test_py_and_c_restatements_agree_on_the_live_reference_scenes(kind, S, T, seed):
+    """The scenes of the live-reference test below, which include ship counts no stored trace has (16-ship stress,
+    9-ship lattice): the two restatements, each pinned to the reference by the stored traces, agree bit for bit on every
+    frame's observation heads, ship and laser state, events and maps."""
+    spawn, actions = traces.make_tapes(seed, 2, T, S, kind)
+    tr = traces.run_py(spawn, actions, map_frames=(0, 7))
+    tr.update(spawn=spawn.astype(np.int32), actions=actions.astype(np.int16))
+    assert tu.run_engine(tu.COracleEngine, tr) == []
+
+
+# ---- live reference (needs the original source tree, OFB_REFERENCE_ROOT) --------------------
 @pytest.mark.reference
-@pytest.mark.parametrize("kind,S,T,seed", [("random", 7, 120, 11), ("stress", 16, 40, 12), ("lattice", 9, 80, 13)])
+@pytest.mark.parametrize("kind,S,T,seed", LIVE_CASES)
 def test_py_restatement_matches_live_reference(kind, S, T, seed):
     spawn, actions = traces.make_tapes(seed, 2, T, S, kind)
     ref = traces.run_reference(spawn, actions, vector_ships=(0,), map_frames=(0, 7))

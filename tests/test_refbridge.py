@@ -4,6 +4,45 @@ import numpy as np
 import pytest
 
 from oracle import ref_shim
+from tests import trace_util as tu
+
+
+@pytest.mark.parametrize("name", ["default_s7_seed0", "default_s7_seed1"])
+def test_observation_fields_equal_the_reference_traces(name):
+    """At every frame of a stored trace of the reference that keeps its full maps, the bridge's Observation built from the
+    batch formats (the C restatement's observation heads, bit maps and alive flags) equals what the reference recorded:
+    the 8-value head its bots were shown, its ship_map / laser_map arrays, the ships' positions, pointings and rewards,
+    and done = not playable.  The vector is the head followed by both maps, row by row."""
+    from ofighters_b200.refbridge import observation_fields
+    from oracle.step_c import ArenasC
+    gold = tu.load_golden(tu.GOLDEN_DIR + "/" + name + ".npz")
+    spawn, actions = gold["spawn"], gold["actions"]
+    E, T, S, _ = actions.shape
+    frames = list(gold["map_frames"])
+    c = ArenasC(spawn[:1])
+    n_checked = n_done = 0
+    for e in range(E):
+        if e > 0:
+            c.reset(spawn[e:e + 1])
+        for t in range(T):
+            c.step(actions[e, t][None])
+            if t not in frames or t + 1 == T:             # the head of frame t + 1 shows the state after frame t
+                continue
+            heads, bits, alive = c.obs_vec()[0], c.raster_bits()[0], c.arr["ship_alive"][0]
+            ref_maps = np.unpackbits(gold["maps"][e, frames.index(t)], axis=-1, bitorder="little").reshape(2, 400, 400)
+            for i in range(S):
+                got = observation_fields(heads[i], bits[0], bits[1], alive[i])
+                assert got.vector.shape == (320008, 1) and got.vector.dtype == np.float64
+                assert np.array_equal(got.vector[:8, 0].astype(np.float32), gold["obs_vec"][e, t + 1, i])
+                assert np.array_equal(got.vector[8:, 0], ref_maps.reshape(-1))
+                assert np.array_equal(got.ship_map, ref_maps[0]) and np.array_equal(got.laser_map, ref_maps[1])
+                assert (got.pos.x, got.pos.y) == (gold["ship_x"][e, t, i], gold["ship_y"][e, t, i])
+                assert (got.pointing.x, got.pointing.y) == (gold["ship_px"][e, t, i], gold["ship_py"][e, t, i])
+                assert (got.dim.x, got.dim.y) == (400, 400) and got.can_shoot == gold["obs_vec"][e, t + 1, i, 1]
+                assert got.reward == gold["ship_reward"][e, t, i] and got.done == (not gold["ship_alive"][e, t, i])
+                n_checked += 1
+                n_done += got.done
+    assert n_checked >= 6 * S and 0 < n_done < n_checked      # frames with both playable ships and wreckage
 
 
 @pytest.mark.reference
