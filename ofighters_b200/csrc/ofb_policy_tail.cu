@@ -40,7 +40,8 @@ __device__ __forceinline__ void tc_ld16(uint32_t taddr, uint32_t *r) {
 }
 __device__ __forceinline__ void named_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-// order-preserving map float -> int (for an atomic maximum on values of either sign)
+// order-preserving map float -> int (for an atomic maximum on values of either sign).  It orders -0.0 below +0.0; the keys are
+// taken on v + bias4 with a bias4 that is never -0.0 (pol_tz_tail), and x + (+0.0) is never -0.0.
 __device__ __forceinline__ int okey(float v) { const int b = __float_as_int(v); return b >= 0 ? b : b ^ 0x7fffffff; }
 
 // ---- CTA pairs (cta_group::2): M = 256 MMAs over two CTAs of a cluster, each supplying its own 128 A rows and HALF of the B columns
@@ -510,7 +511,9 @@ k_tz_tail(const TlArgs a, const int n_ships) {
             for (int h = 16; h > 0; h >>= 1)
 #pragma unroll
                 for (int n = 0; n < h; n++) mx[n] = fmaxf(mx[n], mx[n + h]);
-            const float M = mx[0];
+            // the map is v + bias4: fp32 addition is monotone but not injective, so the maximum and its first index are taken
+            // on the biased values (two pixels with v1 > v2 can both round to the same v + bias4)
+            const float M = mx[0] + a.bias4;
             const int key = okey(M);
             // only a value that reaches the ship's best so far can be its maximum: the index scan is rare
             const bool cand = valid && key >= *reinterpret_cast<volatile int *>(vship);
@@ -520,7 +523,7 @@ k_tz_tail(const TlArgs a, const int n_ships) {
 #pragma unroll
                     for (int n = 0; n < 64; n++) {
                         const int cn = ((n >> 5) * 2 + ((n >> 1) & 1)) * 400 + 2 * ((n & 31) >> 2) + (n & 1);
-                        if (v[n] == M) cmin = min(cmin, cn);
+                        if (v[n] + a.bias4 == M) cmin = min(cmin, cn);
                     }
                     const int idx = 1600 * i + 16 * xb + cmin;
                     if (key > best_key || (key == best_key && idx < best_idx)) { best_key = key; best_idx = idx; }
@@ -573,7 +576,7 @@ int pol_tz_tail(const ofb_policy *p, const __nv_bfloat16 *up2_pairs, float *ptr_
     TlArgs a = {};
     a.in = reinterpret_cast<const uint8_t *>(up2_pairs);
     a.wblob = reinterpret_cast<const uint8_t *>(p->w.tail_blob);
-    a.bias4 = p->u4_bias;
+    a.bias4 = p->u4_bias == 0.f ? 0.f : p->u4_bias;         // +0.0 for a bias of -0.0: -0.0 and +0.0 are one value for the argmax
     a.ptr_out = ptr_out;
     a.xy = xy;
     a.up3_dbg = up3_dbg;
