@@ -1,0 +1,71 @@
+/* ofb_replay.h -- C ABI of the device-resident replay memory in libofb.so (sm_100a).
+ *
+ * The reference keeps Trainer.memory as a deque of (obs, iaction, ipointer, reward, next_obs, done) with every observation
+ * a pair of 400x400 maps (agents/qlearnIA_V2.py:237-238).  At batch scale the maps are far too large to keep: 40 000 B per
+ * arena and frame in OFB_MAP_BITS format.  This memory keeps arena STATE SNAPSHOTS instead -- the header, the ship records
+ * and the live prefix of the laser list of ofb_common.cuh's arena block, about 1 KB at the default workload -- and
+ * rasterises only the transitions that are sampled, with the raster code of the frame kernel, so the gathered maps are
+ * bit-identical to those the frame wrote.
+ *
+ * A transition of tracked arena a and policy ship p is (obs_t, a_t, r_{t+1}, obs_{t+1}, done_{t+1}) from two consecutive
+ * snapshots of the arena (QlearnIA.play's rules, agents/qlearnIA_V2.py:372-401):
+ *   - it exists only if the ship was alive at t and both snapshots belong to the same episode (the header's episode
+ *     counter, which every ofb_reset of the arena increments -- masked resets included);
+ *   - reward = the ship's pending reward at t+1 (obs_vec[0] of the next observation), done = the ship is dead at t+1;
+ *     so a death yields exactly one transition, with done = 1.
+ *
+ * Conventions are those of ofb.h.  The handle owns the ring of `depth` frame slots (64-bit addressed: depth x count x
+ * ofb_state_stride bytes) and its per-transition fields, all allocated at create time; push, index and gather allocate
+ * nothing and never synchronise the host.  A ring of depth D holds the transitions of the last D-1 pushed frames: the
+ * newest slot has no successor yet.
+ *
+ * Tensor formats (P = policy ships of the memory, in the order of ship_index_host)
+ *   iaction  int32 [N, P]          played action index of every policy ship of the handle's N arenas (PolicyB200.act)
+ *   xy       int32 [N, P, 2]       played pointer (x, y)
+ *   ids      int32 [M]             transition ids from ofb_replay_index (opaque; valid until the next push)
+ *   gather outputs, per sampled transition b: maps_* uint32 [B, 2, W*H/32] (OFB_MAP_BITS), vec_* float [B, 8] (ofb_obs_vec's
+ *   head of the ship), iaction int32 [B], pointer int32 [B, 2] = (x, y), reward float [B], done uint8 [B] -- the formats of
+ *   ofb_trainer_td_targets and ofb_trainer_fit (ofb_train.h).
+ */
+#ifndef OFB_REPLAY_H
+#define OFB_REPLAY_H
+
+#include <stdint.h>
+#include "ofb.h"
+
+#ifdef __cplusplus
+extern "C" {
+#endif
+
+typedef struct ofb_replay ofb_replay;
+
+/* Track arenas [first, first + count) of handle h and their policy ships ship_index_host[P] (host, distinct, < n_ships), with
+ * a ring of depth >= 2 frames.  depth * count * P must stay below 2^31. */
+int ofb_replay_create(const ofb_arenas *h, int64_t first, int64_t count, const int32_t *ship_index_host, int32_t n_policy,
+                      int32_t depth, ofb_replay **out);
+int ofb_replay_destroy(ofb_replay *r);
+/* device bytes the handle owns (ring + per-transition fields + index scratch) */
+int64_t ofb_replay_device_bytes(const ofb_replay *r);
+/* frames pushed since create (host counter) */
+int64_t ofb_replay_pushes(const ofb_replay *r);
+
+/* Snapshot the tracked arenas' current state into the next slot, with the PLAYED (iaction, xy) of their policy ships, and
+ * complete the previous slot's transitions (valid flag, reward, done).  Call it after the actions of the frame were
+ * chosen and before the frame is stepped, so the snapshot is the observation the action was chosen on.  h must be the
+ * handle the memory was created on. */
+int ofb_replay_push(ofb_replay *r, const ofb_arenas *h, const int32_t *iaction_dev, const int32_t *xy_dev, void *stream);
+
+/* Compact the ids of the valid transitions into ids_dev (capacity (depth - 1) * count * P) in age order: oldest frame first,
+ * then arena, then ship.  count_dev (int32 [1]) receives their number. */
+int ofb_replay_index(ofb_replay *r, int32_t *ids_dev, int32_t *count_dev, void *stream);
+
+/* Rasterise both snapshots of each of the `batch` transitions ids_dev[0..batch) and write their fields (any output may be
+ * NULL to skip it). */
+int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, int32_t batch, uint32_t *maps_obs_dev, float *vec_obs_dev,
+                      uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev, int32_t *pointer_dev,
+                      float *reward_dev, uint8_t *done_dev, void *stream);
+
+#ifdef __cplusplus
+}
+#endif
+#endif /* OFB_REPLAY_H */

@@ -148,6 +148,17 @@ def load():
     lib.ofb_trainer_get_grads.argtypes = [vp, vp, vp]
     lib.ofb_trainer_steps.argtypes = [vp]
     lib.ofb_trainer_steps.restype = i64
+    lib.ofb_replay_create.argtypes = [vp, i64, i64, vp, i32, i32, C.POINTER(vp)]
+    lib.ofb_replay_destroy.argtypes = [vp]
+    lib.ofb_replay_device_bytes.argtypes = [vp]
+    lib.ofb_replay_device_bytes.restype = i64
+    lib.ofb_replay_pushes.argtypes = [vp]
+    lib.ofb_replay_pushes.restype = i64
+    lib.ofb_replay_push.argtypes = [vp, vp, vp, vp, vp]
+    lib.ofb_replay_index.argtypes = [vp, vp, vp, vp]
+    lib.ofb_replay_gather.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    for name in ("ofb_replay_create", "ofb_replay_destroy", "ofb_replay_push", "ofb_replay_index", "ofb_replay_gather"):
+        getattr(lib, name).restype = i32
     for name in ("ofb_trainer_create", "ofb_trainer_destroy", "ofb_trainer_fit", "ofb_trainer_forward",
                  "ofb_trainer_td_targets", "ofb_trainer_get_weights", "ofb_trainer_get_grads"):
         getattr(lib, name).restype = i32

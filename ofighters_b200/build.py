@@ -23,6 +23,7 @@ UNITS = [
     ("ofb_arena.cu", ["-fmad=false"]),
     ("ofb_step.cu", ["-fmad=false"]),
     ("ofb_raster.cu", ["-fmad=false"]),
+    ("ofb_replay.cu", ["-fmad=false"]),
     ("ofb_policy.cu", []),
     ("ofb_policy_tc.cu", []),
     ("ofb_policy_tz.cu", []),

@@ -1,0 +1,353 @@
+// Device-resident replay memory (include/ofb_replay.h) for sm_100a (compiled with -fmad=false: the gather rasterises
+// lasers in fp64 with the frame kernel's code, ofb_raster_dev.cuh, so its maps are bit-identical to the frame's).
+//
+// Ring layout: slot s, tracked arena a -> ring + (s * count + a) * stride, the first bytes of an arena block (header,
+// ships, live laser groups) copied from the handle's state.  Per transition id = s * count * P + a * P + p (P policy ships):
+// the played action and pointer of frame s, and -- once frame s + 1 was pushed -- valid / reward / done.
+#include <cstring>
+#include <new>
+#include "ofb_common.cuh"
+#include "ofb_raster_dev.cuh"
+#include "../../include/ofb_replay.h"
+
+#define OFB_REPLAY_TILE 2048          // candidates per block of the index kernels: 256 threads x 8
+struct ofb_replay {
+    const ofb_arenas *h;
+    ArenaLayout lay;
+    int device;
+    long long first, count;
+    int P, depth;
+    int32_t *ships;              // [P] ship index of each policy ship
+    char *ring;                  // depth * count * stride bytes
+    int32_t *act;                // [depth * count * P]
+    int2 *xy;                    // [depth * count * P]
+    float *reward;               // [depth * count * P]
+    uint8_t *valid, *done;       // [depth * count * P]
+    int32_t *tile_count;         // [n_tiles] scratch of ofb_replay_index
+    long long n_tiles;
+    long long pushes;            // frames pushed so far
+    int newest;                  // slot of the last push
+    size_t bytes;
+};
+
+// ---------------------------------------------------------------- push: one warp per tracked arena
+__global__ void __launch_bounds__(128)
+k_replay_push(const char *__restrict__ state, const ArenaLayout lay, long long first, long long count,
+              const int32_t *__restrict__ ships, int P, char *__restrict__ ring, int slot, int prev, const int32_t *__restrict__ iaction_in,
+              const int2 *__restrict__ xy_in, int32_t *__restrict__ act, int2 *__restrict__ xy, float *__restrict__ reward,
+              uint8_t *__restrict__ valid, uint8_t *__restrict__ done) {
+    const long long a = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (a >= count) return;
+    const char *src = state + (first + a) * (long long)lay.stride;
+    char *dst = ring + ((long long)slot * count + a) * (long long)lay.stride;
+    const int *hdr = reinterpret_cast<const int *>(src);
+    const int n = hdr[HDR_NLASERS];
+    // header + ships + the live laser groups: a multiple of 16 bytes (off_laser and OFB_GROUP_BYTES both are)
+    const int n16 = (lay.off_laser + ((n + 7) >> 3) * OFB_GROUP_BYTES) >> 4;
+    const uint4 *s4 = reinterpret_cast<const uint4 *>(src);
+    uint4 *d4 = reinterpret_cast<uint4 *>(dst);
+#pragma unroll 4                                           // (the default unroll spills to local memory)
+    for (int i = lane; i < n16; i += 32) d4[i] = s4[i];
+    if (lane < P) {
+        const long long cP = count * P;
+        const long long j = a * P + lane;
+        const int si = ships[lane];
+        const uint4 rec = reinterpret_cast<const uint4 *>(src + lay.off_ship)[si];
+        if (prev >= 0) {                                   // frame t = slot `prev` gets its successor t+1 = this state
+            const char *old = ring + ((long long)prev * count + a) * (long long)lay.stride;
+            const uint4 orec = reinterpret_cast<const uint4 *>(old + lay.off_ship)[si];
+            const bool same_episode = reinterpret_cast<const int *>(old)[HDR_EPISODE] == hdr[HDR_EPISODE];
+            valid[prev * cP + j] = (same_episode && (orec.x >> 31)) ? 1 : 0;
+            reward[prev * cP + j] = (float)ship_unpack(rec).reward;
+            done[prev * cP + j] = (rec.x >> 31) ? 0 : 1;
+        }
+        const long long o = (long long)slot * cP + j;
+        valid[o] = 0;                                      // the newest frame has no successor yet
+        act[o] = iaction_in[(first + a) * P + lane];
+        xy[o] = xy_in[(first + a) * P + lane];
+    }
+}
+
+// ---------------------------------------------------------------- index: count per tile, scan, scatter in order
+// candidate c in [0, nf * cP): frame f = c / cP (0 = oldest complete frame), its transition c % cP
+__device__ __forceinline__ long long replay_id(long long c, long long cP, int oldest, int depth) {
+    const long long f = c / cP;
+    return (long long)((oldest + f) % depth) * cP + (c - f * cP);
+}
+
+__global__ void __launch_bounds__(256)
+k_replay_count(const uint8_t *__restrict__ valid, long long cP, long long n_cand, int oldest, int depth,
+               int32_t *__restrict__ tile_count) {
+    __shared__ int s_warp[8];
+    const long long c0 = (long long)blockIdx.x * OFB_REPLAY_TILE + threadIdx.x * 8;
+    int k = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++)
+        if (c0 + i < n_cand) k += valid[replay_id(c0 + i, cP, oldest, depth)];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) k += __shfl_xor_sync(0xffffffffu, k, o);
+    if ((threadIdx.x & 31) == 0) s_warp[threadIdx.x >> 5] = k;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        int t = 0;
+        for (int w = 0; w < 8; w++) t += s_warp[w];
+        tile_count[blockIdx.x] = t;
+    }
+}
+
+// exclusive scan of the tile counts in place (one block); the total goes to count_out
+__global__ void __launch_bounds__(1024) k_replay_scan(int32_t *tile_count, long long n_tiles, int32_t *count_out) {
+    __shared__ int s_sum[1024];
+    const long long per = (n_tiles + 1023) / 1024;
+    const long long b0 = threadIdx.x * per, b1 = min(n_tiles, b0 + per);
+    int k = 0;
+    for (long long i = b0; i < b1; i++) k += tile_count[i];
+    s_sum[threadIdx.x] = k;
+    __syncthreads();
+    for (int o = 1; o < 1024; o <<= 1) {                   // Hillis-Steele inclusive scan of the per-thread sums
+        const int v = threadIdx.x >= o ? s_sum[threadIdx.x - o] : 0;
+        __syncthreads();
+        s_sum[threadIdx.x] += v;
+        __syncthreads();
+    }
+    int run = s_sum[threadIdx.x] - k;
+    for (long long i = b0; i < b1; i++) {
+        const int c = tile_count[i];
+        tile_count[i] = run;
+        run += c;
+    }
+    if (threadIdx.x == 1023) *count_out = s_sum[1023];
+}
+
+__global__ void __launch_bounds__(256)
+k_replay_scatter(const uint8_t *__restrict__ valid, long long cP, long long n_cand, int oldest, int depth,
+                 const int32_t *__restrict__ tile_off, int32_t *__restrict__ ids) {
+    __shared__ int s_warp[8];
+    const long long c0 = (long long)blockIdx.x * OFB_REPLAY_TILE + threadIdx.x * 8;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    long long id[8];
+    unsigned m = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        id[i] = c0 + i < n_cand ? replay_id(c0 + i, cP, oldest, depth) : 0;
+        if (c0 + i < n_cand && valid[id[i]]) m |= 1u << i;
+    }
+    const int k = __popc(m);
+    int incl = k;                                          // warp inclusive scan
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    int base = tile_off[blockIdx.x];
+    for (int w = 0; w < warp; w++) base += s_warp[w];
+    int pos = base + incl - k;
+#pragma unroll
+    for (int i = 0; i < 8; i++)
+        if (m & (1u << i)) ids[pos++] = (int32_t)id[i];
+}
+
+// ---------------------------------------------------------------- gather: one CTA per (sample, obs | next)
+__global__ void __launch_bounds__(256)
+k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long count, int P, int depth,
+                const int32_t *__restrict__ ships,                const int32_t *__restrict__ ids, const int32_t *__restrict__ act, const int2 *__restrict__ axy,
+                const float *__restrict__ rew, const uint8_t *__restrict__ dn, uint32_t *__restrict__ maps_obs,
+                float *__restrict__ vec_obs, uint32_t *__restrict__ maps_next, float *__restrict__ vec_next,
+                int32_t *__restrict__ iaction, int32_t *__restrict__ pointer, float *__restrict__ reward,
+                uint8_t *__restrict__ done) {
+    extern __shared__ __align__(128) uint32_t bits[];      // [2][words], as k_raster
+    const int W = lay.W, H = lay.H;
+    const int words = (W * H) >> 5;
+    const int b = blockIdx.x, next = blockIdx.y;
+    const long long cP = count * P;
+    const long long id = ids[b];
+    const long long slot = id / cP, j = id - slot * cP;
+    const long long a = j / P;
+    const int p = (int)(j - a * P);
+    const long long s = next ? (slot + 1) % depth : slot;
+    const char *base = ring + (s * count + a) * (long long)lay.stride;
+    const int *hdr = reinterpret_cast<const int *>(base);
+    const uint4 *ship = reinterpret_cast<const uint4 *>(base + lay.off_ship);
+    uint32_t *maps = next ? maps_next : maps_obs;
+    float *vec = next ? vec_next : vec_obs;
+
+    if (vec && threadIdx.x == 0) {                         // ofb_obs_vec's head (k_obs_vec) of the ship
+        const ShipRec r = ship_unpack(ship[ships[p]]);
+        float4 *v = reinterpret_cast<float4 *>(vec + (long long)b * 8);
+        v[0] = make_float4((float)r.reward, 1.0f, (float)r.px, (float)r.py);
+        v[1] = make_float4((float)lay.W, (float)lay.H, (float)r.x, (float)r.y);
+    }
+    if (!next && threadIdx.x == 1) {
+        if (iaction) iaction[b] = act[id];
+        if (pointer) reinterpret_cast<int2 *>(pointer)[b] = axy[id];
+        if (reward) reward[b] = rew[id];
+        if (done) done[b] = dn[id];
+    }
+    if (!maps) return;
+
+    const int n = hdr[HDR_NLASERS];
+    {
+        uint4 *b4 = reinterpret_cast<uint4 *>(bits);
+        for (int i = threadIdx.x; i < (2 * words) / 4; i += blockDim.x) b4[i] = make_uint4(0, 0, 0, 0);
+    }
+    __syncthreads();
+    const int rows = 2 * OFB_R_SHIP - 1;
+    for (int t = threadIdx.x; t < lay.S * rows; t += blockDim.x)
+        raster_ship_row(bits, W, H, ship[t / rows].x, t % rows - (OFB_R_SHIP - 1));
+    for (int k = threadIdx.x; k < n; k += blockDim.x) {
+        const double *lp = reinterpret_cast<const double *>(base + laser_off(lay.off_laser, k));
+        raster_laser(bits + words, W, H, lp[0], lp[OFB_G_Y / 8]);
+    }
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const unsigned bytes = (unsigned)(2 * words * 4);
+        char *dst = reinterpret_cast<char *>(maps) + (long long)b * bytes;
+        const unsigned src = (unsigned)__cvta_generic_to_shared(bits);
+        asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" :: "l"(dst), "r"(src), "r"(bytes) : "memory");
+        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+    }
+}
+
+// ---------------------------------------------------------------- C ABI
+static void replay_free(ofb_replay *r) {
+    cudaFree(r->ring);
+    cudaFree(r->act);
+    cudaFree(r->xy);
+    cudaFree(r->reward);
+    cudaFree(r->valid);
+    cudaFree(r->done);
+    cudaFree(r->tile_count);
+    cudaFree(r->ships);
+    delete r;
+}
+
+extern "C" int ofb_replay_create(const ofb_arenas *h, int64_t first, int64_t count, const int32_t *ship_index_host,
+                                 int32_t n_policy, int32_t depth, ofb_replay **out) {
+    if (!h || !out || !ship_index_host) { ofb_set_error("ofb_replay_create: null argument"); return OFB_E_ARG; }
+    if (first < 0 || count < 1 || first + count > h->n_arenas) {
+        ofb_set_error("ofb_replay_create: the tracked arenas must lie in [0, %lld)", (long long)h->n_arenas);
+        return OFB_E_ARG;
+    }
+    if (n_policy < 1 || n_policy > h->lay.S || depth < 2) {
+        ofb_set_error("ofb_replay_create: need 1 <= P <= n_ships (%d) policy ships and depth >= 2", h->lay.S);
+        return OFB_E_ARG;
+    }
+    const long long cP = (long long)count * n_policy;
+    if ((long long)depth * cP >= (1ll << 31)) {
+        ofb_set_error("ofb_replay_create: depth x count x P = %lld transitions does not fit int32 ids", (long long)depth * cP);
+        return OFB_E_ARG;
+    }
+    OFB_CUDA_CHECK(cudaSetDevice(h->device));
+    ofb_replay *r = new (std::nothrow) ofb_replay();
+    if (!r) return OFB_E_NOMEM;
+    for (int p = 0; p < n_policy; p++) {
+        const int s = ship_index_host[p];
+        bool dup = false;
+        for (int q = 0; q < p; q++) dup |= ship_index_host[q] == s;
+        if (s < 0 || s >= h->lay.S || dup) {
+            delete r;
+            ofb_set_error("ofb_replay_create: ship indices must be distinct and below n_ships (%d)", h->lay.S);
+            return OFB_E_ARG;
+        }
+    }
+    r->h = h;
+    r->lay = h->lay;
+    r->device = h->device;
+    r->first = first;
+    r->count = count;
+    r->P = n_policy;
+    r->depth = depth;
+    r->pushes = 0;
+    r->newest = depth - 1;
+    r->n_tiles = ((long long)(depth - 1) * cP + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
+    const size_t nt = (size_t)depth * cP;
+    const size_t ring = (size_t)depth * count * h->lay.stride;
+    r->bytes = ring + nt * (sizeof(int32_t) + sizeof(int2) + sizeof(float) + 2) + (size_t)r->n_tiles * sizeof(int32_t) +
+               n_policy * sizeof(int32_t);
+    if (cudaMalloc(&r->ships, n_policy * sizeof(int32_t)) != cudaSuccess || cudaMalloc(&r->ring, ring) != cudaSuccess ||
+        cudaMalloc(&r->act, nt * sizeof(int32_t)) != cudaSuccess ||
+        cudaMalloc(&r->xy, nt * sizeof(int2)) != cudaSuccess || cudaMalloc(&r->reward, nt * sizeof(float)) != cudaSuccess ||
+        cudaMalloc(&r->valid, nt) != cudaSuccess || cudaMalloc(&r->done, nt) != cudaSuccess ||
+        cudaMalloc(&r->tile_count, (size_t)r->n_tiles * sizeof(int32_t)) != cudaSuccess) {
+        cudaGetLastError();
+        ofb_set_error("ofb_replay_create: cudaMalloc of %zu bytes failed", r->bytes);
+        replay_free(r);
+        return OFB_E_NOMEM;
+    }
+    if (cudaMemset(r->valid, 0, nt) != cudaSuccess ||
+        cudaMemcpy(r->ships, ship_index_host, n_policy * sizeof(int32_t), cudaMemcpyHostToDevice) != cudaSuccess) {
+        ofb_set_error("ofb_replay_create: initialisation failed: %s", cudaGetErrorString(cudaGetLastError()));
+        replay_free(r);
+        return OFB_E_CUDA;
+    }
+    *out = r;
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_destroy(ofb_replay *r) {
+    if (!r) return OFB_OK;
+    cudaSetDevice(r->device);
+    replay_free(r);
+    return OFB_OK;
+}
+
+extern "C" int64_t ofb_replay_device_bytes(const ofb_replay *r) { return r ? (int64_t)r->bytes : OFB_E_ARG; }
+extern "C" int64_t ofb_replay_pushes(const ofb_replay *r) { return r ? (int64_t)r->pushes : OFB_E_ARG; }
+
+extern "C" int ofb_replay_push(ofb_replay *r, const ofb_arenas *h, const int32_t *iaction_dev, const int32_t *xy_dev,
+                               void *stream) {
+    if (!r || !iaction_dev || !xy_dev) { ofb_set_error("ofb_replay_push: null argument"); return OFB_E_ARG; }
+    if (h != r->h) { ofb_set_error("ofb_replay_push: the arenas are not the ones the memory was created on"); return OFB_E_ARG; }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    const int slot = (r->newest + 1) % r->depth;
+    const int prev = r->pushes > 0 ? r->newest : -1;
+    const long long threads = r->count * 32;
+    k_replay_push<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+        h->state, r->lay, r->first, r->count, r->ships, r->P, r->ring, slot, prev, iaction_dev,
+        reinterpret_cast<const int2 *>(xy_dev), r->act, r->xy, r->reward, r->valid, r->done);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    r->newest = slot;
+    r->pushes += 1;
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_index(ofb_replay *r, int32_t *ids_dev, int32_t *count_dev, void *stream) {
+    if (!r || !ids_dev || !count_dev) { ofb_set_error("ofb_replay_index: null argument"); return OFB_E_ARG; }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long filled = r->pushes < r->depth ? r->pushes : r->depth;
+    const long long nf = filled > 0 ? filled - 1 : 0;           // frames with a successor
+    const long long cP = r->count * r->P, n_cand = nf * cP;
+    if (n_cand == 0) {
+        OFB_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, sizeof(int32_t), st));
+        return OFB_OK;
+    }
+    const int oldest = (int)((r->newest - nf + r->depth) % r->depth);
+    const long long tiles = (n_cand + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
+    k_replay_count<<<(unsigned)tiles, 256, 0, st>>>(r->valid, cP, n_cand, oldest, r->depth, r->tile_count);
+    k_replay_scan<<<1, 1024, 0, st>>>(r->tile_count, tiles, count_dev);
+    k_replay_scatter<<<(unsigned)tiles, 256, 0, st>>>(r->valid, cP, n_cand, oldest, r->depth, r->tile_count, ids_dev);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, int32_t batch, uint32_t *maps_obs_dev,
+                                 float *vec_obs_dev, uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev,
+                                 int32_t *pointer_dev, float *reward_dev, uint8_t *done_dev, void *stream) {
+    if (!r || !ids_dev || batch < 0) { ofb_set_error("ofb_replay_gather: bad argument"); return OFB_E_ARG; }
+    if (batch == 0) return OFB_OK;
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    const size_t smem = (size_t)(r->lay.W * r->lay.H / 32) * 2 * sizeof(uint32_t);
+    static thread_local SmemAttrCache attr = {};
+    if (smem > 48 * 1024) OFB_CUDA_CHECK(attr.ensure(k_replay_gather, (int)smem));
+    k_replay_gather<<<dim3((unsigned)batch, 2), 256, smem, (cudaStream_t)stream>>>(
+        r->ring, r->lay, r->count, r->P, r->depth, r->ships, ids_dev, r->act, r->xy, r->reward, r->done, maps_obs_dev,
+        vec_obs_dev, maps_next_dev, vec_next_dev, iaction_dev, pointer_dev, reward_dev, done_dev);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}

@@ -1,0 +1,160 @@
+"""Device-resident replay memory: the ``Trainer.memory`` of the reference (agents/qlearnIA_V2.py:237-238) for every arena of a
+batch, through include/ofb_replay.h.
+
+``Trainer.memory`` is a deque of (obs, iaction, ipointer, reward, next_obs, done) whose observations are a pair of 400x400
+maps.  Kept like that for a batch, every arena would cost 40 KB of bit maps per frame.  ``DeviceReplayMemory`` keeps a ring
+of arena state snapshots on the device instead -- header, ships and the live laser list, about 1 KB per arena at the
+default workload -- and rasterises only the transitions a replay samples, with the frame kernel's raster code, so a
+gathered map is bit for bit the map the frame wrote.  Transitions follow ``QlearnIA.play`` (:372-401): one per policy ship
+that is alive at t, none across a restart (masked restarts included), a death once with done = 1.
+
+    memory = DeviceReplayMemory(bg, depth=16)     # all arenas, the battleground's QlearnIA / external ships
+    iact, xy = policy.act(bg, maps, ...)          # the PLAYED actions
+    memory.push(iact, xy)                         # before bg.frame(): the snapshot is the observation acted on
+    bg.frame(maps=maps)
+    trainer.replay(trainer.batch_size, memory=memory)
+
+``push`` never synchronises the host.  ``len()`` does (it compacts the valid transitions and reads their number), and so does
+``sample``.  The order of the transitions -- oldest frame first, then arena, then ship -- is the order in which ``QLearner``
+appends to ``trainer.memory``, and ``sample`` draws ``random.sample(range(len), batch_size)`` with Python's ``random`` as
+``Trainer.replay`` does on its deque, so the same ``random`` state picks the same minibatch.
+"""
+import ctypes as C
+import random
+from types import SimpleNamespace
+
+import torch
+
+from . import _lib
+
+_POLICY_BEHAVIORS = ("QlearnIA", "external")
+
+
+def _ptr(t):
+    return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(None)
+
+
+class DeviceReplayMemory:
+    def __init__(self, bg, depth=16, track=None, ships=None):
+        """``bg``: the BatchedBattleground whose arenas are remembered.  ``depth``: frames in the ring (>= 2); it holds the
+        transitions of the last ``depth - 1`` pushed frames.  ``track``: the first ``track`` arenas (default: all).
+        ``ships``: ship indices to remember, among the battleground's QlearnIA / external ships (default: all of them);
+        ``push`` takes the actions of all those ships, as ``PolicyB200.act`` returns them."""
+        if not torch.cuda.is_available():
+            raise _lib.OfbError("DeviceReplayMemory needs a CUDA device: the ring lives in HBM and has no CPU fallback")
+        policy = [i for i, b in enumerate(bg.behaviors) if b in _POLICY_BEHAVIORS]
+        if not policy:
+            raise Exception("no policy-driven ship in this battleground")
+        ships = list(policy) if ships is None else [int(s) for s in ships]
+        if not ships or len(set(ships)) != len(ships) or any(s not in policy for s in ships):
+            raise Exception("Invalid ships {} : expected distinct policy-driven ships among {}.".format(ships, policy))
+        track = bg.n_arenas if track is None else int(track)
+        if not 1 <= track <= bg.n_arenas:
+            raise Exception("Invalid track {} : the batch holds {} arenas.".format(track, bg.n_arenas))
+        self.bg = bg
+        self.device = bg.device
+        self.depth = int(depth)
+        self.track = track
+        self.ships = ships
+        self.n_policy = len(policy)                      # policy ships per arena in the actions push() takes
+        self._cols = None if ships == policy else torch.tensor([policy.index(s) for s in ships], dtype=torch.long,
+                                                               device=self.device)
+        self._lib = _lib.load()
+        idx = (C.c_int32 * len(ships))(*ships)
+        h = C.c_void_p()
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.ofb_replay_create(bg._h, 0, track, idx, len(ships), self.depth, C.byref(h)))
+        self._h = h
+        self._ids = torch.empty(max(1, (self.depth - 1) * track * len(ships)), dtype=torch.int32, device=self.device)
+        self._count = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._n = 0
+        self._stale = False
+        self.launch_count = 0
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h:
+            try:
+                self._lib.ofb_replay_destroy(h)
+            except Exception:
+                pass
+            self._h = None
+
+    def _stream(self):
+        return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    @property
+    def device_bytes(self):
+        """HBM the memory owns: the ring of snapshots, the per-transition fields and the index scratch."""
+        return int(self._lib.ofb_replay_device_bytes(self._h))
+
+    @property
+    def frames(self):
+        """Frames pushed so far."""
+        return int(self._lib.ofb_replay_pushes(self._h))
+
+    # ------------------------------------------------------------------ write
+    def push(self, iaction, xy, bg=None):
+        """Remember the current state of the tracked arenas with the actions their policy ships PLAY from it: ``iaction``
+        int32 [A*P] and ``xy`` int32 [A*P, 2] as ``PolicyB200.act`` returns them (A arenas, P policy ships).  Call it after
+        the actions were chosen and before ``bg.frame``.  Asynchronous: no host synchronisation."""
+        if bg is not None and bg is not self.bg:
+            raise Exception("Invalid battleground : this memory remembers another battleground's arenas.")
+        N, P = self.bg.n_arenas, self.n_policy
+        for name, t, shapes in (("iaction", iaction, ((N * P,), (N, P))), ("xy", xy, ((N * P, 2), (N, P, 2)))):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.int32 or t.device != self.device or \
+                    tuple(t.shape) not in shapes:
+                raise Exception("Invalid {} : expected an int32 tensor of shape {} on {}.".format(name, shapes[0], self.device))
+        iaction, xy = iaction.reshape(N, P), xy.reshape(N, P, 2)
+        if self._cols is not None:
+            iaction, xy = iaction.index_select(1, self._cols), xy.index_select(1, self._cols)
+        iaction, xy = iaction.contiguous(), xy.contiguous()
+        _lib.check(self._lib.ofb_replay_push(self._h, self.bg._h, _ptr(iaction), _ptr(xy), self._stream()))
+        self.launch_count += 1
+        self._stale = True
+
+    # ------------------------------------------------------------------ read
+    def __len__(self):
+        """Number of valid transitions (synchronises with the device)."""
+        if self._stale:
+            _lib.check(self._lib.ofb_replay_index(self._h, _ptr(self._ids), _ptr(self._count), self._stream()))
+            self.launch_count += 3
+            self._n = int(self._count.item())
+            self._stale = False
+        return self._n
+
+    def gather(self, positions):
+        """The transitions at ``positions`` (0 = oldest) -> SimpleNamespace of device tensors: maps_obs / maps_next int32
+        [B, 2, W*H/32] bit maps, vec_obs / vec_next float32 [B, 8], iaction int32 [B], pointer int32 [B, 2] = (x, y),
+        reward float32 [B], done uint8 [B] -- the inputs of ``TrainerB200.replay``'s targets and fit."""
+        n = len(self)
+        pos = torch.as_tensor(positions, dtype=torch.int64).reshape(-1)
+        if pos.numel() < 1:
+            raise Exception("gather of no transition")
+        if int(pos.min()) < 0 or int(pos.max()) >= n:
+            raise Exception("Invalid positions : the memory holds {} transitions.".format(n))
+        ids = self._ids.index_select(0, pos.to(self.device)).contiguous()
+        B = ids.numel()
+        words = self.bg.config.width * self.bg.config.height // 32
+        dev = self.device
+        out = SimpleNamespace(
+            maps_obs=torch.empty((B, 2, words), dtype=torch.int32, device=dev),
+            vec_obs=torch.empty((B, 8), dtype=torch.float32, device=dev),
+            maps_next=torch.empty((B, 2, words), dtype=torch.int32, device=dev),
+            vec_next=torch.empty((B, 8), dtype=torch.float32, device=dev),
+            iaction=torch.empty((B,), dtype=torch.int32, device=dev),
+            pointer=torch.empty((B, 2), dtype=torch.int32, device=dev),
+            reward=torch.empty((B,), dtype=torch.float32, device=dev),
+            done=torch.empty((B,), dtype=torch.uint8, device=dev))
+        _lib.check(self._lib.ofb_replay_gather(self._h, _ptr(ids), B, _ptr(out.maps_obs), _ptr(out.vec_obs), _ptr(out.maps_next),
+                                               _ptr(out.vec_next), _ptr(out.iaction), _ptr(out.pointer), _ptr(out.reward),
+                                               _ptr(out.done), self._stream()))
+        self.launch_count += 1
+        return out
+
+    def sample(self, batch_size):
+        """``random.sample(range(len(self)), batch_size)`` -- the draw ``Trainer.replay`` makes on its deque -- gathered."""
+        n = len(self)
+        if n < 1:
+            raise Exception("sample on an empty replay memory")
+        return self.gather(random.sample(range(n), batch_size))

@@ -214,22 +214,36 @@ class TrainerB200:
         """:237-238.  ``state`` / ``next_state`` = (maps_bits int32 [2,5000], vec float32 [8]) device tensors."""
         self.memory.append([state, iaction, ipointer, reward, next_state, done])
 
-    def replay(self, batch_size):
+    def replay(self, batch_size, memory=None):
         """:240-287.  Targets from predictions on obs and next_obs; like the reference, the fitted INPUTS are the
-        next observations (``inputs1[i] = img_input`` is evaluated after img_input was rebuilt from next_obs, :281-282)."""
-        batch_size = min(batch_size, len(self.memory))
-        if batch_size < 1:
-            raise Exception("replay on an empty memory")
-        minibatch = random.sample(self.memory, batch_size)
+        next observations (``inputs1[i] = img_input`` is evaluated after img_input was rebuilt from next_obs, :281-282).
+        ``memory``: a ``replay.DeviceReplayMemory`` to draw the minibatch from instead of ``self.memory`` (same
+        ``random.sample`` draw over its transitions in age order)."""
         dev = self.device
-        maps_o = torch.stack([m[0][0] for m in minibatch]).to(dev).contiguous()
-        vec_o = torch.stack([m[0][1] for m in minibatch]).to(dev).contiguous()
-        maps_n = torch.stack([m[4][0] for m in minibatch]).to(dev).contiguous()
-        vec_n = torch.stack([m[4][1] for m in minibatch]).to(dev).contiguous()
-        iaction = torch.tensor([int(m[1]) for m in minibatch], dtype=torch.int32, device=dev)
-        pointer = torch.tensor([[int(m[2][0]), int(m[2][1])] for m in minibatch], dtype=torch.int32, device=dev)
-        reward = torch.tensor([float(m[3]) for m in minibatch], dtype=torch.float32, device=dev)
-        done = torch.tensor([1 if m[5] else 0 for m in minibatch], dtype=torch.uint8, device=dev)
+        if memory is None:
+            batch_size = min(batch_size, len(self.memory))
+            if batch_size < 1:
+                raise Exception("replay on an empty memory")
+            minibatch = random.sample(self.memory, batch_size)
+            maps_o = torch.stack([m[0][0] for m in minibatch]).to(dev).contiguous()
+            vec_o = torch.stack([m[0][1] for m in minibatch]).to(dev).contiguous()
+            maps_n = torch.stack([m[4][0] for m in minibatch]).to(dev).contiguous()
+            vec_n = torch.stack([m[4][1] for m in minibatch]).to(dev).contiguous()
+            iaction = torch.tensor([int(m[1]) for m in minibatch], dtype=torch.int32, device=dev)
+            pointer = torch.tensor([[int(m[2][0]), int(m[2][1])] for m in minibatch], dtype=torch.int32, device=dev)
+            reward = torch.tensor([float(m[3]) for m in minibatch], dtype=torch.float32, device=dev)
+            done = torch.tensor([1 if m[5] else 0 for m in minibatch], dtype=torch.uint8, device=dev)
+        else:
+            if memory.device != dev:
+                raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, dev))
+            batch_size = min(batch_size, len(memory))
+            if batch_size < 1:
+                raise Exception("replay on an empty memory")
+            if batch_size > self.max_batch:
+                raise Exception("Invalid batch : {} samples but the trainer was sized for {}.".format(batch_size, self.max_batch))
+            mb = memory.sample(batch_size)
+            maps_o, vec_o, maps_n, vec_n = mb.maps_obs, mb.vec_obs, mb.maps_next, mb.vec_next
+            iaction, pointer, reward, done = mb.iaction, mb.pointer, mb.reward, mb.done
         act_o, ptr_o = self.predict(maps_o, vec_o)
         act_n, ptr_n = self.predict(maps_n, vec_n)
         _lib.check(self._lib.ofb_trainer_td_targets(_ptr(act_o), _ptr(ptr_o), _ptr(act_n), _ptr(ptr_n), _ptr(iaction),
@@ -348,3 +362,69 @@ class QLearner:
         h = self.trainer.replay(self.trainer.batch_size)
         self.losses.append(h.history["loss"][0])
         return True
+
+
+class BatchedQLearner:
+    """``QLearner``'s loop for every arena a ``replay.DeviceReplayMemory`` tracks: the policy ships of the whole batch feed one
+    shared ``TrainerB200``.  Each frame ``act`` chooses the actions (the collecting phase's ``random_play()`` for the first
+    ``collecting_steps`` frames, then eps-greedy with the trainer's schedule, on the device), pushes the snapshot and the
+    PLAYED actions into the memory, advances epsilon once outside the collecting phase, replays ``trainer.batch_size``
+    transitions every ``replay_every`` frames once the memory holds one, and saves a snapshot of the model on the first frame
+    of every ``snapshot``-th episode.  The caller steps the frame and calls ``reset`` at every restart, as with ``QLearner``.
+
+    Departures from ``QlearnIA.play`` (agents/qlearnIA_V2.py:372-417), which ``QLearner`` follows for a few tracked arenas:
+      * no replay at each death: at this scale that would be thousands of fits per frame; replays come every
+        ``replay_every`` frames only;
+      * the memory is bounded in frames (the last ``depth - 1``), not in transitions (``memory_size``);
+      * epsilon advances once per frame, not once per decision of bot 1 (which stops at its death);
+      * no host synchronisation on frames without a replay.
+
+    ``actor``: the inference engine that drives the arenas (default: the trainer's own ``model``, which every fit refreshes)."""
+
+    def __init__(self, trainer, memory, replay_every=50, collecting_steps=20, snapshot=50, actor=None, snapshot_folder="networks"):
+        if memory.device != trainer.device:
+            raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, trainer.device))
+        self.trainer = trainer
+        self.memory = memory
+        self.actor = actor if actor is not None else trainer.model
+        self.replay_every = int(replay_every)
+        self.collecting_steps = int(collecting_steps)
+        self.snapshot = int(snapshot)
+        self.snapshot_folder = snapshot_folder
+        self.total_steps = 0
+        self.steps = 0
+        self.episode = 0
+        self.losses = []
+        self.epsilons = []
+        self.saved = []
+
+    @property
+    def collecting(self):
+        """True while the NEXT frame belongs to the random collecting phase (as ``QLearner.collecting``)."""
+        return self.total_steps + 1 < self.collecting_steps
+
+    def reset(self):
+        """Episode bookkeeping at a restart: log epsilon, count the episode."""
+        self.episode += 1
+        self.steps = 0
+        self.epsilons.append(self.trainer.epsilon.get())
+
+    def act(self, bg, maps_bits):
+        """One frame of every policy ship: choose and write the action rows, remember, learn.  -> (iaction, xy, replayed)"""
+        if bg is not self.memory.bg:
+            raise Exception("Invalid battleground : the memory remembers another battleground's arenas.")
+        collecting = self.collecting
+        iact, xy = self.actor.act(bg, maps_bits, epsilon=self.trainer.epsilon, collecting=collecting)
+        self.memory.push(iact, xy)
+        self.total_steps += 1
+        self.steps += 1
+        if not collecting:
+            self.trainer.decay_epsilon()
+        replayed = False
+        if self.total_steps % self.replay_every == 0 and len(self.memory) > 0:
+            h = self.trainer.replay(self.trainer.batch_size, memory=self.memory)
+            self.losses.append(h.history["loss"][0])
+            replayed = True
+        if self.snapshot > 0 and self.episode > 0 and self.episode % self.snapshot == 0 and self.steps < 2:
+            self.saved.append(self.trainer.save(id="iteration-%s" % self.episode, overwrite=True, folder=self.snapshot_folder))
+        return iact, xy, replayed
