@@ -19,6 +19,9 @@
  * nothing and never synchronise the host.  A ring of depth D holds the transitions of the last D-1 pushed frames: the
  * newest slot has no successor yet.
  *
+ * Opt-in prioritized replay (ofb_replay_enable_priorities) adds a sampling mass per transition, a device sampler that
+ * draws in proportion to it over the same candidates as ofb_replay_index, and the update of the masses from TD errors.
+ *
  * Tensor formats (P = policy ships of the memory, in the order of ship_index_host)
  *   iaction  int32 [N, P]          played action index of every policy ship of the handle's N arenas (PolicyB200.act)
  *   xy       int32 [N, P, 2]       played pointer (x, y)
@@ -64,6 +67,42 @@ int ofb_replay_index(ofb_replay *r, int32_t *ids_dev, int32_t *count_dev, void *
 int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, int32_t batch, uint32_t *maps_obs_dev, float *vec_obs_dev,
                       uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev, int32_t *pointer_dev,
                       float *reward_dev, uint8_t *done_dev, void *stream);
+
+/* ---- Prioritized replay (Schaul et al. 2016, proportional variant).
+ * Every transition id carries a sampling mass; a transition is drawn with probability mass / (sum of the valid masses).
+ * The mass is (|td_act| + |td_ptr| + eps)^alpha, the TD errors of ofb_trainer_td_errors (both heads regress on the same
+ * return r + gamma * max).  A transition gets the largest mass set so far (initially 1) when it becomes valid, so a new
+ * transition is likely drawn at least once. */
+typedef struct ofb_replay_prio_config {
+    float alpha;          /* >= 0; 0 = uniform */
+    float eps;            /* >= 0, added to |td| so that a zero error keeps a chance */
+    uint64_t seed;        /* key of the sampler's Philox stream */
+    int32_t reserved[8];
+} ofb_replay_prio_config;
+
+/* Allocate the masses (fp32 [depth * count * P], indexed by transition id), the device maximum mass and the sampler's tile
+ * scratch.  Allowed once, before the first push; nothing allocates afterwards.  ofb_replay_device_bytes counts them. */
+int ofb_replay_enable_priorities(ofb_replay *r, const ofb_replay_prio_config *cfg);
+
+/* Draw `batch` transitions in proportion to their masses, stratified: draw b falls in [b, b+1) / batch of the total mass,
+ * with U_b from Philox keyed by (seed, samples drawn so far, b) -- a run is reproducible.  No host synchronisation, no
+ * allocation.  ids_out int32 [batch] (age order is non-decreasing in b), weight_out float [batch] = the importance weight
+ * (mass_b / mass_min)^(-beta) <= 1 with mass_min the smallest non-zero valid mass, which equals Schaul's
+ * (N P(i))^(-beta) / max_j w_j over the whole memory.  n_valid_out int32 [1] = number of valid transitions of non-zero mass
+ * (all valid ones when eps > 0); when it is 0 the ids and weights are left undefined.  Ids stay valid until the next push.
+ * Cost: one pass over the valid flags and masses of all candidates, then one tile of 2048 candidates per draw. */
+int ofb_replay_sample_prioritized(ofb_replay *r, int32_t batch, float beta, int32_t *ids_out, float *weight_out,
+                                  int32_t *n_valid_out, void *stream);
+
+/* mass[ids[b]] = (|td_act[b]| + |td_ptr[b]| + eps)^alpha and raise the maximum mass.  ids int32 [batch] (ids out of
+ * [0, depth * count * P) are skipped), td_* float [batch].  Duplicate ids must carry identical errors (they do when they come
+ * from one forward), so the result is deterministic. */
+int ofb_replay_update_priorities(ofb_replay *r, const int32_t *ids_dev, const float *td_act_dev, const float *td_ptr_dev,
+                                 int32_t batch, void *stream);
+
+/* Copy to device buffers, any of which may be NULL: the masses (float [depth * count * P]), the maximum mass (float [1]) and
+ * the fp64 total mass the last ofb_replay_sample_prioritized drew from (double [1]). */
+int ofb_replay_read_priorities(const ofb_replay *r, float *mass_dev, float *max_mass_dev, double *last_total_dev, void *stream);
 
 #ifdef __cplusplus
 }

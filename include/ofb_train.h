@@ -6,6 +6,8 @@
  *   model.fit(x, y, epochs=1, batch_size=B)          :281-286    -> ofb_trainer_fit
  *        = one optimiser step on  mse(output1) + mse(output2)  with BatchNormalization in
  *          training mode (batch statistics, moving averages updated) and Adam(lr)   :188,308
+ * and, for prioritized replay (ofb_replay.h), the sample-weighted fit (ofb_trainer_fit_weighted) and the TD errors that
+ * set the priorities (ofb_trainer_td_errors).
  *   model weights (save / load_model)                :70,298      -> ofb_trainer_get_weights
  *
  * Conventions are those of ofb.h: int return codes, ofb_last_error(), caller-owned device buffers,
@@ -63,6 +65,16 @@ int ofb_trainer_destroy(ofb_trainer *t);
 int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps_bits_dev, const float *vec_dev, const float *target_act_dev,
                     const float *target_ptr_dev, int batch, float *loss_dev, void *stream);
 
+/* model.fit(..., sample_weight=w) (prioritized replay's importance weights): one Adam step on
+ *   sum over the two heads of (1/B) sum_b w_b * mse_b,   mse_b = sample b's mean squared error over that head's elements,
+ * which is tf.keras' sample_weight under SUM_OVER_BATCH_SIZE; with w = 1 it is ofb_trainer_fit's loss.  loss_dev receives
+ * the weighted losses (what history['loss'] reports when sample_weight is given).  BatchNormalization keeps unweighted
+ * batch statistics, as Keras does.  sample_weight_dev float [B], every w_b >= 0.  Standalone Keras 2.2 divided instead by
+ * the fraction of non-zero weights, so the two forms differ only when some w_b = 0. */
+int ofb_trainer_fit_weighted(ofb_trainer *t, const uint32_t *maps_bits_dev, const float *vec_dev, const float *target_act_dev,
+                             const float *target_ptr_dev, const float *sample_weight_dev, int batch, float *loss_dev,
+                             void *stream);
+
 /* Training-mode forward only (the predictions fit() differentiates): act [B,2], ptr [B,400,400], either may be NULL. */
 int ofb_trainer_forward(ofb_trainer *t, const uint32_t *maps_bits_dev, const float *vec_dev, int batch, float *act_dev,
                         float *ptr_dev, void *stream);
@@ -77,6 +89,15 @@ int ofb_trainer_td_targets(const float *act_obs_dev, const float *ptr_obs_dev, c
                            const float *ptr_next_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
                            const float *reward_dev, const uint8_t *done_dev, float gamma, int batch,
                            float *target_act_dev, float *target_ptr_dev, void *stream);
+
+/* Signed TD errors (prioritized replay's priorities) at the entries ofb_trainer_td_targets overwrites, same arguments:
+ *   td_act[b] = target[b][iaction[b]] - act_obs[b][iaction[b]],   td_ptr[b] = ptr_target[b][px][py] - ptr_obs[b][px][py]
+ * with each target computed by ofb_trainer_td_targets' own fp32 expression, so td equals t_target - prediction exactly.
+ * Call it before ofb_trainer_td_targets overwrites act_obs / ptr_obs in place.  td_* float [B]. */
+int ofb_trainer_td_errors(const float *act_obs_dev, const float *ptr_obs_dev, const float *act_next_dev,
+                          const float *ptr_next_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
+                          const float *reward_dev, const uint8_t *done_dev, float gamma, int batch, float *td_act_dev,
+                          float *td_ptr_dev, void *stream);
 
 /* Flat copies to HOST (synchronise `stream` first): current weights / gradients of the last fit. */
 int ofb_trainer_get_weights(ofb_trainer *t, float *weights_flat_host, void *stream);

@@ -49,6 +49,10 @@ class OfbTrainConfig(C.Structure):
                 ("max_batch", C.c_int32), ("reserved", C.c_int32 * 8)]
 
 
+class OfbReplayPrioConfig(C.Structure):
+    _fields_ = [("alpha", C.c_float), ("eps", C.c_float), ("seed", C.c_uint64), ("reserved", C.c_int32 * 8)]
+
+
 class OfbEpsSchedule(C.Structure):
     _fields_ = [("kind", C.c_int32), ("reserved", C.c_int32), ("start", C.c_double), ("period", C.c_double),
                 ("decay", C.c_double), ("floor", C.c_double)]
@@ -144,6 +148,8 @@ def load():
     lib.ofb_trainer_fit.argtypes = [vp, vp, vp, vp, vp, i32, vp, vp]
     lib.ofb_trainer_forward.argtypes = [vp, vp, vp, i32, vp, vp, vp]
     lib.ofb_trainer_td_targets.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, i32, vp, vp, vp]
+    lib.ofb_trainer_fit_weighted.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, vp]
+    lib.ofb_trainer_td_errors.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, i32, vp, vp, vp]
     lib.ofb_trainer_get_weights.argtypes = [vp, vp, vp]
     lib.ofb_trainer_get_grads.argtypes = [vp, vp, vp]
     lib.ofb_trainer_steps.argtypes = [vp]
@@ -157,10 +163,16 @@ def load():
     lib.ofb_replay_push.argtypes = [vp, vp, vp, vp, vp]
     lib.ofb_replay_index.argtypes = [vp, vp, vp, vp]
     lib.ofb_replay_gather.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
-    for name in ("ofb_replay_create", "ofb_replay_destroy", "ofb_replay_push", "ofb_replay_index", "ofb_replay_gather"):
+    lib.ofb_replay_enable_priorities.argtypes = [vp, C.POINTER(OfbReplayPrioConfig)]
+    lib.ofb_replay_sample_prioritized.argtypes = [vp, i32, C.c_float, vp, vp, vp, vp]
+    lib.ofb_replay_update_priorities.argtypes = [vp, vp, vp, vp, i32, vp]
+    lib.ofb_replay_read_priorities.argtypes = [vp, vp, vp, vp, vp]
+    for name in ("ofb_replay_create", "ofb_replay_destroy", "ofb_replay_push", "ofb_replay_index", "ofb_replay_gather",
+                 "ofb_replay_enable_priorities", "ofb_replay_sample_prioritized", "ofb_replay_update_priorities",
+                 "ofb_replay_read_priorities"):
         getattr(lib, name).restype = i32
     for name in ("ofb_trainer_create", "ofb_trainer_destroy", "ofb_trainer_fit", "ofb_trainer_forward",
-                 "ofb_trainer_td_targets", "ofb_trainer_get_weights", "ofb_trainer_get_grads"):
+                 "ofb_trainer_td_targets", "ofb_trainer_fit_weighted", "ofb_trainer_td_errors", "ofb_trainer_get_weights", "ofb_trainer_get_grads"):
         getattr(lib, name).restype = i32
     for name in ("ofb_policy_create", "ofb_policy_destroy", "ofb_policy_set_engine", "ofb_policy_forward",
                  "ofb_policy_write_actions", "ofb_policy_pack_image", "ofb_policy_debug_tap"):

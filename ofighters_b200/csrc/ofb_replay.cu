@@ -11,6 +11,11 @@
 #include "../../include/ofb_replay.h"
 
 #define OFB_REPLAY_TILE 2048          // candidates per block of the index kernels: 256 threads x 8
+struct PrioStats {                   // written by k_prio_scan for the draws of the same sample
+    double total;                    // sum of the valid masses
+    float mass_min;                  // smallest non-zero valid mass
+    int last_tile;                   // last tile with a non-zero sum
+};
 struct ofb_replay {
     const ofb_arenas *h;
     ArenaLayout lay;
@@ -28,6 +33,17 @@ struct ofb_replay {
     long long pushes;            // frames pushed so far
     int newest;                  // slot of the last push
     size_t bytes;
+    // prioritized replay: all NULL until ofb_replay_enable_priorities
+    float *mass;                 // [depth * count * P] sampling mass of each transition id
+    float *max_mass;             // [1] largest mass set so far (initially 1)
+    double *tile_sum;            // [n_tiles] sum of the valid masses of each tile
+    double *tile_prefix;         // [n_tiles] exclusive prefix of tile_sum
+    float *tile_min;             // [n_tiles] smallest non-zero valid mass of each tile
+    int32_t *tile_valid;         // [n_tiles] valid transitions with a non-zero mass in each tile
+    PrioStats *stats;            // [1]
+    float alpha, eps;
+    unsigned long long seed;
+    long long samples;           // prioritized samples drawn so far: the Philox counter
 };
 
 // ---------------------------------------------------------------- push: one warp per tracked arena
@@ -35,7 +51,7 @@ __global__ void __launch_bounds__(128)
 k_replay_push(const char *__restrict__ state, const ArenaLayout lay, long long first, long long count,
               const int32_t *__restrict__ ships, int P, char *__restrict__ ring, int slot, int prev, const int32_t *__restrict__ iaction_in,
               const int2 *__restrict__ xy_in, int32_t *__restrict__ act, int2 *__restrict__ xy, float *__restrict__ reward,
-              uint8_t *__restrict__ valid, uint8_t *__restrict__ done) {
+              uint8_t *__restrict__ valid, uint8_t *__restrict__ done, float *__restrict__ mass, const float *__restrict__ max_mass) {
     const long long a = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     const int lane = threadIdx.x & 31;
     if (a >= count) return;
@@ -61,6 +77,7 @@ k_replay_push(const char *__restrict__ state, const ArenaLayout lay, long long f
             valid[prev * cP + j] = (same_episode && (orec.x >> 31)) ? 1 : 0;
             reward[prev * cP + j] = (float)ship_unpack(rec).reward;
             done[prev * cP + j] = (rec.x >> 31) ? 0 : 1;
+            if (mass) mass[prev * cP + j] = *max_mass;    // prioritized replay: a new transition gets the largest mass
         }
         const long long o = (long long)slot * cP + j;
         valid[o] = 0;                                      // the newest frame has no successor yet
@@ -213,8 +230,202 @@ k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long 
     }
 }
 
+// ---------------------------------------------------------------- prioritized sampling: tile sums, scan, one block per draw
+// The candidates and their order are ofb_replay_index's; a candidate's mass counts only while it is valid, so invalid
+// transitions, the newest frame and slots overwritten by the ring have mass 0 and are never drawn.
+__device__ __forceinline__ float prio_mass(const uint8_t *valid, const float *mass, long long c, long long cP, long long n_cand,
+                                           int oldest, int depth) {
+    if (c >= n_cand) return 0.0f;
+    const long long id = replay_id(c, cP, oldest, depth);
+    return valid[id] ? mass[id] : 0.0f;
+}
+
+__global__ void __launch_bounds__(256)
+k_prio_tiles(const uint8_t *__restrict__ valid, const float *__restrict__ mass, long long cP, long long n_cand, int oldest, int depth,
+             double *__restrict__ tile_sum, float *__restrict__ tile_min, int32_t *__restrict__ tile_valid) {
+    __shared__ double s_sum[8];
+    __shared__ float s_min[8];
+    __shared__ int s_cnt[8];
+    const long long c0 = (long long)blockIdx.x * OFB_REPLAY_TILE + threadIdx.x * 8;
+    double s = 0.0;
+    float mn = INFINITY;
+    int k = 0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        const float m = prio_mass(valid, mass, c0 + i, cP, n_cand, oldest, depth);
+        if (m > 0.0f) { s += (double)m; mn = fminf(mn, m); k++; }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        s += __shfl_xor_sync(0xffffffffu, s, o);
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        k += __shfl_xor_sync(0xffffffffu, k, o);
+    }
+    if ((threadIdx.x & 31) == 0) { s_sum[threadIdx.x >> 5] = s; s_min[threadIdx.x >> 5] = mn; s_cnt[threadIdx.x >> 5] = k; }
+    __syncthreads();
+    if (threadIdx.x == 0) {                                // (s, mn, k) already hold warp 0's reduction
+        for (int w = 1; w < 8; w++) { s += s_sum[w]; mn = fminf(mn, s_min[w]); k += s_cnt[w]; }
+        tile_sum[blockIdx.x] = s;
+        tile_min[blockIdx.x] = mn;
+        tile_valid[blockIdx.x] = k;
+    }
+}
+
+// One block: exclusive fp64 prefix of the tile sums, the total, the smallest mass, the drawable count.  The prefix is made
+// exactly non-decreasing, which the draws' binary search and their order in b rely on: the per-thread chunk sums are scanned,
+// their running maximum M_t (exact) starts chunk t + 1, and chunk t's prefixes are clamped to M_t.  total = M_1023.
+__global__ void __launch_bounds__(1024)
+k_prio_scan(const double *__restrict__ tile_sum, const float *__restrict__ tile_min, const int32_t *__restrict__ tile_valid,
+            long long n_tiles, double *__restrict__ tile_prefix, PrioStats *__restrict__ stats, int32_t *__restrict__ n_valid_out) {
+    __shared__ double s_sum[1024];
+    __shared__ float s_min[32];
+    __shared__ int s_cnt[32], s_last[32];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const long long per = (n_tiles + 1023) / 1024;
+    const long long b0 = tid * per, b1 = min(n_tiles, b0 + per);
+    double s = 0.0;
+    float mn = INFINITY;
+    int k = 0, last = -1;
+    for (long long i = b0; i < b1; i++) {
+        const double v = tile_sum[i];
+        s += v;
+        mn = fminf(mn, tile_min[i]);
+        k += tile_valid[i];
+        if (v > 0.0) last = (int)i;
+    }
+    s_sum[tid] = s;
+    __syncthreads();
+    for (int o = 1; o < 1024; o <<= 1) {                   // Hillis-Steele inclusive scan of the per-thread sums
+        const double v = tid >= o ? s_sum[tid - o] : 0.0;
+        __syncthreads();
+        s_sum[tid] += v;
+        __syncthreads();
+    }
+    for (int o = 1; o < 1024; o <<= 1) {                   // its running maximum: exact, so non-decreasing
+        const double v = tid >= o ? s_sum[tid - o] : 0.0;
+        __syncthreads();
+        s_sum[tid] = fmax(s_sum[tid], v);
+        __syncthreads();
+    }
+    const double hi = s_sum[tid];
+    double run = tid > 0 ? s_sum[tid - 1] : 0.0;
+    for (long long i = b0; i < b1; i++) {
+        tile_prefix[i] = fmin(run, hi);
+        run += tile_sum[i];
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+        mn = fminf(mn, __shfl_xor_sync(0xffffffffu, mn, o));
+        k += __shfl_xor_sync(0xffffffffu, k, o);
+        last = max(last, __shfl_xor_sync(0xffffffffu, last, o));
+    }
+    if (lane == 0) { s_min[warp] = mn; s_cnt[warp] = k; s_last[warp] = last; }
+    __syncthreads();
+    if (tid == 0) {
+        for (int w = 1; w < 32; w++) { mn = fminf(mn, s_min[w]); k += s_cnt[w]; last = max(last, s_last[w]); }
+        stats->total = s_sum[1023];
+        stats->mass_min = mn;
+        stats->last_tile = last;
+        *n_valid_out = k;
+    }
+}
+
+// Draw b: u = (b + U) / B * total.  Thread 0 binary-searches the tile prefix, then the block scans that tile's masses in fp64
+// and takes the first candidate whose inclusive prefix exceeds u.  When rounding leaves u at or past the tile's (or the
+// memory's) sum, the last candidate of non-zero mass is taken instead: a zero mass is never drawn.  Every step is
+// non-decreasing in u, and u in b, so the draws of one sample are in age order.
+__global__ void __launch_bounds__(256)
+k_prio_draw(const uint8_t *__restrict__ valid, const float *__restrict__ mass, long long cP, long long n_cand, int oldest, int depth,
+            const double *__restrict__ tile_sum, const double *__restrict__ tile_prefix, const PrioStats *__restrict__ stats,
+            unsigned long long seed,
+            unsigned long long counter, float beta, int B, int32_t *__restrict__ ids_out, float *__restrict__ weight_out) {
+    __shared__ int s_tile, s_first, s_last;
+    __shared__ double s_r, s_warp[8];
+    const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const PrioStats st = *stats;
+    if (!(st.total > 0.0)) return;                         // no drawable transition: n_valid = 0
+    if (tid == 0) {
+        uint32_t c[4] = {(uint32_t)b, (uint32_t)counter, (uint32_t)(counter >> 32), 0x50524552u};
+        philox4x32_10(c, (uint32_t)seed, (uint32_t)(seed >> 32));
+        const double U = ((double)(c[0] >> 5) * 67108864.0 + (double)(c[1] >> 6)) * (1.0 / 9007199254740992.0);   // 53 bits, [0, 1)
+        const double u = ((double)b + U) / (double)B * st.total;
+        int lo = 0, hi = st.last_tile;                     // the last tile t <= last_tile with prefix[t] <= u
+        while (lo < hi) {
+            const int mid = (lo + hi + 1) >> 1;
+            if (tile_prefix[mid] <= u) lo = mid;
+            else hi = mid - 1;
+        }
+        double r = u - tile_prefix[lo];
+        if (tile_sum[lo] == 0.0) {                         // an empty tile whose prefix rounded below the next one's:
+            while (tile_sum[lo] == 0.0) lo++;              // the next tile with mass (last_tile at the latest), its first
+            r = -1.0;                                      // candidate of non-zero mass
+        }
+        s_tile = lo;
+        s_r = r;
+        s_first = 0x7fffffff;
+        s_last = -1;
+    }
+    __syncthreads();
+    const long long c0 = (long long)s_tile * OFB_REPLAY_TILE + tid * 8;
+    const double r = s_r;
+    double m[8], own = 0.0;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        m[i] = (double)prio_mass(valid, mass, c0 + i, cP, n_cand, oldest, depth);
+        own += m[i];
+    }
+    double incl = own;                                     // block exclusive scan of the per-thread sums
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const double v = __shfl_up_sync(0xffffffffu, incl, o);
+        if (lane >= o) incl += v;
+    }
+    if (lane == 31) s_warp[warp] = incl;
+    __syncthreads();
+    double run = incl - own;
+    for (int w = 0; w < warp; w++) run += s_warp[w];
+    int first = 0x7fffffff, last = -1;
+#pragma unroll
+    for (int i = 0; i < 8; i++) {
+        run += m[i];
+        if (m[i] > 0.0) {
+            last = (int)(c0 + i);
+            if (run > r && first == 0x7fffffff) first = (int)(c0 + i);
+        }
+    }
+    if (first != 0x7fffffff) atomicMin(&s_first, first);
+    if (last >= 0) atomicMax(&s_last, last);
+    __syncthreads();
+    if (tid == 0) {
+        const long long c = s_first != 0x7fffffff ? s_first : s_last;
+        const long long id = replay_id(c, cP, oldest, depth);
+        ids_out[b] = (int32_t)id;
+        // fp32 pow (the fp64 one spills), within a few ulp; mass >= mass_min makes w <= 1, kept so under that rounding
+        weight_out[b] = fminf(powf((float)((double)mass[id] / (double)st.mass_min), -beta), 1.0f);
+    }
+}
+
+__global__ void k_prio_update(const int32_t *__restrict__ ids, const float *__restrict__ td_act, const float *__restrict__ td_ptr, int B,
+                              long long n_ids, float alpha, float eps, float *__restrict__ mass, float *__restrict__ max_mass) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const long long id = ids[b];
+    if (id < 0 || id >= n_ids) return;
+    float m = (float)pow(fabs((double)td_act[b]) + fabs((double)td_ptr[b]) + (double)eps, (double)alpha);
+    if (!(m <= 3.402823466e38f)) m = 3.402823466e38f;     // a non-finite error must not poison the sampler's sums
+    mass[id] = m;
+    atomicMax(reinterpret_cast<int *>(max_mass), __float_as_int(m));   // masses are >= 0: their bits order like the values
+}
+
 // ---------------------------------------------------------------- C ABI
 static void replay_free(ofb_replay *r) {
+    cudaFree(r->mass);
+    cudaFree(r->max_mass);
+    cudaFree(r->tile_sum);
+    cudaFree(r->tile_prefix);
+    cudaFree(r->tile_min);
+    cudaFree(r->tile_valid);
+    cudaFree(r->stats);
     cudaFree(r->ring);
     cudaFree(r->act);
     cudaFree(r->xy);
@@ -309,7 +520,7 @@ extern "C" int ofb_replay_push(ofb_replay *r, const ofb_arenas *h, const int32_t
     const long long threads = r->count * 32;
     k_replay_push<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
         h->state, r->lay, r->first, r->count, r->ships, r->P, r->ring, slot, prev, iaction_dev,
-        reinterpret_cast<const int2 *>(xy_dev), r->act, r->xy, r->reward, r->valid, r->done);
+        reinterpret_cast<const int2 *>(xy_dev), r->act, r->xy, r->reward, r->valid, r->done, r->mass, r->max_mass);
     OFB_CUDA_CHECK(cudaGetLastError());
     r->newest = slot;
     r->pushes += 1;
@@ -349,5 +560,101 @@ extern "C" int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, in
         r->ring, r->lay, r->count, r->P, r->depth, r->ships, ids_dev, r->act, r->xy, r->reward, r->done, maps_obs_dev,
         vec_obs_dev, maps_next_dev, vec_next_dev, iaction_dev, pointer_dev, reward_dev, done_dev);
     OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+// ---------------------------------------------------------------- prioritized replay
+extern "C" int ofb_replay_enable_priorities(ofb_replay *r, const ofb_replay_prio_config *cfg) {
+    if (!r || !cfg) { ofb_set_error("ofb_replay_enable_priorities: null argument"); return OFB_E_ARG; }
+    if (r->mass) { ofb_set_error("ofb_replay_enable_priorities: priorities are already enabled"); return OFB_E_ARG; }
+    if (r->pushes > 0) { ofb_set_error("ofb_replay_enable_priorities: only before the first push"); return OFB_E_ARG; }
+    if (!(cfg->alpha >= 0.0f && cfg->alpha <= 3.402823466e38f) || !(cfg->eps >= 0.0f && cfg->eps <= 3.402823466e38f)) {
+        ofb_set_error("ofb_replay_enable_priorities: need finite alpha >= 0 and eps >= 0 (got %g, %g)", cfg->alpha, cfg->eps);
+        return OFB_E_ARG;
+    }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    const size_t nt = (size_t)r->depth * r->count * r->P, tiles = (size_t)r->n_tiles;
+    const size_t bytes = nt * sizeof(float) + sizeof(float) + tiles * (2 * sizeof(double) + sizeof(float) + sizeof(int32_t)) +
+                         sizeof(PrioStats);
+    if (cudaMalloc(&r->mass, nt * sizeof(float)) != cudaSuccess || cudaMalloc(&r->max_mass, sizeof(float)) != cudaSuccess ||
+        cudaMalloc(&r->tile_sum, tiles * sizeof(double)) != cudaSuccess ||
+        cudaMalloc(&r->tile_prefix, tiles * sizeof(double)) != cudaSuccess || cudaMalloc(&r->tile_min, tiles * sizeof(float)) != cudaSuccess ||
+        cudaMalloc(&r->tile_valid, tiles * sizeof(int32_t)) != cudaSuccess || cudaMalloc(&r->stats, sizeof(PrioStats)) != cudaSuccess) {
+        cudaGetLastError();
+        ofb_set_error("ofb_replay_enable_priorities: cudaMalloc of %zu bytes failed", bytes);
+        cudaFree(r->mass); cudaFree(r->max_mass); cudaFree(r->tile_sum); cudaFree(r->tile_prefix); cudaFree(r->tile_min);
+        cudaFree(r->tile_valid); cudaFree(r->stats);
+        r->mass = r->max_mass = r->tile_min = nullptr;
+        r->tile_sum = r->tile_prefix = nullptr;
+        r->tile_valid = nullptr;
+        r->stats = nullptr;
+        return OFB_E_NOMEM;
+    }
+    const float one = 1.0f;
+    OFB_CUDA_CHECK(cudaMemset(r->mass, 0, nt * sizeof(float)));
+    OFB_CUDA_CHECK(cudaMemset(r->stats, 0, sizeof(PrioStats)));
+    OFB_CUDA_CHECK(cudaMemcpy(r->max_mass, &one, sizeof(float), cudaMemcpyHostToDevice));
+    r->alpha = cfg->alpha;
+    r->eps = cfg->eps;
+    r->seed = cfg->seed;
+    r->samples = 0;
+    r->bytes += bytes;
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_sample_prioritized(ofb_replay *r, int32_t batch, float beta, int32_t *ids_out, float *weight_out,
+                                             int32_t *n_valid_out, void *stream) {
+    if (!r || !ids_out || !weight_out || !n_valid_out) { ofb_set_error("ofb_replay_sample_prioritized: null argument"); return OFB_E_ARG; }
+    if (!r->mass) { ofb_set_error("ofb_replay_sample_prioritized: priorities are not enabled"); return OFB_E_ARG; }
+    if (batch < 1 || !(beta >= 0.0f && beta <= 3.402823466e38f)) {
+        ofb_set_error("ofb_replay_sample_prioritized: need batch >= 1 and finite beta >= 0 (got %d, %g)", batch, beta);
+        return OFB_E_ARG;
+    }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const long long filled = r->pushes < r->depth ? r->pushes : r->depth;
+    const long long nf = filled > 0 ? filled - 1 : 0;
+    const long long cP = r->count * r->P, n_cand = nf * cP;
+    if (n_cand == 0) {
+        OFB_CUDA_CHECK(cudaMemsetAsync(n_valid_out, 0, sizeof(int32_t), st));
+        return OFB_OK;
+    }
+    const int oldest = (int)((r->newest - nf + r->depth) % r->depth);
+    const long long tiles = (n_cand + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
+    k_prio_tiles<<<(unsigned)tiles, 256, 0, st>>>(r->valid, r->mass, cP, n_cand, oldest, r->depth, r->tile_sum, r->tile_min,
+                                                 r->tile_valid);
+    k_prio_scan<<<1, 1024, 0, st>>>(r->tile_sum, r->tile_min, r->tile_valid, tiles, r->tile_prefix, r->stats, n_valid_out);
+    k_prio_draw<<<(unsigned)batch, 256, 0, st>>>(r->valid, r->mass, cP, n_cand, oldest, r->depth, r->tile_sum, r->tile_prefix,
+                                                 r->stats, r->seed,
+                                                 (unsigned long long)r->samples, beta, batch, ids_out, weight_out);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    r->samples += 1;
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_update_priorities(ofb_replay *r, const int32_t *ids_dev, const float *td_act_dev, const float *td_ptr_dev,
+                                            int32_t batch, void *stream) {
+    if (!r || !ids_dev || !td_act_dev || !td_ptr_dev || batch < 1) {
+        ofb_set_error("ofb_replay_update_priorities: bad argument");
+        return OFB_E_ARG;
+    }
+    if (!r->mass) { ofb_set_error("ofb_replay_update_priorities: priorities are not enabled"); return OFB_E_ARG; }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    k_prio_update<<<(unsigned)((batch + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
+        ids_dev, td_act_dev, td_ptr_dev, batch, (long long)r->depth * r->count * r->P, r->alpha, r->eps, r->mass, r->max_mass);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_read_priorities(const ofb_replay *r, float *mass_dev, float *max_mass_dev, double *last_total_dev,
+                                          void *stream) {
+    if (!r) { ofb_set_error("ofb_replay_read_priorities: null argument"); return OFB_E_ARG; }
+    if (!r->mass) { ofb_set_error("ofb_replay_read_priorities: priorities are not enabled"); return OFB_E_ARG; }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t nt = (size_t)r->depth * r->count * r->P;
+    if (mass_dev) OFB_CUDA_CHECK(cudaMemcpyAsync(mass_dev, r->mass, nt * sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (max_mass_dev) OFB_CUDA_CHECK(cudaMemcpyAsync(max_mass_dev, r->max_mass, sizeof(float), cudaMemcpyDeviceToDevice, st));
+    if (last_total_dev) OFB_CUDA_CHECK(cudaMemcpyAsync(last_total_dev, &r->stats->total, sizeof(double), cudaMemcpyDeviceToDevice, st));
     return OFB_OK;
 }

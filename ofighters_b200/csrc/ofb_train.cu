@@ -343,6 +343,19 @@ __global__ void k_tr_mse(const float *__restrict__ pred, const float *__restrict
     }
     block_accumulate<1>(v, loss_acc, 1);
 }
+// the same with per-sample weights w[b] over `per` elements each: dpred = 2 w_b (pred - target) / n,
+// loss_acc += sum w_b (pred - target)^2  (so loss_acc / n = (1/B) sum_b w_b mse_b)
+__global__ void k_tr_mse_weighted(const float *__restrict__ pred, const float *__restrict__ target, long long n, long long per,
+                                  const float *__restrict__ w, float *__restrict__ dpred, double *__restrict__ loss_acc) {
+    double v[1] = {0.0};
+    const float scale = 2.0f / (float)n;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const float d = pred[i] - target[i], wb = w[i / per];
+        dpred[i] = (d * scale) * wb;
+        v[0] += (double)wb * ((double)d * (double)d);
+    }
+    block_accumulate<1>(v, loss_acc, 1);
+}
 __global__ void k_tr_loss_out(const double *__restrict__ loss_acc, long long n_act, long long n_ptr, float *__restrict__ out) {
     const double la = loss_acc[0] / (double)n_act, lp = loss_acc[1] / (double)n_ptr;
     out[0] = (float)(la + lp); out[1] = (float)la; out[2] = (float)lp;
@@ -700,6 +713,31 @@ __global__ void k_tr_td_targets(const float *__restrict__ act_obs, const float *
     }
 }
 
+// target - prediction at the two entries k_tr_td_targets overwrites, each target by k_tr_td_targets' own fp32 expression (the
+// maximum is order-independent), so td = t_target - prediction exactly.  One block per sample.
+__global__ void k_tr_td_errors(const float *__restrict__ act_obs, const float *__restrict__ ptr_obs, const float *__restrict__ act_next,
+                               const float *__restrict__ ptr_next, const int32_t *__restrict__ iaction, const int32_t *__restrict__ pointer,
+                               const float *__restrict__ reward, const uint8_t *__restrict__ done, float gamma, float *__restrict__ td_act,
+                               float *__restrict__ td_ptr) {
+    const long long b = blockIdx.x;
+    const int n = IMG * IMG;
+    __shared__ float red[32];
+    float mx = -INFINITY;
+    for (int i = threadIdx.x; i < n; i += blockDim.x) mx = fmaxf(mx, ptr_next[b * n + i]);
+    for (int o = 16; o > 0; o >>= 1) mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+    if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = mx;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int wv = 1; wv < (int)((blockDim.x + 31) >> 5); wv++) mx = fmaxf(mx, red[wv]);
+        const float keep = done[b] ? 0.0f : 1.0f, r = reward[b];
+        const float ma = fmaxf(act_next[b * 2], act_next[b * 2 + 1]);
+        const float ta = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, ma), keep));
+        const float tp = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, mx), keep));
+        td_act[b] = __fsub_rn(ta, act_obs[b * 2 + iaction[b]]);
+        td_ptr[b] = __fsub_rn(tp, ptr_obs[b * n + (long long)pointer[b * 2] * IMG + pointer[b * 2 + 1]]);
+    }
+}
+
 // ---------------------------------------------------------------------------------------------- host side
 static inline unsigned blocks_for(long long n, int threads, long long cap = 148 * 16) {
     long long b = (n + threads - 1) / threads;
@@ -891,11 +929,10 @@ extern "C" int ofb_trainer_forward(ofb_trainer *t, const uint32_t *maps, const f
     return OFB_OK;
 }
 
-extern "C" int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act, const float *target_ptr,
-                               int B, float *loss_dev, void *stream) {
-    int rc = check_batch(t, B, "ofb_trainer_fit");
-    if (rc != OFB_OK) return rc;
-    if (!maps || !vec || !target_act || !target_ptr) { ofb_set_error("ofb_trainer_fit: null argument"); return OFB_E_ARG; }
+// one Adam step; sample_weight == NULL: today's unweighted loss, with the kernels of ofb_trainer_fit unchanged
+static int fit_impl(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act, const float *target_ptr,
+                    const float *sample_weight, int B, float *loss_dev, void *stream) {
+    int rc;
     TR_CHECK(cudaSetDevice(t->device));
     cudaStream_t st = (cudaStream_t)stream;
     const Table &T = t->tab;
@@ -909,8 +946,14 @@ extern "C" int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps, const float
 
     // ---- losses: mse(output1) + mse(output2), each a mean over all of its elements
     const long long n_act = (long long)B * 2, n_ptr = (long long)B * IMG * IMG;
-    k_tr_mse<<<1, 64, 0, st>>>(t->act, target_act, n_act, t->dact, t->loss_acc);
-    k_tr_mse<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, t->g0, t->loss_acc + 1);
+    if (!sample_weight) {
+        k_tr_mse<<<1, 64, 0, st>>>(t->act, target_act, n_act, t->dact, t->loss_acc);
+        k_tr_mse<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, t->g0, t->loss_acc + 1);
+    } else {
+        k_tr_mse_weighted<<<1, 64, 0, st>>>(t->act, target_act, n_act, 2, sample_weight, t->dact, t->loss_acc);
+        k_tr_mse_weighted<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, IMG * IMG, sample_weight, t->g0,
+                                                                          t->loss_acc + 1);
+    }
     if (loss_dev) k_tr_loss_out<<<1, 1, 0, st>>>(t->loss_acc, n_act, n_ptr, loss_dev);
 
     // ---- pointer head, top down.  g0 holds the gradient w.r.t. the stage's conv output, g1 w.r.t. its (upsampled) input.
@@ -978,6 +1021,38 @@ extern "C" int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps, const float
     const float lr_t = (float)((double)t->cfg.lr * sqrt(1.0 - pow(b2, (double)t->steps)) / (1.0 - pow(b1, (double)t->steps)));
     k_tr_adam<<<blocks_for(T.total, 256, 1 << 20), 256, 0, st>>>(P, G, t->adam_m, t->adam_v, t->trainable, T.total, lr_t, t->cfg.beta1,
                                                                   t->cfg.beta2, t->cfg.adam_eps);
+    TR_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+extern "C" int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act, const float *target_ptr,
+                               int B, float *loss_dev, void *stream) {
+    int rc = check_batch(t, B, "ofb_trainer_fit");
+    if (rc != OFB_OK) return rc;
+    if (!maps || !vec || !target_act || !target_ptr) { ofb_set_error("ofb_trainer_fit: null argument"); return OFB_E_ARG; }
+    return fit_impl(t, maps, vec, target_act, target_ptr, nullptr, B, loss_dev, stream);
+}
+
+extern "C" int ofb_trainer_fit_weighted(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act,
+                                        const float *target_ptr, const float *sample_weight, int B, float *loss_dev, void *stream) {
+    int rc = check_batch(t, B, "ofb_trainer_fit_weighted");
+    if (rc != OFB_OK) return rc;
+    if (!maps || !vec || !target_act || !target_ptr || !sample_weight) {
+        ofb_set_error("ofb_trainer_fit_weighted: null argument");
+        return OFB_E_ARG;
+    }
+    return fit_impl(t, maps, vec, target_act, target_ptr, sample_weight, B, loss_dev, stream);
+}
+
+extern "C" int ofb_trainer_td_errors(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
+                                     const int32_t *iaction, const int32_t *pointer, const float *reward, const uint8_t *done, float gamma,
+                                     int B, float *td_act, float *td_ptr, void *stream) {
+    if (!act_obs || !ptr_obs || !act_next || !ptr_next || !iaction || !pointer || !reward || !done || !td_act || !td_ptr || B < 1) {
+        ofb_set_error("ofb_trainer_td_errors: bad argument");
+        return OFB_E_ARG;
+    }
+    k_tr_td_errors<<<B, 256, 0, (cudaStream_t)stream>>>(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma, td_act,
+                                                        td_ptr);
     TR_CHECK(cudaGetLastError());
     return OFB_OK;
 }

@@ -18,6 +18,9 @@ that is alive at t, none across a restart (masked restarts included), a death on
 ``sample``.  The order of the transitions -- oldest frame first, then arena, then ship -- is the order in which ``QLearner``
 appends to ``trainer.memory``, and ``sample`` draws ``random.sample(range(len), batch_size)`` with Python's ``random`` as
 ``Trainer.replay`` does on its deque, so the same ``random`` state picks the same minibatch.
+
+``PrioritizedReplayMemory`` adds prioritized replay on the device: masses from the TD errors, a stratified proportional sampler
+and importance weights for ``TrainerB200.fit(..., sample_weight=...)``.
 """
 import ctypes as C
 import random
@@ -133,7 +136,10 @@ class DeviceReplayMemory:
             raise Exception("gather of no transition")
         if int(pos.min()) < 0 or int(pos.max()) >= n:
             raise Exception("Invalid positions : the memory holds {} transitions.".format(n))
-        ids = self._ids.index_select(0, pos.to(self.device)).contiguous()
+        return self._gather_ids(self._ids.index_select(0, pos.to(self.device)).contiguous())
+
+    def _gather_ids(self, ids):
+        """``gather`` of transition ids (int32 [B] on the device, valid until the next push)."""
         B = ids.numel()
         words = self.bg.config.width * self.bg.config.height // 32
         dev = self.device
@@ -158,3 +164,95 @@ class DeviceReplayMemory:
         if n < 1:
             raise Exception("sample on an empty replay memory")
         return self.gather(random.sample(range(n), batch_size))
+
+
+class EmptyReplayMemory(Exception):
+    """A prioritized sample found no transition to draw."""
+
+
+class PrioritizedReplayMemory(DeviceReplayMemory):
+    """``DeviceReplayMemory`` with prioritized replay (Schaul et al. 2016, proportional variant), on the device.
+
+    Every transition carries a sampling mass, ``(|td_act| + |td_ptr| + eps) ** alpha`` from the TD errors of its last replay,
+    or the largest mass set so far when it enters the memory, so that a new transition is likely drawn at least once.
+    ``sample_prioritized`` draws a stratified minibatch in proportion to the masses with the importance weights that undo
+    the bias, ``update_priorities`` writes the new errors back.  ``TrainerB200.replay(..., memory=this, beta=...)`` runs the
+    whole sequence.
+
+        memory = PrioritizedReplayMemory(bg, depth=16, alpha=0.6)
+        ...                                           # push as for DeviceReplayMemory
+        trainer.replay(trainer.batch_size, memory=memory, beta=0.4)
+
+    The sampler's random stream is Philox keyed by ``seed`` and the number of samples drawn, so a run is reproducible."""
+
+    def __init__(self, bg, depth=16, track=None, ships=None, alpha=0.6, eps=1e-6, seed=0):
+        alpha, eps = float(alpha), float(eps)
+        if not (0.0 <= alpha < float("inf")) or not (0.0 <= eps < float("inf")):
+            raise Exception("Invalid priorities : need finite alpha >= 0 and eps >= 0, got alpha={} eps={}.".format(alpha, eps))
+        super().__init__(bg, depth=depth, track=track, ships=ships)
+        cfg = _lib.OfbReplayPrioConfig(alpha=alpha, eps=eps, seed=int(seed) & (2 ** 64 - 1))
+        with torch.cuda.device(self.device):
+            _lib.check(self._lib.ofb_replay_enable_priorities(self._h, C.byref(cfg)))
+        self.alpha, self.eps, self.seed = alpha, eps, int(seed)
+        self._n_transitions = self.depth * self.track * len(self.ships)
+        self._n_valid = torch.zeros(1, dtype=torch.int32, device=self.device)
+        self._sampled = None                             # (frames at the last sample, its ids)
+
+    def sample_prioritized(self, batch_size, beta):
+        """Draw ``batch_size`` transitions in proportion to their masses -> ``gather``'s namespace plus ``ids`` (int32 [B],
+        for ``update_priorities``) and ``weight`` (float32 [B], the importance weights (mass / min mass) ** -beta <= 1).
+        Reads the number of drawable transitions: one host synchronisation.  Raises ``EmptyReplayMemory`` when there is
+        none."""
+        B, beta = int(batch_size), float(beta)
+        if B < 1:
+            raise Exception("Invalid batch : {} samples.".format(B))
+        if not (0.0 <= beta < float("inf")):
+            raise Exception("Invalid beta {} : expected a finite value >= 0.".format(beta))
+        ids = torch.empty((B,), dtype=torch.int32, device=self.device)
+        weight = torch.empty((B,), dtype=torch.float32, device=self.device)
+        _lib.check(self._lib.ofb_replay_sample_prioritized(self._h, B, beta, _ptr(ids), _ptr(weight), _ptr(self._n_valid),
+                                                           self._stream()))
+        self.launch_count += 3
+        if int(self._n_valid.item()) < 1:
+            raise EmptyReplayMemory("sample on an empty replay memory")
+        out = self._gather_ids(ids)
+        out.ids, out.weight = ids, weight
+        self._sampled = (self.frames, ids)
+        return out
+
+    def update_priorities(self, ids, td_act, td_ptr):
+        """Set the masses of the transitions ``ids`` (int32 [B] from ``sample_prioritized``) from their TD errors
+        ``td_act`` / ``td_ptr`` (float32 [B], ``TrainerB200.td_errors``) and raise the largest mass.  The ids must come
+        from a sample taken since the last push; ids other than that sample's own tensor are range-checked, which
+        synchronises the host."""
+        if self._sampled is None or self._sampled[0] != self.frames:
+            raise Exception("Invalid ids : a push happened since the sample they come from.")
+        B = ids.numel() if isinstance(ids, torch.Tensor) else 0
+        for name, t, dt in (("ids", ids, torch.int32), ("td_act", td_act, torch.float32), ("td_ptr", td_ptr, torch.float32)):
+            if not isinstance(t, torch.Tensor) or t.dtype != dt or t.device != self.device or tuple(t.shape) != (B,) or \
+                    not t.is_contiguous():
+                raise Exception("Invalid {} : expected a contiguous {} tensor of shape ({},) on {}.".format(name, dt, B, self.device))
+        if B < 1:
+            raise Exception("Invalid ids : no transition.")
+        if ids is not self._sampled[1] and (int(ids.min()) < 0 or int(ids.max()) >= self._n_transitions):
+            raise Exception("Invalid ids : outside [0, {}).".format(self._n_transitions))
+        _lib.check(self._lib.ofb_replay_update_priorities(self._h, _ptr(ids), _ptr(td_act), _ptr(td_ptr), B, self._stream()))
+        self.launch_count += 1
+
+    def masses(self):
+        """Device copy of the sampling masses, float32 [depth * track * P] indexed by transition id (slot, arena, ship)."""
+        out = torch.empty((self._n_transitions,), dtype=torch.float32, device=self.device)
+        _lib.check(self._lib.ofb_replay_read_priorities(self._h, _ptr(out), None, None, self._stream()))
+        return out
+
+    def max_mass(self):
+        """Device copy of the largest mass set so far (float32 [1]); new transitions enter with it."""
+        out = torch.empty((1,), dtype=torch.float32, device=self.device)
+        _lib.check(self._lib.ofb_replay_read_priorities(self._h, None, _ptr(out), None, self._stream()))
+        return out
+
+    def last_total(self):
+        """Device copy of the fp64 total mass the last ``sample_prioritized`` drew from (float64 [1])."""
+        out = torch.empty((1,), dtype=torch.float64, device=self.device)
+        _lib.check(self._lib.ofb_replay_read_priorities(self._h, None, None, _ptr(out), self._stream()))
+        return out

@@ -28,6 +28,7 @@ import torch
 from . import _lib
 from .epsilon import Epsilon_cos, Epsilon_decay, EpsilonSchedule  # noqa: F401  (re-exported: Trainer(epsilon=Epsilon_cos(...)))
 from .policy import WEIGHT_SPEC, PolicyB200, keras_default_weights
+from .replay import EmptyReplayMemory, PrioritizedReplayMemory
 
 
 def flatten_weights(weights):
@@ -160,16 +161,25 @@ class TrainerB200:
             raise Exception("Invalid vector input : expected shape {} but got shape {}.".format((B, 8), tuple(vec.shape)))
         return B, vec
 
-    def fit(self, maps_bits, vec, target_act, target_ptr, sync_model=True):
+    def fit(self, maps_bits, vec, target_act, target_ptr, sync_model=True, sample_weight=None):
         """``model.fit(x=[img, vec], y=[act, ptr], epochs=1, batch_size=B)`` (:286): one Adam step.  Returns the loss
-        tensor (total, mse(output1), mse(output2)) of the batch before the update (device, float32 [3])."""
+        tensor (total, mse(output1), mse(output2)) of the batch before the update (device, float32 [3]).
+        ``sample_weight``: float [B] of weights >= 0 -- ``model.fit(..., sample_weight=w)``: each head's loss becomes
+        (1/B) sum_b w_b mse_b, and the returned losses are the weighted ones (include/ofb_train.h)."""
         B, vec = self._check_batch(maps_bits, vec)
         target_act = target_act.to(device=self.device, dtype=torch.float32).contiguous()
         target_ptr = target_ptr.to(device=self.device, dtype=torch.float32).contiguous()
         if tuple(target_act.shape) != (B, 2) or target_ptr.numel() != B * 160000:
             raise Exception("Invalid targets : expected shapes {} and {}.".format((B, 2), (B, 400, 400, 1)))
-        _lib.check(self._lib.ofb_trainer_fit(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr), B,
-                                             _ptr(self._loss), self._stream()))
+        if sample_weight is None:
+            _lib.check(self._lib.ofb_trainer_fit(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr), B,
+                                                 _ptr(self._loss), self._stream()))
+        else:
+            sample_weight = torch.as_tensor(sample_weight).to(device=self.device, dtype=torch.float32).contiguous()
+            if tuple(sample_weight.shape) != (B,):
+                raise Exception("Invalid sample_weight : expected shape {} but got shape {}.".format((B,), tuple(sample_weight.shape)))
+            _lib.check(self._lib.ofb_trainer_fit_weighted(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr),
+                                                          _ptr(sample_weight), B, _ptr(self._loss), self._stream()))
         self.launch_count += self.KERNELS_PER_FIT
         loss = self._loss.clone()
         if sync_model:
@@ -214,11 +224,28 @@ class TrainerB200:
         """:237-238.  ``state`` / ``next_state`` = (maps_bits int32 [2,5000], vec float32 [8]) device tensors."""
         self.memory.append([state, iaction, ipointer, reward, next_state, done])
 
-    def replay(self, batch_size, memory=None):
+    def td_errors(self, act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done):
+        """Signed TD errors target - prediction at the entries ``replay``'s targets overwrite, with the targets' own fp32
+        arithmetic: (td_act, td_ptr) float32 [B] on the device.  Inputs as ``ofb_trainer_td_targets`` takes them."""
+        B = act_obs.shape[0]
+        td_act = torch.empty((B,), dtype=torch.float32, device=self.device)
+        td_ptr = torch.empty((B,), dtype=torch.float32, device=self.device)
+        _lib.check(self._lib.ofb_trainer_td_errors(_ptr(act_obs), _ptr(ptr_obs), _ptr(act_next), _ptr(ptr_next), _ptr(iaction),
+                                                   _ptr(pointer), _ptr(reward), _ptr(done), float(self.gamma), B, _ptr(td_act),
+                                                   _ptr(td_ptr), self._stream()))
+        self.launch_count += 1
+        return td_act, td_ptr
+
+    def replay(self, batch_size, memory=None, beta=1.0):
         """:240-287.  Targets from predictions on obs and next_obs; like the reference, the fitted INPUTS are the
         next observations (``inputs1[i] = img_input`` is evaluated after img_input was rebuilt from next_obs, :281-282).
         ``memory``: a ``replay.DeviceReplayMemory`` to draw the minibatch from instead of ``self.memory`` (same
-        ``random.sample`` draw over its transitions in age order)."""
+        ``random.sample`` draw over its transitions in age order).  With a ``replay.PrioritizedReplayMemory`` the minibatch
+        is drawn in proportion to the priorities, the TD errors of the predictions set the drawn transitions' new
+        priorities, and the fit weighs each sample by its importance weight, annealed by ``beta`` (ignored otherwise); the
+        History then also reports ``td_error``, the batch mean of |td_act| + |td_ptr|."""
+        if isinstance(memory, PrioritizedReplayMemory):
+            return self._replay_prioritized(batch_size, memory, beta)
         dev = self.device
         if memory is None:
             batch_size = min(batch_size, len(self.memory))
@@ -253,6 +280,25 @@ class TrainerB200:
         loss = self.fit(maps_n, vec_n, act_o, ptr_o)
         host = loss.cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]]})
+
+    def _replay_prioritized(self, batch_size, memory, beta):
+        if memory.device != self.device:
+            raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, self.device))
+        batch_size = int(batch_size)
+        if batch_size < 1 or batch_size > self.max_batch:
+            raise Exception("Invalid batch : {} samples but the trainer was sized for {}.".format(batch_size, self.max_batch))
+        mb = memory.sample_prioritized(batch_size, beta)
+        act_o, ptr_o = self.predict(mb.maps_obs, mb.vec_obs)
+        act_n, ptr_n = self.predict(mb.maps_next, mb.vec_next)
+        args = [_ptr(t) for t in (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)]
+        td_act, td_ptr = self.td_errors(act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
+        memory.update_priorities(mb.ids, td_act, td_ptr)
+        _lib.check(self._lib.ofb_trainer_td_targets(*args, float(self.gamma), batch_size, _ptr(act_o), _ptr(ptr_o), self._stream()))
+        self.launch_count += 1
+        loss = self.fit(mb.maps_next, mb.vec_next, act_o, ptr_o, sample_weight=mb.weight)
+        host = torch.cat([loss, (td_act.abs() + td_ptr.abs()).mean().reshape(1)]).cpu().tolist()
+        return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]],
+                                        "td_error": [host[3]]})
 
 
 def len_flat():
@@ -379,9 +425,14 @@ class BatchedQLearner:
       * epsilon advances once per frame, not once per decision of bot 1 (which stops at its death);
       * no host synchronisation on frames without a replay.
 
-    ``actor``: the inference engine that drives the arenas (default: the trainer's own ``model``, which every fit refreshes)."""
+    ``actor``: the inference engine that drives the arenas (default: the trainer's own ``model``, which every fit refreshes).
 
-    def __init__(self, trainer, memory, replay_every=50, collecting_steps=20, snapshot=50, actor=None, snapshot_folder="networks"):
+    With a ``replay.PrioritizedReplayMemory`` each replay is prioritized, with the importance-sampling exponent annealed
+    linearly from ``beta0`` to 1 over ``beta_frames`` frames: beta = min(1, beta0 + (1 - beta0) * total_steps / beta_frames)
+    (``betas`` logs the value of every replay).  With a uniform memory ``beta0`` and ``beta_frames`` play no part."""
+
+    def __init__(self, trainer, memory, replay_every=50, collecting_steps=20, snapshot=50, actor=None, snapshot_folder="networks",
+                 beta0=0.4, beta_frames=100_000):
         if memory.device != trainer.device:
             raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, trainer.device))
         self.trainer = trainer
@@ -397,6 +448,16 @@ class BatchedQLearner:
         self.losses = []
         self.epsilons = []
         self.saved = []
+        self.prioritized = isinstance(memory, PrioritizedReplayMemory)
+        self.beta0, self.beta_frames = float(beta0), int(beta_frames)
+        if self.prioritized and (not 0.0 <= self.beta0 <= 1.0 or self.beta_frames < 1):
+            raise Exception("Invalid beta schedule : need 0 <= beta0 <= 1 and beta_frames >= 1.")
+        self.betas = []
+
+    @property
+    def beta(self):
+        """The importance-sampling exponent of a replay at this frame (prioritized memory)."""
+        return min(1.0, self.beta0 + (1.0 - self.beta0) * self.total_steps / self.beta_frames)
 
     @property
     def collecting(self):
@@ -421,7 +482,16 @@ class BatchedQLearner:
         if not collecting:
             self.trainer.decay_epsilon()
         replayed = False
-        if self.total_steps % self.replay_every == 0 and len(self.memory) > 0:
+        if self.total_steps % self.replay_every == 0 and self.prioritized:
+            try:                                          # the sample reads whether there is a transition to draw
+                h = self.trainer.replay(self.trainer.batch_size, memory=self.memory, beta=self.beta)
+            except EmptyReplayMemory:
+                h = None
+            if h is not None:
+                self.losses.append(h.history["loss"][0])
+                self.betas.append(self.beta)
+                replayed = True
+        elif self.total_steps % self.replay_every == 0 and len(self.memory) > 0:
             h = self.trainer.replay(self.trainer.batch_size, memory=self.memory)
             self.losses.append(h.history["loss"][0])
             replayed = True
