@@ -17,7 +17,7 @@
  * Conventions are those of ofb.h.  The handle owns the ring of `depth` frame slots (64-bit addressed: depth x count x
  * ofb_state_stride bytes) and its per-transition fields, all allocated at create time; push, index and gather allocate
  * nothing and never synchronise the host.  A ring of depth D holds the transitions of the last D-1 pushed frames: the
- * newest slot has no successor yet.
+ * newest slot has no successor yet (D - n frames for an n-step memory, ofb_replay_set_n_step).
  *
  * Opt-in prioritized replay (ofb_replay_enable_priorities) adds a sampling mass per transition, a device sampler that
  * draws in proportion to it over the same candidates as ofb_replay_index, and the update of the masses from TD errors.
@@ -68,10 +68,37 @@ int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, int32_t batch
                       uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev, int32_t *pointer_dev,
                       float *reward_dev, uint8_t *done_dev, void *stream);
 
+/* ---- N-step returns (Sutton 1988; Hessel et al. 2018).
+ * An n-step memory keeps the same one-step fields per frame t -- valid1[t] (alive at t, same episode at t and t+1),
+ * r[t] (the pending reward at t+1), done1[t] (dead at t+1) -- and builds the target R + gamma^k max Q(s_{t+k}) when it gathers.
+ * Transition (t, a, p) exists iff valid1[t] and t <= T - n (T = the newest frame), so a ring of depth D holds the transitions of
+ * the frames [T - D + 1, T - n].  Its window of k frames walks j = 0, 1, ...:
+ *   - done1[t+j]:          k = j + 1, done = 1 (a death: no bootstrap);
+ *   - else j + 1 = n:      k = n, done = 0;
+ *   - else !valid1[t+j+1]: k = j + 1, done = 0 (the episode ends after frame t+j+1 through a restart, full or masked: a
+ *                          time-limit truncation, so the target bootstraps from s_{t+j+1}, the episode's last observation).
+ * Gathered: obs = s_t, next = s_{t+k}, the action of frame t, steps = k, the return R and discount = gamma^k, in fp32 without
+ * fma: R = r[t+k-1], then R = r[t+j] + gamma * R for j = k-2 .. 0; discount = k - 1 products starting from gamma.  With
+ * priorities, frame T - n gets the largest mass at the push of T, the push that makes it a candidate.
+ * For n = 1 every rule above is the one-step memory's. */
+
+/* Make the memory's transitions n-step, 1 <= n <= depth - 1 (default 1).  Only before the first push; in either order with
+ * ofb_replay_enable_priorities. */
+int ofb_replay_set_n_step(ofb_replay *r, int32_t n);
+
+/* ofb_replay_gather for n-step transitions, with the discount gamma: maps / vec / iaction / pointer as there (next = s_{t+k}),
+ * return_out float [B] = R, done_out uint8 [B], discount_out float [B] = gamma^k, steps_out int32 [B] = k; any output may be
+ * NULL.  The targets are ofb_trainer_td_targets_discounted's.  On a one-step memory it equals ofb_replay_gather with
+ * discount = gamma and steps = 1; ofb_replay_gather refuses an n-step memory (its reward, done and next are one-step). */
+int ofb_replay_gather_nstep(const ofb_replay *r, const int32_t *ids_dev, int32_t batch, float gamma, uint32_t *maps_obs_dev,
+                            float *vec_obs_dev, uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev,
+                            int32_t *pointer_dev, float *return_dev, uint8_t *done_dev, float *discount_dev, int32_t *steps_dev,
+                            void *stream);
+
 /* ---- Prioritized replay (Schaul et al. 2016, proportional variant).
  * Every transition id carries a sampling mass; a transition is drawn with probability mass / (sum of the valid masses).
  * The mass is (|td_act| + |td_ptr| + eps)^alpha, the TD errors of ofb_trainer_td_errors (both heads regress on the same
- * return r + gamma * max).  A transition gets the largest mass set so far (initially 1) when it becomes valid, so a new
+ * return r + gamma * max).  A transition gets the largest mass set so far (initially 1) when it becomes a candidate, so a new
  * transition is likely drawn at least once. */
 typedef struct ofb_replay_prio_config {
     float alpha;          /* >= 0; 0 = uniform */

@@ -99,6 +99,18 @@ int ofb_trainer_td_errors(const float *act_obs_dev, const float *ptr_obs_dev, co
                           const float *reward_dev, const uint8_t *done_dev, float gamma, int batch, float *td_act_dev,
                           float *td_ptr_dev, void *stream);
 
+/* ofb_trainer_td_targets / ofb_trainer_td_errors with a discount per sample in place of gamma (n-step returns,
+ * ofb_replay_gather_nstep): the overwritten entries become  r[b] + (discount[b] * max) * !done[b],  in the same rounding
+ * order, so discount[b] = gamma gives the scalar forms' results bit for bit.  discount_dev float [B]. */
+int ofb_trainer_td_targets_discounted(const float *act_obs_dev, const float *ptr_obs_dev, const float *act_next_dev,
+                                      const float *ptr_next_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
+                                      const float *reward_dev, const uint8_t *done_dev, const float *discount_dev, int batch,
+                                      float *target_act_dev, float *target_ptr_dev, void *stream);
+int ofb_trainer_td_errors_discounted(const float *act_obs_dev, const float *ptr_obs_dev, const float *act_next_dev,
+                                     const float *ptr_next_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
+                                     const float *reward_dev, const uint8_t *done_dev, const float *discount_dev, int batch,
+                                     float *td_act_dev, float *td_ptr_dev, void *stream);
+
 /* Flat copies to HOST (synchronise `stream` first): current weights / gradients of the last fit. */
 int ofb_trainer_get_weights(ofb_trainer *t, float *weights_flat_host, void *stream);
 int ofb_trainer_get_grads(ofb_trainer *t, float *grads_flat_host, void *stream);

@@ -150,6 +150,8 @@ def load():
     lib.ofb_trainer_td_targets.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, i32, vp, vp, vp]
     lib.ofb_trainer_fit_weighted.argtypes = [vp, vp, vp, vp, vp, vp, i32, vp, vp]
     lib.ofb_trainer_td_errors.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, i32, vp, vp, vp]
+    lib.ofb_trainer_td_targets_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
+    lib.ofb_trainer_td_errors_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.ofb_trainer_get_weights.argtypes = [vp, vp, vp]
     lib.ofb_trainer_get_grads.argtypes = [vp, vp, vp]
     lib.ofb_trainer_steps.argtypes = [vp]
@@ -163,16 +165,19 @@ def load():
     lib.ofb_replay_push.argtypes = [vp, vp, vp, vp, vp]
     lib.ofb_replay_index.argtypes = [vp, vp, vp, vp]
     lib.ofb_replay_gather.argtypes = [vp, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.ofb_replay_set_n_step.argtypes = [vp, i32]
+    lib.ofb_replay_gather_nstep.argtypes = [vp, vp, i32, C.c_float, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.ofb_replay_enable_priorities.argtypes = [vp, C.POINTER(OfbReplayPrioConfig)]
     lib.ofb_replay_sample_prioritized.argtypes = [vp, i32, C.c_float, vp, vp, vp, vp]
     lib.ofb_replay_update_priorities.argtypes = [vp, vp, vp, vp, i32, vp]
     lib.ofb_replay_read_priorities.argtypes = [vp, vp, vp, vp, vp]
     for name in ("ofb_replay_create", "ofb_replay_destroy", "ofb_replay_push", "ofb_replay_index", "ofb_replay_gather",
                  "ofb_replay_enable_priorities", "ofb_replay_sample_prioritized", "ofb_replay_update_priorities",
-                 "ofb_replay_read_priorities"):
+                 "ofb_replay_read_priorities", "ofb_replay_set_n_step", "ofb_replay_gather_nstep"):
         getattr(lib, name).restype = i32
     for name in ("ofb_trainer_create", "ofb_trainer_destroy", "ofb_trainer_fit", "ofb_trainer_forward",
-                 "ofb_trainer_td_targets", "ofb_trainer_fit_weighted", "ofb_trainer_td_errors", "ofb_trainer_get_weights", "ofb_trainer_get_grads"):
+                 "ofb_trainer_td_targets", "ofb_trainer_fit_weighted", "ofb_trainer_td_errors", "ofb_trainer_get_weights", "ofb_trainer_get_grads",
+                 "ofb_trainer_td_targets_discounted", "ofb_trainer_td_errors_discounted"):
         getattr(lib, name).restype = i32
     for name in ("ofb_policy_create", "ofb_policy_destroy", "ofb_policy_set_engine", "ofb_policy_forward",
                  "ofb_policy_write_actions", "ofb_policy_pack_image", "ofb_policy_debug_tap"):

@@ -3,7 +3,8 @@
 //
 // Ring layout: slot s, tracked arena a -> ring + (s * count + a) * stride, the first bytes of an arena block (header,
 // ships, live laser groups) copied from the handle's state.  Per transition id = s * count * P + a * P + p (P policy ships):
-// the played action and pointer of frame s, and -- once frame s + 1 was pushed -- valid / reward / done.
+// the played action and pointer of frame s, and -- once frame s + 1 was pushed -- valid / reward / done.  An n-step memory
+// keeps the same one-step fields: ofb_replay_gather_nstep walks them at gather time.
 #include <cstring>
 #include <new>
 #include "ofb_common.cuh"
@@ -22,6 +23,7 @@ struct ofb_replay {
     int device;
     long long first, count;
     int P, depth;
+    int n_step;                  // frames of an n-step return (1 = one-step transitions)
     int32_t *ships;              // [P] ship index of each policy ship
     char *ring;                  // depth * count * stride bytes
     int32_t *act;                // [depth * count * P]
@@ -49,7 +51,8 @@ struct ofb_replay {
 // ---------------------------------------------------------------- push: one warp per tracked arena
 __global__ void __launch_bounds__(128)
 k_replay_push(const char *__restrict__ state, const ArenaLayout lay, long long first, long long count,
-              const int32_t *__restrict__ ships, int P, char *__restrict__ ring, int slot, int prev, const int32_t *__restrict__ iaction_in,
+              const int32_t *__restrict__ ships, int P, char *__restrict__ ring, int slot, int prev, int mslot,
+              const int32_t *__restrict__ iaction_in,
               const int2 *__restrict__ xy_in, int32_t *__restrict__ act, int2 *__restrict__ xy, float *__restrict__ reward,
               uint8_t *__restrict__ valid, uint8_t *__restrict__ done, float *__restrict__ mass, const float *__restrict__ max_mass) {
     const long long a = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -77,8 +80,9 @@ k_replay_push(const char *__restrict__ state, const ArenaLayout lay, long long f
             valid[prev * cP + j] = (same_episode && (orec.x >> 31)) ? 1 : 0;
             reward[prev * cP + j] = (float)ship_unpack(rec).reward;
             done[prev * cP + j] = (rec.x >> 31) ? 0 : 1;
-            if (mass) mass[prev * cP + j] = *max_mass;    // prioritized replay: a new transition gets the largest mass
         }
+        // prioritized replay: the frame that becomes a candidate with this push (prev for n = 1) gets the largest mass
+        if (mass && mslot >= 0) mass[mslot * cP + j] = *max_mass;
         const long long o = (long long)slot * cP + j;
         valid[o] = 0;                                      // the newest frame has no successor yet
         act[o] = iaction_in[(first + a) * P + lane];
@@ -168,40 +172,23 @@ k_replay_scatter(const uint8_t *__restrict__ valid, long long cP, long long n_ca
 }
 
 // ---------------------------------------------------------------- gather: one CTA per (sample, obs | next)
-__global__ void __launch_bounds__(256)
-k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long count, int P, int depth,
-                const int32_t *__restrict__ ships,                const int32_t *__restrict__ ids, const int32_t *__restrict__ act, const int2 *__restrict__ axy,
-                const float *__restrict__ rew, const uint8_t *__restrict__ dn, uint32_t *__restrict__ maps_obs,
-                float *__restrict__ vec_obs, uint32_t *__restrict__ maps_next, float *__restrict__ vec_next,
-                int32_t *__restrict__ iaction, int32_t *__restrict__ pointer, float *__restrict__ reward,
-                uint8_t *__restrict__ done) {
-    extern __shared__ __align__(128) uint32_t bits[];      // [2][words], as k_raster
+// One observation of sample b: the snapshot of tracked arena a in ring slot s -> the ship's head (ofb_obs_vec's, k_obs_vec)
+// and the two bit maps, rasterised with the frame kernel's code and written with one bulk store.  Every thread of the CTA
+// calls it (it synchronises the block).
+__device__ __forceinline__ void gather_observation(uint32_t *bits, const char *__restrict__ ring, const ArenaLayout &lay,
+                                                   long long count, long long s, long long a, int ship, int b,
+                                                   uint32_t *__restrict__ maps, float *__restrict__ vec) {
     const int W = lay.W, H = lay.H;
     const int words = (W * H) >> 5;
-    const int b = blockIdx.x, next = blockIdx.y;
-    const long long cP = count * P;
-    const long long id = ids[b];
-    const long long slot = id / cP, j = id - slot * cP;
-    const long long a = j / P;
-    const int p = (int)(j - a * P);
-    const long long s = next ? (slot + 1) % depth : slot;
     const char *base = ring + (s * count + a) * (long long)lay.stride;
     const int *hdr = reinterpret_cast<const int *>(base);
-    const uint4 *ship = reinterpret_cast<const uint4 *>(base + lay.off_ship);
-    uint32_t *maps = next ? maps_next : maps_obs;
-    float *vec = next ? vec_next : vec_obs;
+    const uint4 *shp = reinterpret_cast<const uint4 *>(base + lay.off_ship);
 
-    if (vec && threadIdx.x == 0) {                         // ofb_obs_vec's head (k_obs_vec) of the ship
-        const ShipRec r = ship_unpack(ship[ships[p]]);
+    if (vec && threadIdx.x == 0) {
+        const ShipRec r = ship_unpack(shp[ship]);
         float4 *v = reinterpret_cast<float4 *>(vec + (long long)b * 8);
         v[0] = make_float4((float)r.reward, 1.0f, (float)r.px, (float)r.py);
         v[1] = make_float4((float)lay.W, (float)lay.H, (float)r.x, (float)r.y);
-    }
-    if (!next && threadIdx.x == 1) {
-        if (iaction) iaction[b] = act[id];
-        if (pointer) reinterpret_cast<int2 *>(pointer)[b] = axy[id];
-        if (reward) reward[b] = rew[id];
-        if (done) done[b] = dn[id];
     }
     if (!maps) return;
 
@@ -213,7 +200,7 @@ k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long 
     __syncthreads();
     const int rows = 2 * OFB_R_SHIP - 1;
     for (int t = threadIdx.x; t < lay.S * rows; t += blockDim.x)
-        raster_ship_row(bits, W, H, ship[t / rows].x, t % rows - (OFB_R_SHIP - 1));
+        raster_ship_row(bits, W, H, shp[t / rows].x, t % rows - (OFB_R_SHIP - 1));
     for (int k = threadIdx.x; k < n; k += blockDim.x) {
         const double *lp = reinterpret_cast<const double *>(base + laser_off(lay.off_laser, k));
         raster_laser(bits + words, W, H, lp[0], lp[OFB_G_Y / 8]);
@@ -228,6 +215,90 @@ k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long 
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
     }
+}
+
+__global__ void __launch_bounds__(256)
+k_replay_gather(const char *__restrict__ ring, const ArenaLayout lay, long long count, int P, int depth,
+                const int32_t *__restrict__ ships, const int32_t *__restrict__ ids, const int32_t *__restrict__ act,
+                const int2 *__restrict__ axy, const float *__restrict__ rew, const uint8_t *__restrict__ dn,
+                uint32_t *__restrict__ maps_obs, float *__restrict__ vec_obs, uint32_t *__restrict__ maps_next,
+                float *__restrict__ vec_next, int32_t *__restrict__ iaction, int32_t *__restrict__ pointer,
+                float *__restrict__ reward, uint8_t *__restrict__ done) {
+    extern __shared__ __align__(128) uint32_t bits[];      // [2][words], as k_raster
+    const int b = blockIdx.x, next = blockIdx.y;
+    const long long cP = count * P;
+    const long long id = ids[b];
+    const long long slot = id / cP, j = id - slot * cP;
+    const long long a = j / P;
+    const int p = (int)(j - a * P);
+    if (!next && threadIdx.x == 1) {
+        if (iaction) iaction[b] = act[id];
+        if (pointer) reinterpret_cast<int2 *>(pointer)[b] = axy[id];
+        if (reward) reward[b] = rew[id];
+        if (done) done[b] = dn[id];
+    }
+    gather_observation(bits, ring, lay, count, next ? (slot + 1) % depth : slot, a, ships[p], b, next ? maps_next : maps_obs,
+                       next ? vec_next : vec_obs);
+}
+
+// The n-step window of transition (frame t = `slot`, arena x ship j), from the one-step fields of frames t, t+1, ...:
+// k frames, ended by a death (done), by the end of the episode after frame t+k, or at k = n.  R = r[t+k-1], then
+// R = r[t+i] + gamma * R for i = k-2 .. 0, and discount = gamma^k as k-1 products from gamma, all rounded without fma.
+struct NStepWindow {
+    int k;
+    int done;
+    float ret, discount;
+};
+
+__device__ __forceinline__ NStepWindow nstep_window(const uint8_t *__restrict__ valid, const uint8_t *__restrict__ dn,
+                                                    const float *__restrict__ rew, long long slot, long long j, long long cP,
+                                                    int depth, int n, float gamma) {
+    NStepWindow w = {n, 0, 0.0f, 0.0f};
+    for (int i = 0; i < n; i++) {
+        if (dn[((slot + i) % depth) * cP + j]) { w.k = i + 1; w.done = 1; break; }
+        if (i + 1 == n) break;
+        if (!valid[((slot + i + 1) % depth) * cP + j]) { w.k = i + 1; break; }   // the episode ends after frame t+i+1
+    }
+    float R = rew[((slot + w.k - 1) % depth) * cP + j];
+    for (int i = w.k - 2; i >= 0; i--) R = __fadd_rn(rew[((slot + i) % depth) * cP + j], __fmul_rn(gamma, R));
+    float d = gamma;
+    for (int i = 1; i < w.k; i++) d = __fmul_rn(d, gamma);
+    w.ret = R;
+    w.discount = d;
+    return w;
+}
+
+// k_replay_gather for n-step transitions: obs = frame t, next = frame t+k.  Thread 0 of the next-CTA walks the window before
+// the raster; thread 1 of the obs-CTA walks it again to write the scalar fields (at most n bytes and floats each).
+__global__ void __launch_bounds__(256)
+k_replay_gather_nstep(const char *__restrict__ ring, const ArenaLayout lay, long long count, int P, int depth, int n_step,
+                      float gamma, const int32_t *__restrict__ ships, const int32_t *__restrict__ ids,
+                      const int32_t *__restrict__ act, const int2 *__restrict__ axy, const float *__restrict__ rew,
+                      const uint8_t *__restrict__ valid, const uint8_t *__restrict__ dn, uint32_t *__restrict__ maps_obs,
+                      float *__restrict__ vec_obs, uint32_t *__restrict__ maps_next, float *__restrict__ vec_next,
+                      int32_t *__restrict__ iaction, int32_t *__restrict__ pointer, float *__restrict__ ret,
+                      uint8_t *__restrict__ done, float *__restrict__ discount, int32_t *__restrict__ steps) {
+    extern __shared__ __align__(128) uint32_t bits[];
+    __shared__ int s_k;
+    const int b = blockIdx.x, next = blockIdx.y;
+    const long long cP = count * P;
+    const long long id = ids[b];
+    const long long slot = id / cP, j = id - slot * cP;
+    const long long a = j / P;
+    const int p = (int)(j - a * P);
+    if (next && threadIdx.x == 0) s_k = nstep_window(valid, dn, rew, slot, j, cP, depth, n_step, gamma).k;
+    if (!next && threadIdx.x == 1) {
+        const NStepWindow w = nstep_window(valid, dn, rew, slot, j, cP, depth, n_step, gamma);
+        if (iaction) iaction[b] = act[id];
+        if (pointer) reinterpret_cast<int2 *>(pointer)[b] = axy[id];
+        if (ret) ret[b] = w.ret;
+        if (done) done[b] = (uint8_t)w.done;
+        if (discount) discount[b] = w.discount;
+        if (steps) steps[b] = w.k;
+    }
+    if (next) __syncthreads();                             // s_k (uniform branch: the whole CTA takes it)
+    gather_observation(bits, ring, lay, count, next ? (slot + s_k) % depth : slot, a, ships[p], b, next ? maps_next : maps_obs,
+                       next ? vec_next : vec_obs);
 }
 
 // ---------------------------------------------------------------- prioritized sampling: tile sums, scan, one block per draw
@@ -473,6 +544,7 @@ extern "C" int ofb_replay_create(const ofb_arenas *h, int64_t first, int64_t cou
     r->count = count;
     r->P = n_policy;
     r->depth = depth;
+    r->n_step = 1;
     r->pushes = 0;
     r->newest = depth - 1;
     r->n_tiles = ((long long)(depth - 1) * cP + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
@@ -510,6 +582,26 @@ extern "C" int ofb_replay_destroy(ofb_replay *r) {
 extern "C" int64_t ofb_replay_device_bytes(const ofb_replay *r) { return r ? (int64_t)r->bytes : OFB_E_ARG; }
 extern "C" int64_t ofb_replay_pushes(const ofb_replay *r) { return r ? (int64_t)r->pushes : OFB_E_ARG; }
 
+extern "C" int ofb_replay_set_n_step(ofb_replay *r, int32_t n) {
+    if (!r) { ofb_set_error("ofb_replay_set_n_step: null argument"); return OFB_E_ARG; }
+    if (r->pushes > 0) { ofb_set_error("ofb_replay_set_n_step: only before the first push"); return OFB_E_ARG; }
+    if (n < 1 || n > r->depth - 1) {
+        ofb_set_error("ofb_replay_set_n_step: need 1 <= n <= depth - 1 = %d (got %d)", r->depth - 1, n);
+        return OFB_E_ARG;
+    }
+    r->n_step = n;
+    return OFB_OK;
+}
+
+// Candidates of ofb_replay_index and ofb_replay_sample_prioritized: the frames [T - filled + 1, T - n] of the ring, starting at
+// the oldest slot.  Returns their number of frames.
+static long long replay_candidates(const ofb_replay *r, int *oldest) {
+    const long long filled = r->pushes < r->depth ? r->pushes : r->depth;
+    const long long nf = filled > 0 ? filled - 1 : 0;
+    *oldest = (int)((r->newest - nf + r->depth) % r->depth);
+    return filled > r->n_step ? filled - r->n_step : 0;
+}
+
 extern "C" int ofb_replay_push(ofb_replay *r, const ofb_arenas *h, const int32_t *iaction_dev, const int32_t *xy_dev,
                                void *stream) {
     if (!r || !iaction_dev || !xy_dev) { ofb_set_error("ofb_replay_push: null argument"); return OFB_E_ARG; }
@@ -517,9 +609,11 @@ extern "C" int ofb_replay_push(ofb_replay *r, const ofb_arenas *h, const int32_t
     OFB_CUDA_CHECK(cudaSetDevice(r->device));
     const int slot = (r->newest + 1) % r->depth;
     const int prev = r->pushes > 0 ? r->newest : -1;
+    // frame T - n becomes a candidate with this push of frame T = pushes (prev for n = 1)
+    const int mslot = r->pushes >= r->n_step ? (slot - r->n_step + r->depth) % r->depth : -1;
     const long long threads = r->count * 32;
     k_replay_push<<<(unsigned)((threads + 127) / 128), 128, 0, (cudaStream_t)stream>>>(
-        h->state, r->lay, r->first, r->count, r->ships, r->P, r->ring, slot, prev, iaction_dev,
+        h->state, r->lay, r->first, r->count, r->ships, r->P, r->ring, slot, prev, mslot, iaction_dev,
         reinterpret_cast<const int2 *>(xy_dev), r->act, r->xy, r->reward, r->valid, r->done, r->mass, r->max_mass);
     OFB_CUDA_CHECK(cudaGetLastError());
     r->newest = slot;
@@ -531,14 +625,12 @@ extern "C" int ofb_replay_index(ofb_replay *r, int32_t *ids_dev, int32_t *count_
     if (!r || !ids_dev || !count_dev) { ofb_set_error("ofb_replay_index: null argument"); return OFB_E_ARG; }
     OFB_CUDA_CHECK(cudaSetDevice(r->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const long long filled = r->pushes < r->depth ? r->pushes : r->depth;
-    const long long nf = filled > 0 ? filled - 1 : 0;           // frames with a successor
-    const long long cP = r->count * r->P, n_cand = nf * cP;
+    int oldest = 0;
+    const long long cP = r->count * r->P, n_cand = replay_candidates(r, &oldest) * cP;
     if (n_cand == 0) {
         OFB_CUDA_CHECK(cudaMemsetAsync(count_dev, 0, sizeof(int32_t), st));
         return OFB_OK;
     }
-    const int oldest = (int)((r->newest - nf + r->depth) % r->depth);
     const long long tiles = (n_cand + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
     k_replay_count<<<(unsigned)tiles, 256, 0, st>>>(r->valid, cP, n_cand, oldest, r->depth, r->tile_count);
     k_replay_scan<<<1, 1024, 0, st>>>(r->tile_count, tiles, count_dev);
@@ -551,6 +643,10 @@ extern "C" int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, in
                                  float *vec_obs_dev, uint32_t *maps_next_dev, float *vec_next_dev, int32_t *iaction_dev,
                                  int32_t *pointer_dev, float *reward_dev, uint8_t *done_dev, void *stream) {
     if (!r || !ids_dev || batch < 0) { ofb_set_error("ofb_replay_gather: bad argument"); return OFB_E_ARG; }
+    if (r->n_step > 1) {
+        ofb_set_error("ofb_replay_gather: the memory holds %d-step transitions: use ofb_replay_gather_nstep", r->n_step);
+        return OFB_E_ARG;
+    }
     if (batch == 0) return OFB_OK;
     OFB_CUDA_CHECK(cudaSetDevice(r->device));
     const size_t smem = (size_t)(r->lay.W * r->lay.H / 32) * 2 * sizeof(uint32_t);
@@ -559,6 +655,28 @@ extern "C" int ofb_replay_gather(const ofb_replay *r, const int32_t *ids_dev, in
     k_replay_gather<<<dim3((unsigned)batch, 2), 256, smem, (cudaStream_t)stream>>>(
         r->ring, r->lay, r->count, r->P, r->depth, r->ships, ids_dev, r->act, r->xy, r->reward, r->done, maps_obs_dev,
         vec_obs_dev, maps_next_dev, vec_next_dev, iaction_dev, pointer_dev, reward_dev, done_dev);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_gather_nstep(const ofb_replay *r, const int32_t *ids_dev, int32_t batch, float gamma,
+                                       uint32_t *maps_obs_dev, float *vec_obs_dev, uint32_t *maps_next_dev, float *vec_next_dev,
+                                       int32_t *iaction_dev, int32_t *pointer_dev, float *return_dev, uint8_t *done_dev,
+                                       float *discount_dev, int32_t *steps_dev, void *stream) {
+    if (!r || !ids_dev || batch < 0) { ofb_set_error("ofb_replay_gather_nstep: bad argument"); return OFB_E_ARG; }
+    if (!(gamma >= 0.0f && gamma <= 3.402823466e38f)) {
+        ofb_set_error("ofb_replay_gather_nstep: need a finite gamma >= 0 (got %g)", gamma);
+        return OFB_E_ARG;
+    }
+    if (batch == 0) return OFB_OK;
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    const size_t smem = (size_t)(r->lay.W * r->lay.H / 32) * 2 * sizeof(uint32_t);
+    static thread_local SmemAttrCache attr = {};
+    if (smem > 48 * 1024) OFB_CUDA_CHECK(attr.ensure(k_replay_gather_nstep, (int)smem));
+    k_replay_gather_nstep<<<dim3((unsigned)batch, 2), 256, smem, (cudaStream_t)stream>>>(
+        r->ring, r->lay, r->count, r->P, r->depth, r->n_step, gamma, r->ships, ids_dev, r->act, r->xy, r->reward, r->valid,
+        r->done, maps_obs_dev, vec_obs_dev, maps_next_dev, vec_next_dev, iaction_dev, pointer_dev, return_dev, done_dev,
+        discount_dev, steps_dev);
     OFB_CUDA_CHECK(cudaGetLastError());
     return OFB_OK;
 }
@@ -612,14 +730,12 @@ extern "C" int ofb_replay_sample_prioritized(ofb_replay *r, int32_t batch, float
     }
     OFB_CUDA_CHECK(cudaSetDevice(r->device));
     cudaStream_t st = (cudaStream_t)stream;
-    const long long filled = r->pushes < r->depth ? r->pushes : r->depth;
-    const long long nf = filled > 0 ? filled - 1 : 0;
-    const long long cP = r->count * r->P, n_cand = nf * cP;
+    int oldest = 0;
+    const long long cP = r->count * r->P, n_cand = replay_candidates(r, &oldest) * cP;
     if (n_cand == 0) {
         OFB_CUDA_CHECK(cudaMemsetAsync(n_valid_out, 0, sizeof(int32_t), st));
         return OFB_OK;
     }
-    const int oldest = (int)((r->newest - nf + r->depth) % r->depth);
     const long long tiles = (n_cand + OFB_REPLAY_TILE - 1) / OFB_REPLAY_TILE;
     k_prio_tiles<<<(unsigned)tiles, 256, 0, st>>>(r->valid, r->mass, cP, n_cand, oldest, r->depth, r->tile_sum, r->tile_min,
                                                  r->tile_valid);

@@ -686,9 +686,10 @@ __global__ void k_tr_adam(float *__restrict__ p, const float *__restrict__ g, fl
 
 __global__ void k_tr_td_targets(const float *__restrict__ act_obs, const float *__restrict__ ptr_obs, const float *__restrict__ act_next,
                                 const float *__restrict__ ptr_next, const int32_t *__restrict__ iaction, const int32_t *__restrict__ pointer,
-                                const float *__restrict__ reward, const uint8_t *__restrict__ done, float gamma, float *__restrict__ t_act,
-                                float *__restrict__ t_ptr) {
-    // one block per sample: max over the next pointer map, copy of the obs predictions, the two overwritten entries
+                                const float *__restrict__ reward, const uint8_t *__restrict__ done, float gamma,
+                                const float *__restrict__ discount, float *__restrict__ t_act, float *__restrict__ t_ptr) {
+    // one block per sample: max over the next pointer map, copy of the obs predictions, the two overwritten entries.
+    // discount [B] (n-step returns) replaces the scalar gamma when it is not NULL.
     const long long b = blockIdx.x;
     const int n = IMG * IMG;
     __shared__ float red[32];
@@ -703,13 +704,14 @@ __global__ void k_tr_td_targets(const float *__restrict__ act_obs, const float *
     if (threadIdx.x == 0) {
         for (int wv = 1; wv < (int)((blockDim.x + 31) >> 5); wv++) mx = fmaxf(mx, red[wv]);
         const float keep = done[b] ? 0.0f : 1.0f, r = reward[b];
+        const float g = discount ? discount[b] : gamma;
         const float a0 = act_obs[b * 2], a1 = act_obs[b * 2 + 1];
         const float ma = fmaxf(act_next[b * 2], act_next[b * 2 + 1]);
         t_act[b * 2] = a0;
         t_act[b * 2 + 1] = a1;
-        t_act[b * 2 + iaction[b]] = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, ma), keep));      // no fma: same roundings as the host oracle
+        t_act[b * 2 + iaction[b]] = __fadd_rn(r, __fmul_rn(__fmul_rn(g, ma), keep));      // no fma: same roundings as the host oracle
         // ptr_target[ipointer] with ipointer = (x, y) indexes the [row, col] map as [x][y]   (qlearnIA_V2.py:280)
-        t_ptr[b * n + (long long)pointer[b * 2] * IMG + pointer[b * 2 + 1]] = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, mx), keep));
+        t_ptr[b * n + (long long)pointer[b * 2] * IMG + pointer[b * 2 + 1]] = __fadd_rn(r, __fmul_rn(__fmul_rn(g, mx), keep));
     }
 }
 
@@ -717,8 +719,8 @@ __global__ void k_tr_td_targets(const float *__restrict__ act_obs, const float *
 // maximum is order-independent), so td = t_target - prediction exactly.  One block per sample.
 __global__ void k_tr_td_errors(const float *__restrict__ act_obs, const float *__restrict__ ptr_obs, const float *__restrict__ act_next,
                                const float *__restrict__ ptr_next, const int32_t *__restrict__ iaction, const int32_t *__restrict__ pointer,
-                               const float *__restrict__ reward, const uint8_t *__restrict__ done, float gamma, float *__restrict__ td_act,
-                               float *__restrict__ td_ptr) {
+                               const float *__restrict__ reward, const uint8_t *__restrict__ done, float gamma,
+                               const float *__restrict__ discount, float *__restrict__ td_act, float *__restrict__ td_ptr) {
     const long long b = blockIdx.x;
     const int n = IMG * IMG;
     __shared__ float red[32];
@@ -730,9 +732,10 @@ __global__ void k_tr_td_errors(const float *__restrict__ act_obs, const float *_
     if (threadIdx.x == 0) {
         for (int wv = 1; wv < (int)((blockDim.x + 31) >> 5); wv++) mx = fmaxf(mx, red[wv]);
         const float keep = done[b] ? 0.0f : 1.0f, r = reward[b];
+        const float g = discount ? discount[b] : gamma;
         const float ma = fmaxf(act_next[b * 2], act_next[b * 2 + 1]);
-        const float ta = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, ma), keep));
-        const float tp = __fadd_rn(r, __fmul_rn(__fmul_rn(gamma, mx), keep));
+        const float ta = __fadd_rn(r, __fmul_rn(__fmul_rn(g, ma), keep));
+        const float tp = __fadd_rn(r, __fmul_rn(__fmul_rn(g, mx), keep));
         td_act[b] = __fsub_rn(ta, act_obs[b * 2 + iaction[b]]);
         td_ptr[b] = __fsub_rn(tp, ptr_obs[b * n + (long long)pointer[b * 2] * IMG + pointer[b * 2 + 1]]);
     }
@@ -1044,30 +1047,62 @@ extern "C" int ofb_trainer_fit_weighted(ofb_trainer *t, const uint32_t *maps, co
     return fit_impl(t, maps, vec, target_act, target_ptr, sample_weight, B, loss_dev, stream);
 }
 
+static int td_errors_impl(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
+                          const int32_t *iaction, const int32_t *pointer, const float *reward, const uint8_t *done, float gamma,
+                          const float *discount, int B, float *td_act, float *td_ptr, void *stream, const char *who) {
+    if (!act_obs || !ptr_obs || !act_next || !ptr_next || !iaction || !pointer || !reward || !done || !td_act || !td_ptr || B < 1) {
+        ofb_set_error("%s: bad argument", who);
+        return OFB_E_ARG;
+    }
+    k_tr_td_errors<<<B, 256, 0, (cudaStream_t)stream>>>(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma,
+                                                        discount, td_act, td_ptr);
+    TR_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+static int td_targets_impl(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
+                           const int32_t *iaction, const int32_t *pointer, const float *reward, const uint8_t *done, float gamma,
+                           const float *discount, int B, float *t_act, float *t_ptr, void *stream, const char *who) {
+    if (!act_obs || !ptr_obs || !act_next || !ptr_next || !iaction || !pointer || !reward || !done || !t_act || !t_ptr || B < 1) {
+        ofb_set_error("%s: bad argument", who);
+        return OFB_E_ARG;
+    }
+    k_tr_td_targets<<<B, 256, 0, (cudaStream_t)stream>>>(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma,
+                                                         discount, t_act, t_ptr);
+    TR_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
 extern "C" int ofb_trainer_td_errors(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
                                      const int32_t *iaction, const int32_t *pointer, const float *reward, const uint8_t *done, float gamma,
                                      int B, float *td_act, float *td_ptr, void *stream) {
-    if (!act_obs || !ptr_obs || !act_next || !ptr_next || !iaction || !pointer || !reward || !done || !td_act || !td_ptr || B < 1) {
-        ofb_set_error("ofb_trainer_td_errors: bad argument");
-        return OFB_E_ARG;
-    }
-    k_tr_td_errors<<<B, 256, 0, (cudaStream_t)stream>>>(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma, td_act,
-                                                        td_ptr);
-    TR_CHECK(cudaGetLastError());
-    return OFB_OK;
+    return td_errors_impl(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma, nullptr, B, td_act, td_ptr,
+                          stream, "ofb_trainer_td_errors");
 }
 
 extern "C" int ofb_trainer_td_targets(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
                                       const int32_t *iaction, const int32_t *pointer, const float *reward, const uint8_t *done, float gamma,
                                       int B, float *t_act, float *t_ptr, void *stream) {
-    if (!act_obs || !ptr_obs || !act_next || !ptr_next || !iaction || !pointer || !reward || !done || !t_act || !t_ptr || B < 1) {
-        ofb_set_error("ofb_trainer_td_targets: bad argument");
-        return OFB_E_ARG;
-    }
-    k_tr_td_targets<<<B, 256, 0, (cudaStream_t)stream>>>(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma, t_act,
-                                                         t_ptr);
-    TR_CHECK(cudaGetLastError());
-    return OFB_OK;
+    return td_targets_impl(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, gamma, nullptr, B, t_act, t_ptr,
+                           stream, "ofb_trainer_td_targets");
+}
+
+extern "C" int ofb_trainer_td_errors_discounted(const float *act_obs, const float *ptr_obs, const float *act_next,
+                                                const float *ptr_next, const int32_t *iaction, const int32_t *pointer,
+                                                const float *reward, const uint8_t *done, const float *discount, int B, float *td_act,
+                                                float *td_ptr, void *stream) {
+    if (!discount) { ofb_set_error("ofb_trainer_td_errors_discounted: null discount"); return OFB_E_ARG; }
+    return td_errors_impl(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, 0.0f, discount, B, td_act, td_ptr,
+                          stream, "ofb_trainer_td_errors_discounted");
+}
+
+extern "C" int ofb_trainer_td_targets_discounted(const float *act_obs, const float *ptr_obs, const float *act_next,
+                                                 const float *ptr_next, const int32_t *iaction, const int32_t *pointer,
+                                                 const float *reward, const uint8_t *done, const float *discount, int B, float *t_act,
+                                                 float *t_ptr, void *stream) {
+    if (!discount) { ofb_set_error("ofb_trainer_td_targets_discounted: null discount"); return OFB_E_ARG; }
+    return td_targets_impl(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, 0.0f, discount, B, t_act, t_ptr,
+                           stream, "ofb_trainer_td_targets_discounted");
 }
 
 static int copy_out(ofb_trainer *t, const float *src, float *dst_host, void *stream, const char *who) {

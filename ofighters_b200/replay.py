@@ -21,6 +21,13 @@ appends to ``trainer.memory``, and ``sample`` draws ``random.sample(range(len), 
 
 ``PrioritizedReplayMemory`` adds prioritized replay on the device: masses from the TD errors, a stratified proportional sampler
 and importance weights for ``TrainerB200.fit(..., sample_weight=...)``.
+
+Either memory takes ``n_step``: with n > 1 a transition is an n-step window, gathered on the device with its discounted return
+R = sum_j gamma^j r_{t+j} over k <= n frames, its bootstrap observation s_{t+k} and discount = gamma^k (include/ofb_replay.h
+states the rules).  A shot bonus then reaches back n frames per fit instead of one.
+
+    memory = DeviceReplayMemory(bg, depth=16, n_step=3)       # gamma = trainer.gamma = 0.9
+    learner = BatchedQLearner(trainer, memory)
 """
 import ctypes as C
 import random
@@ -38,11 +45,15 @@ def _ptr(t):
 
 
 class DeviceReplayMemory:
-    def __init__(self, bg, depth=16, track=None, ships=None):
+    def __init__(self, bg, depth=16, track=None, ships=None, n_step=1, gamma=0.9):
         """``bg``: the BatchedBattleground whose arenas are remembered.  ``depth``: frames in the ring (>= 2); it holds the
         transitions of the last ``depth - 1`` pushed frames.  ``track``: the first ``track`` arenas (default: all).
         ``ships``: ship indices to remember, among the battleground's QlearnIA / external ships (default: all of them);
-        ``push`` takes the actions of all those ships, as ``PolicyB200.act`` returns them."""
+        ``push`` takes the actions of all those ships, as ``PolicyB200.act`` returns them.
+        ``n_step``: frames of a transition's return (1 <= n_step <= depth - 1); with n_step > 1 the ring holds the
+        transitions of the frames [T - depth + 1, T - n_step] (T = the newest), ``gather`` returns the n-step return R in
+        ``reward`` with ``discount`` = gamma^k and ``steps`` = k, and ``gamma`` discounts the rewards inside the window (it
+        must be the trainer's)."""
         if not torch.cuda.is_available():
             raise _lib.OfbError("DeviceReplayMemory needs a CUDA device: the ring lives in HBM and has no CPU fallback")
         policy = [i for i, b in enumerate(bg.behaviors) if b in _POLICY_BEHAVIORS]
@@ -54,11 +65,17 @@ class DeviceReplayMemory:
         track = bg.n_arenas if track is None else int(track)
         if not 1 <= track <= bg.n_arenas:
             raise Exception("Invalid track {} : the batch holds {} arenas.".format(track, bg.n_arenas))
+        n_step, gamma = int(n_step), float(gamma)
+        if n_step < 1 or (n_step > 1 and int(depth) < n_step + 1):      # (a one-step memory's depth is ofb_replay_create's)
+            raise Exception("Invalid n_step {} : need 1 <= n_step <= depth - 1 = {}.".format(n_step, int(depth) - 1))
+        if not 0.0 <= gamma < float("inf"):
+            raise Exception("Invalid gamma {} : expected a finite value >= 0.".format(gamma))
         self.bg = bg
         self.device = bg.device
         self.depth = int(depth)
         self.track = track
         self.ships = ships
+        self.n_step, self.gamma = n_step, gamma
         self.n_policy = len(policy)                      # policy ships per arena in the actions push() takes
         self._cols = None if ships == policy else torch.tensor([policy.index(s) for s in ships], dtype=torch.long,
                                                                device=self.device)
@@ -68,6 +85,8 @@ class DeviceReplayMemory:
         with torch.cuda.device(self.device):
             _lib.check(self._lib.ofb_replay_create(bg._h, 0, track, idx, len(ships), self.depth, C.byref(h)))
         self._h = h
+        if n_step > 1:
+            _lib.check(self._lib.ofb_replay_set_n_step(h, n_step))
         self._ids = torch.empty(max(1, (self.depth - 1) * track * len(ships)), dtype=torch.int32, device=self.device)
         self._count = torch.zeros(1, dtype=torch.int32, device=self.device)
         self._n = 0
@@ -129,7 +148,9 @@ class DeviceReplayMemory:
     def gather(self, positions):
         """The transitions at ``positions`` (0 = oldest) -> SimpleNamespace of device tensors: maps_obs / maps_next int32
         [B, 2, W*H/32] bit maps, vec_obs / vec_next float32 [B, 8], iaction int32 [B], pointer int32 [B, 2] = (x, y),
-        reward float32 [B], done uint8 [B] -- the inputs of ``TrainerB200.replay``'s targets and fit."""
+        reward float32 [B], done uint8 [B] -- the inputs of ``TrainerB200.replay``'s targets and fit.  An n-step memory
+        (n_step > 1) puts the return R in ``reward``, s_{t+k} in maps_next / vec_next and adds ``discount`` float32 [B]
+        (gamma^k) and ``steps`` int32 [B] (k)."""
         n = len(self)
         pos = torch.as_tensor(positions, dtype=torch.int64).reshape(-1)
         if pos.numel() < 1:
@@ -152,6 +173,15 @@ class DeviceReplayMemory:
             pointer=torch.empty((B, 2), dtype=torch.int32, device=dev),
             reward=torch.empty((B,), dtype=torch.float32, device=dev),
             done=torch.empty((B,), dtype=torch.uint8, device=dev))
+        if self.n_step > 1:
+            out.discount = torch.empty((B,), dtype=torch.float32, device=dev)
+            out.steps = torch.empty((B,), dtype=torch.int32, device=dev)
+            _lib.check(self._lib.ofb_replay_gather_nstep(
+                self._h, _ptr(ids), B, self.gamma, _ptr(out.maps_obs), _ptr(out.vec_obs), _ptr(out.maps_next), _ptr(out.vec_next),
+                _ptr(out.iaction), _ptr(out.pointer), _ptr(out.reward), _ptr(out.done), _ptr(out.discount), _ptr(out.steps),
+                self._stream()))
+            self.launch_count += 1
+            return out
         _lib.check(self._lib.ofb_replay_gather(self._h, _ptr(ids), B, _ptr(out.maps_obs), _ptr(out.vec_obs), _ptr(out.maps_next),
                                                _ptr(out.vec_next), _ptr(out.iaction), _ptr(out.pointer), _ptr(out.reward),
                                                _ptr(out.done), self._stream()))
@@ -183,13 +213,14 @@ class PrioritizedReplayMemory(DeviceReplayMemory):
         ...                                           # push as for DeviceReplayMemory
         trainer.replay(trainer.batch_size, memory=memory, beta=0.4)
 
-    The sampler's random stream is Philox keyed by ``seed`` and the number of samples drawn, so a run is reproducible."""
+    The sampler's random stream is Philox keyed by ``seed`` and the number of samples drawn, so a run is reproducible.
+    With ``n_step`` > 1 a transition enters with the largest mass at the push that makes it a candidate (n frames later)."""
 
-    def __init__(self, bg, depth=16, track=None, ships=None, alpha=0.6, eps=1e-6, seed=0):
+    def __init__(self, bg, depth=16, track=None, ships=None, alpha=0.6, eps=1e-6, seed=0, n_step=1, gamma=0.9):
         alpha, eps = float(alpha), float(eps)
         if not (0.0 <= alpha < float("inf")) or not (0.0 <= eps < float("inf")):
             raise Exception("Invalid priorities : need finite alpha >= 0 and eps >= 0, got alpha={} eps={}.".format(alpha, eps))
-        super().__init__(bg, depth=depth, track=track, ships=ships)
+        super().__init__(bg, depth=depth, track=track, ships=ships, n_step=n_step, gamma=gamma)
         cfg = _lib.OfbReplayPrioConfig(alpha=alpha, eps=eps, seed=int(seed) & (2 ** 64 - 1))
         with torch.cuda.device(self.device):
             _lib.check(self._lib.ofb_replay_enable_priorities(self._h, C.byref(cfg)))

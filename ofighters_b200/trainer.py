@@ -224,17 +224,38 @@ class TrainerB200:
         """:237-238.  ``state`` / ``next_state`` = (maps_bits int32 [2,5000], vec float32 [8]) device tensors."""
         self.memory.append([state, iaction, ipointer, reward, next_state, done])
 
-    def td_errors(self, act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done):
+    def td_errors(self, act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, discount=None):
         """Signed TD errors target - prediction at the entries ``replay``'s targets overwrite, with the targets' own fp32
-        arithmetic: (td_act, td_ptr) float32 [B] on the device.  Inputs as ``ofb_trainer_td_targets`` takes them."""
+        arithmetic: (td_act, td_ptr) float32 [B] on the device.  Inputs as ``ofb_trainer_td_targets`` takes them;
+        ``discount`` (float32 [B], an n-step memory's gamma^k) replaces ``gamma`` when it is given."""
         B = act_obs.shape[0]
         td_act = torch.empty((B,), dtype=torch.float32, device=self.device)
         td_ptr = torch.empty((B,), dtype=torch.float32, device=self.device)
-        _lib.check(self._lib.ofb_trainer_td_errors(_ptr(act_obs), _ptr(ptr_obs), _ptr(act_next), _ptr(ptr_next), _ptr(iaction),
-                                                   _ptr(pointer), _ptr(reward), _ptr(done), float(self.gamma), B, _ptr(td_act),
-                                                   _ptr(td_ptr), self._stream()))
+        args = [_ptr(t) for t in (act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done)]
+        if discount is None:
+            _lib.check(self._lib.ofb_trainer_td_errors(*args, float(self.gamma), B, _ptr(td_act), _ptr(td_ptr), self._stream()))
+        else:
+            _lib.check(self._lib.ofb_trainer_td_errors_discounted(*args, _ptr(discount), B, _ptr(td_act), _ptr(td_ptr),
+                                                                  self._stream()))
         self.launch_count += 1
         return td_act, td_ptr
+
+    def _td_targets(self, act_o, ptr_o, act_n, ptr_n, iaction, pointer, reward, done, discount, B):
+        """``ofb_trainer_td_targets`` in place on (act_o, ptr_o); with a ``discount`` [B] its discounted form."""
+        args = [_ptr(t) for t in (act_o, ptr_o, act_n, ptr_n, iaction, pointer, reward, done)]
+        if discount is None:
+            _lib.check(self._lib.ofb_trainer_td_targets(*args, float(self.gamma), B, _ptr(act_o), _ptr(ptr_o), self._stream()))
+        else:
+            _lib.check(self._lib.ofb_trainer_td_targets_discounted(*args, _ptr(discount), B, _ptr(act_o), _ptr(ptr_o),
+                                                                   self._stream()))
+        self.launch_count += 1
+
+    def _check_memory(self, memory):
+        if memory.device != self.device:
+            raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, self.device))
+        if memory.n_step > 1 and float(memory.gamma) != float(self.gamma):
+            raise Exception("Invalid memory : its {}-step returns are discounted by gamma = {} but the trainer's gamma is {}."
+                            .format(memory.n_step, memory.gamma, self.gamma))
 
     def replay(self, batch_size, memory=None, beta=1.0):
         """:240-287.  Targets from predictions on obs and next_obs; like the reference, the fitted INPUTS are the
@@ -243,7 +264,9 @@ class TrainerB200:
         ``random.sample`` draw over its transitions in age order).  With a ``replay.PrioritizedReplayMemory`` the minibatch
         is drawn in proportion to the priorities, the TD errors of the predictions set the drawn transitions' new
         priorities, and the fit weighs each sample by its importance weight, annealed by ``beta`` (ignored otherwise); the
-        History then also reports ``td_error``, the batch mean of |td_act| + |td_ptr|."""
+        History then also reports ``td_error``, the batch mean of |td_act| + |td_ptr|.  With an n-step memory
+        (``memory.n_step`` > 1, whose ``gamma`` must be the trainer's) the targets are R + gamma^k max Q(s_{t+k}) of each
+        sample's window (``ofb_trainer_td_targets_discounted``)."""
         if isinstance(memory, PrioritizedReplayMemory):
             return self._replay_prioritized(batch_size, memory, beta)
         dev = self.device
@@ -260,9 +283,9 @@ class TrainerB200:
             pointer = torch.tensor([[int(m[2][0]), int(m[2][1])] for m in minibatch], dtype=torch.int32, device=dev)
             reward = torch.tensor([float(m[3]) for m in minibatch], dtype=torch.float32, device=dev)
             done = torch.tensor([1 if m[5] else 0 for m in minibatch], dtype=torch.uint8, device=dev)
+            discount = None
         else:
-            if memory.device != dev:
-                raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, dev))
+            self._check_memory(memory)
             batch_size = min(batch_size, len(memory))
             if batch_size < 1:
                 raise Exception("replay on an empty memory")
@@ -271,30 +294,27 @@ class TrainerB200:
             mb = memory.sample(batch_size)
             maps_o, vec_o, maps_n, vec_n = mb.maps_obs, mb.vec_obs, mb.maps_next, mb.vec_next
             iaction, pointer, reward, done = mb.iaction, mb.pointer, mb.reward, mb.done
+            discount = mb.discount if memory.n_step > 1 else None
         act_o, ptr_o = self.predict(maps_o, vec_o)
         act_n, ptr_n = self.predict(maps_n, vec_n)
-        _lib.check(self._lib.ofb_trainer_td_targets(_ptr(act_o), _ptr(ptr_o), _ptr(act_n), _ptr(ptr_n), _ptr(iaction),
-                                                    _ptr(pointer), _ptr(reward), _ptr(done), float(self.gamma), batch_size,
-                                                    _ptr(act_o), _ptr(ptr_o), self._stream()))
-        self.launch_count += 1
+        self._td_targets(act_o, ptr_o, act_n, ptr_n, iaction, pointer, reward, done, discount, batch_size)
         loss = self.fit(maps_n, vec_n, act_o, ptr_o)
         host = loss.cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]]})
 
     def _replay_prioritized(self, batch_size, memory, beta):
-        if memory.device != self.device:
-            raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, self.device))
+        self._check_memory(memory)
         batch_size = int(batch_size)
         if batch_size < 1 or batch_size > self.max_batch:
             raise Exception("Invalid batch : {} samples but the trainer was sized for {}.".format(batch_size, self.max_batch))
         mb = memory.sample_prioritized(batch_size, beta)
         act_o, ptr_o = self.predict(mb.maps_obs, mb.vec_obs)
         act_n, ptr_n = self.predict(mb.maps_next, mb.vec_next)
-        args = [_ptr(t) for t in (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)]
-        td_act, td_ptr = self.td_errors(act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
+        discount = mb.discount if memory.n_step > 1 else None
+        fields = (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
+        td_act, td_ptr = self.td_errors(*fields, discount=discount)
         memory.update_priorities(mb.ids, td_act, td_ptr)
-        _lib.check(self._lib.ofb_trainer_td_targets(*args, float(self.gamma), batch_size, _ptr(act_o), _ptr(ptr_o), self._stream()))
-        self.launch_count += 1
+        self._td_targets(*fields, discount, batch_size)
         loss = self.fit(mb.maps_next, mb.vec_next, act_o, ptr_o, sample_weight=mb.weight)
         host = torch.cat([loss, (td_act.abs() + td_ptr.abs()).mean().reshape(1)]).cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]],
