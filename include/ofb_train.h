@@ -7,7 +7,9 @@
  *        = one optimiser step on  mse(output1) + mse(output2)  with BatchNormalization in
  *          training mode (batch statistics, moving averages updated) and Adam(lr)   :188,308
  * and, for prioritized replay (ofb_replay.h), the sample-weighted fit (ofb_trainer_fit_weighted) and the TD errors that
- * set the priorities (ofb_trainer_td_errors).
+ * set the priorities (ofb_trainer_td_errors); for a target network with Double DQN, targets whose pointer and action are
+ * chosen by the online predictions and scored by the target network's (ofb_trainer_td_targets_double; the reference has
+ * neither, both are opt-in departures).
  *   model weights (save / load_model)                :70,298      -> ofb_trainer_get_weights
  *
  * Conventions are those of ofb.h: int return codes, ofb_last_error(), caller-owned device buffers,
@@ -110,6 +112,28 @@ int ofb_trainer_td_errors_discounted(const float *act_obs_dev, const float *ptr_
                                      const float *ptr_next_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
                                      const float *reward_dev, const uint8_t *done_dev, const float *discount_dev, int batch,
                                      float *td_act_dev, float *td_ptr_dev, void *stream);
+
+/* Double DQN targets (van Hasselt, Guez & Silver 2016) for a target network: the online network's predictions on next_obs
+ * SELECT, the target network's EVALUATE, in one pass over the maps.  Other arguments as ofb_trainer_td_targets_discounted;
+ * discount_dev [B] replaces gamma when it is not NULL.
+ *   act head:      a* = (act_next_online[b][1] > act_next_online[b][0]) ? 1 : 0        (ties to 0, the decode's rule)
+ *                  target[b][iaction[b]]   = r + (g * act_next_target[b][a*]) * keep
+ *   pointer head:  p* = the first flat index (row-major [400][400], as stored) at which ptr_next_online[b] attains its
+ *                  maximum in fmaxf semantics, so a NaN is never selected; p* = 0 when the map holds no non-NaN value.
+ *                  ptr_target[b][px][py]   = r + (g * ptr_next_target[b][p*]) * keep        (the [x][y] entry, as today)
+ * with g = discount ? discount[b] : gamma, keep = done[b] ? 0 : 1 and the same fp32 roundings as ofb_trainer_td_targets
+ * (no fma).  The rest of target_* is a copy of the obs predictions; target_act_dev may alias act_obs_dev and target_ptr_dev
+ * may alias ptr_obs_dev (in place).  td_act_dev / td_ptr_dev (float [B], both or neither NULL) receive target - prediction,
+ * the prediction read before an in-place overwrite, so the prioritized path needs this one pass instead of
+ * ofb_trainer_td_errors + ofb_trainer_td_targets.  ptr_obs_dev, ptr_next_online_dev and target_ptr_dev must be 16-byte
+ * aligned.  With target maps equal to the online maps the results equal ofb_trainer_td_targets[_discounted] and
+ * ofb_trainer_td_errors[_discounted] bit for bit, for maps without NaN and without a +0 / -0 tie at the maximum.
+ * Deterministic, allocates nothing. */
+int ofb_trainer_td_targets_double(const float *act_obs_dev, const float *ptr_obs_dev, const float *act_next_online_dev,
+                                  const float *ptr_next_online_dev, const float *act_next_target_dev,
+                                  const float *ptr_next_target_dev, const int32_t *iaction_dev, const int32_t *pointer_dev,
+                                  const float *reward_dev, const uint8_t *done_dev, float gamma, const float *discount_dev, int batch,
+                                  float *target_act_dev, float *target_ptr_dev, float *td_act_dev, float *td_ptr_dev, void *stream);
 
 /* Flat copies to HOST (synchronise `stream` first): current weights / gradients of the last fit. */
 int ofb_trainer_get_weights(ofb_trainer *t, float *weights_flat_host, void *stream);

@@ -152,6 +152,7 @@ def load():
     lib.ofb_trainer_td_errors.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, C.c_float, i32, vp, vp, vp]
     lib.ofb_trainer_td_targets_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.ofb_trainer_td_errors_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
+    lib.ofb_trainer_td_targets_double.argtypes = [vp] * 10 + [C.c_float, vp, i32] + [vp] * 5
     lib.ofb_trainer_get_weights.argtypes = [vp, vp, vp]
     lib.ofb_trainer_get_grads.argtypes = [vp, vp, vp]
     lib.ofb_trainer_steps.argtypes = [vp]
@@ -177,7 +178,7 @@ def load():
         getattr(lib, name).restype = i32
     for name in ("ofb_trainer_create", "ofb_trainer_destroy", "ofb_trainer_fit", "ofb_trainer_forward",
                  "ofb_trainer_td_targets", "ofb_trainer_fit_weighted", "ofb_trainer_td_errors", "ofb_trainer_get_weights", "ofb_trainer_get_grads",
-                 "ofb_trainer_td_targets_discounted", "ofb_trainer_td_errors_discounted"):
+                 "ofb_trainer_td_targets_discounted", "ofb_trainer_td_errors_discounted", "ofb_trainer_td_targets_double"):
         getattr(lib, name).restype = i32
     for name in ("ofb_policy_create", "ofb_policy_destroy", "ofb_policy_set_engine", "ofb_policy_forward",
                  "ofb_policy_write_actions", "ofb_policy_pack_image", "ofb_policy_debug_tap"):

@@ -3,6 +3,7 @@
 // training mode (reference: agents/qlearnIA_V2.py:123-190 model, :237-287 replay / fit; Keras defaults of SURVEY.md
 // Appendix B).  fp32 NHWC activations, fp64 accumulation of every sum over the batch.  The batch is tiny (8 samples,
 // 3.7 GFLOP per step), so these are plain CUDA-core kernels: one thread per output element, weights in shared memory.
+#include <cooperative_groups.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -741,6 +742,111 @@ __global__ void k_tr_td_errors(const float *__restrict__ act_obs, const float *_
     }
 }
 
+// Double DQN targets (ofb_trainer_td_targets_double): one cluster of DD_CTAS blocks per sample.  Block r of the cluster scans
+// the float4 slice [r, r + 1) * DD_SLICE of the online next map for its (value, first index) maximum -- NaN never compares
+// greater or equal, so it is never chosen -- and, out of place, copies the same slice of ptr_obs to t_ptr.  After a cluster
+// barrier rank 0 combines the partials over DSMEM (the comparator is a total order on (value, -index), so the result does not
+// depend on the order), reads the target network's two selected entries and writes the overwritten entries (after the barrier:
+// the other blocks' copy may cover them) and the TD errors.  No atomics, no global scratch.
+#define DD_CTAS 8
+#define DD_THREADS 512
+#define DD_SLICE (IMG * IMG / 4 / DD_CTAS)      // 5000 float4 per block
+#define DD_NONE 0x7fffffff
+
+__device__ __forceinline__ void dd_take(float v, int i, float &bv, int &bi) {
+    if (v > bv || (v == bv && i < bi)) { bv = v; bi = i; }
+}
+
+__global__ void __cluster_dims__(DD_CTAS, 1, 1) __launch_bounds__(DD_THREADS, 2)
+k_tr_td_targets_double(const float *act_obs, const float *ptr_obs, const float *__restrict__ act_on,
+                       const float *__restrict__ ptr_on, const float *__restrict__ act_tg, const float *__restrict__ ptr_tg,
+                       const int32_t *__restrict__ iaction, const int32_t *__restrict__ pointer, const float *__restrict__ reward,
+                       const uint8_t *__restrict__ done, float gamma, const float *__restrict__ discount, float *t_act, float *t_ptr,
+                       float *__restrict__ td_act, float *__restrict__ td_ptr) {
+    namespace cg = cooperative_groups;
+    cg::cluster_group cluster = cg::this_cluster();
+    const unsigned rank = cluster.block_rank();
+    const long long b = blockIdx.x / DD_CTAS;
+    const long long n = IMG * IMG;
+    const float4 *on4 = reinterpret_cast<const float4 *>(ptr_on + b * n);
+    const float4 *src4 = reinterpret_cast<const float4 *>(ptr_obs + b * n);
+    float4 *dst4 = reinterpret_cast<float4 *>(t_ptr + b * n);
+    const bool copy = t_ptr != ptr_obs;
+    const int lo = rank * DD_SLICE, hi = lo + DD_SLICE;
+    __shared__ float red_v[DD_THREADS / 32];
+    __shared__ int red_i[DD_THREADS / 32];
+    __shared__ float part_v;
+    __shared__ int part_i;
+
+    float bv = -INFINITY;
+    int bi = DD_NONE;
+    for (int base = lo + threadIdx.x; base < hi; base += 4 * DD_THREADS) {
+        float4 v[4];
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const int i = base + k * DD_THREADS;
+            if (i < hi) v[k] = __ldcs(on4 + i);
+        }
+        if (copy) {
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                const int i = base + k * DD_THREADS;
+                if (i < hi) __stcs(dst4 + i, __ldcs(src4 + i));
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const int i = base + k * DD_THREADS;
+            if (i < hi) {
+                dd_take(v[k].x, 4 * i, bv, bi);
+                dd_take(v[k].y, 4 * i + 1, bv, bi);
+                dd_take(v[k].z, 4 * i + 2, bv, bi);
+                dd_take(v[k].w, 4 * i + 3, bv, bi);
+            }
+        }
+    }
+    for (int o = 16; o > 0; o >>= 1) {
+        const float ov = __shfl_xor_sync(0xffffffffu, bv, o);
+        const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
+        dd_take(ov, oi, bv, bi);
+    }
+    if ((threadIdx.x & 31) == 0) { red_v[threadIdx.x >> 5] = bv; red_i[threadIdx.x >> 5] = bi; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        for (int w = 1; w < DD_THREADS / 32; w++) dd_take(red_v[w], red_i[w], bv, bi);
+        part_v = bv;
+        part_i = bi;
+    }
+    cluster.sync();                       // partials visible cluster-wide; every block's copy of t_ptr is done
+    if (rank == 0 && threadIdx.x == 0) {
+        bv = -INFINITY;
+        bi = DD_NONE;
+        for (unsigned r = 0; r < DD_CTAS; r++) {
+            const float v = *cluster.map_shared_rank(&part_v, r);
+            const int i = *cluster.map_shared_rank(&part_i, r);
+            dd_take(v, i, bv, bi);
+        }
+        const int p_star = bi == DD_NONE ? 0 : bi;        // a map without a non-NaN value selects index 0
+        const float keep = done[b] ? 0.0f : 1.0f, r = reward[b];
+        const float g = discount ? discount[b] : gamma;
+        const int a_star = act_on[b * 2 + 1] > act_on[b * 2] ? 1 : 0;    // ties to 0, as the decode
+        const float ta = __fadd_rn(r, __fmul_rn(__fmul_rn(g, act_tg[b * 2 + a_star]), keep));
+        const float tp = __fadd_rn(r, __fmul_rn(__fmul_rn(g, ptr_tg[b * n + p_star]), keep));
+        const int ia = iaction[b];
+        const long long e = (long long)pointer[b * 2] * IMG + pointer[b * 2 + 1];     // [x][y], as k_tr_td_targets
+        const float a0 = act_obs[b * 2], a1 = act_obs[b * 2 + 1], pa = ia ? a1 : a0, pp = ptr_obs[b * n + e];
+        if (td_act) {
+            td_act[b] = __fsub_rn(ta, pa);
+            td_ptr[b] = __fsub_rn(tp, pp);
+        }
+        t_act[b * 2] = a0;
+        t_act[b * 2 + 1] = a1;
+        t_act[b * 2 + ia] = ta;
+        t_ptr[b * n + e] = tp;
+    }
+    cluster.sync();                       // keep every block's shared partial alive until rank 0 has read it
+}
+
 // ---------------------------------------------------------------------------------------------- host side
 static inline unsigned blocks_for(long long n, int threads, long long cap = 148 * 16) {
     long long b = (n + threads - 1) / threads;
@@ -1103,6 +1209,31 @@ extern "C" int ofb_trainer_td_targets_discounted(const float *act_obs, const flo
     if (!discount) { ofb_set_error("ofb_trainer_td_targets_discounted: null discount"); return OFB_E_ARG; }
     return td_targets_impl(act_obs, ptr_obs, act_next, ptr_next, iaction, pointer, reward, done, 0.0f, discount, B, t_act, t_ptr,
                            stream, "ofb_trainer_td_targets_discounted");
+}
+
+extern "C" int ofb_trainer_td_targets_double(const float *act_obs, const float *ptr_obs, const float *act_next_online,
+                                             const float *ptr_next_online, const float *act_next_target,
+                                             const float *ptr_next_target, const int32_t *iaction, const int32_t *pointer,
+                                             const float *reward, const uint8_t *done, float gamma, const float *discount, int B,
+                                             float *t_act, float *t_ptr, float *td_act, float *td_ptr, void *stream) {
+    if (!act_obs || !ptr_obs || !act_next_online || !ptr_next_online || !act_next_target || !ptr_next_target || !iaction ||
+        !pointer || !reward || !done || !t_act || !t_ptr || B < 1) {
+        ofb_set_error("ofb_trainer_td_targets_double: bad argument");
+        return OFB_E_ARG;
+    }
+    if (!td_act != !td_ptr) {
+        ofb_set_error("ofb_trainer_td_targets_double: td_act and td_ptr are both given or both NULL");
+        return OFB_E_ARG;
+    }
+    if (((uintptr_t)ptr_obs | (uintptr_t)ptr_next_online | (uintptr_t)t_ptr) & 15) {
+        ofb_set_error("ofb_trainer_td_targets_double: ptr_obs, ptr_next_online and target_ptr must be 16-byte aligned");
+        return OFB_E_ARG;
+    }
+    k_tr_td_targets_double<<<(unsigned)B * DD_CTAS, DD_THREADS, 0, (cudaStream_t)stream>>>(
+        act_obs, ptr_obs, act_next_online, ptr_next_online, act_next_target, ptr_next_target, iaction, pointer, reward, done, gamma,
+        discount, t_act, t_ptr, td_act, td_ptr);
+    TR_CHECK(cudaGetLastError());
+    return OFB_OK;
 }
 
 static int copy_out(ofb_trainer *t, const float *src, float *dst_host, void *stream, const char *who) {

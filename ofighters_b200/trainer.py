@@ -59,11 +59,37 @@ def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else C.c_void_p(None)
 
 
+def blend_weights(weights, target, tau):
+    """The target network's soft update theta- <- tau * theta + (1 - tau) * theta-, elementwise in fp32 over Keras-layout
+    dicts: tau and 1 - tau are rounded to fp32 once and ``tau * w + (1 - tau) * wt`` is evaluated in that order without
+    fma, so tau = 1 returns ``weights``' values exactly."""
+    a = torch.tensor(float(tau), dtype=torch.float32)
+    b = torch.tensor(1.0 - float(tau), dtype=torch.float32)
+    return {k: a * weights[k].to(torch.float32) + b * target[k].to(torch.float32) for k in weights}
+
+
 class TrainerB200:
     def __init__(self, weights=None, name=None, learning_rate=0.001, epsilon=None, batch_size=30, memory_size=400,
-                 device=None, seed=0, max_ships=64, bn_unbiased_moving_var=False):
+                 device=None, seed=0, max_ships=64, bn_unbiased_moving_var=False, target_update=None, target_tau=1.0,
+                 double_dqn=False):
         """Defaults are the reference constructor's (qlearnIA_V2.py:48); the module-level TRAINER is built with
-        ``learning_rate=0.0001, epsilon=Epsilon_cos(period=110*400), batch_size=8`` (:304-310)."""
+        ``learning_rate=0.0001, epsilon=Epsilon_cos(period=110*400), batch_size=8`` (:304-310).
+
+        Target network (Mnih et al. 2015; the reference has none, so it is off by default): ``target_update=C`` keeps a second
+        inference engine, ``target_model``, whose weights start as the initial ones and, after every optimiser step with
+        ``steps % C == 0``, become ``tau * theta + (1 - tau) * theta-`` (``target_tau``, 0 < tau <= 1; BN moving statistics
+        included).  ``replay`` then bootstraps from the target's predictions on the next observations.  ``double_dqn=True``
+        (needs ``target_update``) lets the online network choose the action and the pointer and the target score them
+        (``ofb_trainer_td_targets_double``).  With ``target_update=None`` every path launches what it launched before."""
+        if target_update is not None:
+            if isinstance(target_update, bool) or int(target_update) != target_update or int(target_update) < 1:
+                raise Exception("Invalid target_update {} : expected an int >= 1 (optimiser steps between refreshes) or None."
+                                .format(target_update))
+            if not 0.0 < float(target_tau) <= 1.0:
+                raise Exception("Invalid target_tau {} : expected 0 < tau <= 1.".format(target_tau))
+        elif double_dqn:
+            raise Exception("Invalid double_dqn : Double DQN scores the online choice with a target network; "
+                            "give target_update too.")
         if not torch.cuda.is_available():
             raise _lib.OfbError("TrainerB200 needs a CUDA device: fit and predict are hand-written sm_100a kernels "
                                 "and have no CPU fallback")
@@ -94,6 +120,14 @@ class TrainerB200:
         self.max_batch = cfg.max_batch
         self.model = PolicyB200(weights, device=self.device, max_ships=max_ships)   # the predict() side
         self._loss = torch.zeros(3, dtype=torch.float32, device=self.device)
+        self.target_update = None if target_update is None else int(target_update)
+        self.target_tau = float(target_tau)
+        self.double_dqn = bool(double_dqn)
+        self.target_model = None
+        self.target_updates = 0
+        if self.target_update is not None:
+            self._target_w = unflatten_weights(flat)      # fp32 host copy of theta-, Keras layouts
+            self.target_model = PolicyB200(self._target_w, device=self.device, max_ships=max_ships)
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -112,6 +146,12 @@ class TrainerB200:
         flat = torch.empty(len_flat(), dtype=torch.float32)
         _lib.check(self._lib.ofb_trainer_get_weights(self._h, C.c_void_p(flat.data_ptr()), self._stream()))
         return unflatten_weights(flat)
+
+    def get_target_weights(self):
+        """The target network's weights theta- (Keras-layout fp32 host copies); needs ``target_update``."""
+        if self.target_model is None:
+            raise Exception("no target network : the trainer was built with target_update=None")
+        return {k: v.clone() for k, v in self._target_w.items()}
 
     def get_grads(self):
         flat = torch.empty(len_flat(), dtype=torch.float32)
@@ -182,8 +222,15 @@ class TrainerB200:
                                                           _ptr(sample_weight), B, _ptr(self._loss), self._stream()))
         self.launch_count += self.KERNELS_PER_FIT
         loss = self._loss.clone()
-        if sync_model:
-            self.sync_model()
+        refresh = self.target_update is not None and self.steps % self.target_update == 0
+        if sync_model or refresh:
+            w = self.get_weights()
+            if sync_model:
+                self.model.load_weights(w)
+            if refresh:                                   # the same host weights feed the target's blend
+                self._target_w = blend_weights(w, self._target_w, self.target_tau)
+                self.target_model.load_weights(self._target_w)
+                self.target_updates += 1
         return loss
 
     KERNELS_PER_FIT = 96          # forward 33 + backward 62 + Adam (memsets not counted)
@@ -250,6 +297,28 @@ class TrainerB200:
                                                                    self._stream()))
         self.launch_count += 1
 
+    def _predict_next(self, maps_n, vec_n):
+        """Predictions on the next observations for the max-bootstrap: the target network's when there is one."""
+        if self.target_model is None:
+            return self.predict(maps_n, vec_n)
+        r = self.target_model.forward(maps_n, vec_n, 1, want_ptr=True)
+        return r["act"], r["ptr"]
+
+    def _td_targets_double(self, act_o, ptr_o, maps_n, vec_n, iaction, pointer, reward, done, discount, B, want_td=False):
+        """Double DQN targets in place on (act_o, ptr_o): the online network selects on the next observations, the target
+        network evaluates.  -> (td_act, td_ptr) float32 [B] of the same pass when ``want_td``, else (None, None)."""
+        act_n, ptr_n = self.predict(maps_n, vec_n)
+        tg = self.target_model.forward(maps_n, vec_n, 1, want_ptr=True)
+        td_act = td_ptr = None
+        if want_td:
+            td_act = torch.empty((B,), dtype=torch.float32, device=self.device)
+            td_ptr = torch.empty((B,), dtype=torch.float32, device=self.device)
+        _lib.check(self._lib.ofb_trainer_td_targets_double(
+            *[_ptr(t) for t in (act_o, ptr_o, act_n, ptr_n, tg["act"], tg["ptr"], iaction, pointer, reward, done)],
+            float(self.gamma), _ptr(discount), B, _ptr(act_o), _ptr(ptr_o), _ptr(td_act), _ptr(td_ptr), self._stream()))
+        self.launch_count += 1
+        return td_act, td_ptr
+
     def _check_memory(self, memory):
         if memory.device != self.device:
             raise Exception("Invalid memory : it lives on {} but the trainer on {}.".format(memory.device, self.device))
@@ -266,7 +335,9 @@ class TrainerB200:
         priorities, and the fit weighs each sample by its importance weight, annealed by ``beta`` (ignored otherwise); the
         History then also reports ``td_error``, the batch mean of |td_act| + |td_ptr|.  With an n-step memory
         (``memory.n_step`` > 1, whose ``gamma`` must be the trainer's) the targets are R + gamma^k max Q(s_{t+k}) of each
-        sample's window (``ofb_trainer_td_targets_discounted``)."""
+        sample's window (``ofb_trainer_td_targets_discounted``).  With a target network (``target_update``) the max-bootstrap
+        reads the target's predictions on the next observations; with ``double_dqn`` the online network selects and the
+        target evaluates (``ofb_trainer_td_targets_double``, which on the prioritized path also gives the TD errors)."""
         if isinstance(memory, PrioritizedReplayMemory):
             return self._replay_prioritized(batch_size, memory, beta)
         dev = self.device
@@ -296,8 +367,11 @@ class TrainerB200:
             iaction, pointer, reward, done = mb.iaction, mb.pointer, mb.reward, mb.done
             discount = mb.discount if memory.n_step > 1 else None
         act_o, ptr_o = self.predict(maps_o, vec_o)
-        act_n, ptr_n = self.predict(maps_n, vec_n)
-        self._td_targets(act_o, ptr_o, act_n, ptr_n, iaction, pointer, reward, done, discount, batch_size)
+        if self.double_dqn:
+            self._td_targets_double(act_o, ptr_o, maps_n, vec_n, iaction, pointer, reward, done, discount, batch_size)
+        else:
+            act_n, ptr_n = self._predict_next(maps_n, vec_n)
+            self._td_targets(act_o, ptr_o, act_n, ptr_n, iaction, pointer, reward, done, discount, batch_size)
         loss = self.fit(maps_n, vec_n, act_o, ptr_o)
         host = loss.cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]]})
@@ -309,12 +383,17 @@ class TrainerB200:
             raise Exception("Invalid batch : {} samples but the trainer was sized for {}.".format(batch_size, self.max_batch))
         mb = memory.sample_prioritized(batch_size, beta)
         act_o, ptr_o = self.predict(mb.maps_obs, mb.vec_obs)
-        act_n, ptr_n = self.predict(mb.maps_next, mb.vec_next)
         discount = mb.discount if memory.n_step > 1 else None
-        fields = (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
-        td_act, td_ptr = self.td_errors(*fields, discount=discount)
-        memory.update_priorities(mb.ids, td_act, td_ptr)
-        self._td_targets(*fields, discount, batch_size)
+        if self.double_dqn:
+            td_act, td_ptr = self._td_targets_double(act_o, ptr_o, mb.maps_next, mb.vec_next, mb.iaction, mb.pointer, mb.reward,
+                                                     mb.done, discount, batch_size, want_td=True)
+            memory.update_priorities(mb.ids, td_act, td_ptr)
+        else:
+            act_n, ptr_n = self._predict_next(mb.maps_next, mb.vec_next)
+            fields = (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
+            td_act, td_ptr = self.td_errors(*fields, discount=discount)
+            memory.update_priorities(mb.ids, td_act, td_ptr)
+            self._td_targets(*fields, discount, batch_size)
         loss = self.fit(mb.maps_next, mb.vec_next, act_o, ptr_o, sample_weight=mb.weight)
         host = torch.cat([loss, (td_act.abs() + td_ptr.abs()).mean().reshape(1)]).cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]],
