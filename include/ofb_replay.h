@@ -131,6 +131,23 @@ int ofb_replay_update_priorities(ofb_replay *r, const int32_t *ids_dev, const fl
  * the fp64 total mass the last ofb_replay_sample_prioritized drew from (double [1]). */
 int ofb_replay_read_priorities(const ofb_replay *r, float *mass_dev, float *max_mass_dev, double *last_total_dev, void *stream);
 
+/* ---- Prioritized replay sharded over W ranks (one memory per rank, one global batch).
+ * Each rank draws its share of the batch from its own memory in proportion to its masses, so transition i of rank r is drawn
+ * with P(i) = m_i / (W M_r) (M_r = the rank's total mass).  Schaul's weights over the union of the memories are then
+ *   w_i = (P(i) / min_j P(j))^(-beta) = ((m_i / M_r) / g)^(-beta),   g = min over ranks of m_min,r / M_r,
+ * i.e. the local weight (m_i / m_min,r)^(-beta) of ofb_replay_sample_prioritized times the rank's factor
+ * ((m_min,r / M_r) / g)^(-beta) <= 1.  Both calls below run on the device without a host synchronisation. */
+
+/* out_dev double [2] = (total mass M_r, smallest non-zero mass m_min,r) of the last ofb_replay_sample_prioritized (undefined
+ * when it found no drawable transition). */
+int ofb_replay_sample_stats(const ofb_replay *r, double *out_dev, void *stream);
+
+/* weight_dev[b] *= ((local_stats[1] / local_stats[0]) / global_ratio[0])^(-beta) for b < batch, the factor in fp64 and the
+ * product rounded once to fp32.  local_stats_dev double [2] from ofb_replay_sample_stats, global_ratio_dev double [1] = g (the
+ * minimum over the ranks of local_stats[1] / local_stats[0]).  Leaves the weights unchanged when a total or g is not > 0. */
+int ofb_replay_rescale_weights(float *weight_dev, int32_t batch, float beta, const double *local_stats_dev,
+                               const double *global_ratio_dev, void *stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -135,7 +135,64 @@ int ofb_trainer_td_targets_double(const float *act_obs_dev, const float *ptr_obs
                                   const float *reward_dev, const uint8_t *done_dev, float gamma, const float *discount_dev, int batch,
                                   float *target_act_dev, float *target_ptr_dev, float *td_act_dev, float *td_ptr_dev, void *stream);
 
-/* Flat copies to HOST (synchronise `stream` first): current weights / gradients of the last fit. */
+/* ---- Data-parallel fit (synchronised BatchNormalization over W ranks).
+ * Each rank holds a replica of the model and a shard of one global batch.  A sharded fit equals the fit of the concatenated
+ * batch: every sum over the batch is accumulated locally into an exchange buffer and summed over the ranks by a caller-supplied
+ * reducer before the kernel that consumes it, and the global sample count replaces B in every normalisation.  Adam then runs
+ * on every rank on identical reduced gradients, so the replicas stay identical without a weight broadcast.
+ *
+ * Exchange buffers (caller-owned device memory, so that a framework can hand them straight to its collectives):
+ *   stats_dev  double [OFB_TRAIN_STATS_LEN]
+ *     [OFB_TRAIN_STATS_FWD + 16 l, +16)   forward BN sums of BN layer l = 0..6 (norm1..norm4, upnorm1..upnorm3):
+ *                                         sum y in channels 0..7, sum y^2 in 8..15 (unused channels stay 0)
+ *     [OFB_TRAIN_STATS_LOSS, +2)          the two loss accumulators: sum of (weighted) squared errors of output1, output2
+ *     [OFB_TRAIN_STATS_BWD + 16 l, +16)   backward BN sums of layer l: sum dz in 0..7, sum dz * xhat in 8..15
+ *   grads_dev  float [OFB_TRAIN_N_PARAMS]   the gradients, flat in the weights' order (get_grads reads them)
+ * Reduce stages, in the order a sharded fit calls the reducer (16 calls per fit):
+ *   OFB_STAGE_FWD_BN + l   for l = 0, 1, ..., 6   (the trunk norm1..norm4, then the pointer head upnorm1..upnorm3)
+ *   OFB_STAGE_LOSS
+ *   OFB_STAGE_BWD_BN + l   for l = 6, 5, ..., 0   (the backward walks the pointer head first, then the trunk)
+ *   OFB_STAGE_GRADS
+ * A reducer call must sum its slice over the ranks in `stream` order (the result in place on every rank) before any later
+ * work on `stream` runs; every rank must see the same sums, bit for bit, for the replicas to stay identical. */
+#define OFB_TRAIN_N_BN 7
+#define OFB_TRAIN_STATS_FWD 0
+#define OFB_TRAIN_STATS_LOSS 112
+#define OFB_TRAIN_STATS_BWD 114
+#define OFB_TRAIN_STATS_LEN 226
+enum {
+    OFB_STAGE_FWD_BN = 0,       /* + layer, 0..6 */
+    OFB_STAGE_LOSS = 7,
+    OFB_STAGE_BWD_BN = 8,       /* + layer, 8..14 */
+    OFB_STAGE_GRADS = 15
+};
+
+/* Use stats_dev / grads_dev (layouts above, both non-NULL, on the trainer's device, valid while set) instead of the handle's
+ * own sums, loss accumulators and gradients; both NULL restores the handle's own buffers.  Every entry point then reads and
+ * writes the caller's buffers; with the handle's own buffers every entry point launches exactly what it launched before. */
+int ofb_trainer_set_exchange(ofb_trainer *t, double *stats_dev, float *grads_dev);
+
+/* Reduce hook: fn(ctx, stage, stream) sums stage's slice of the exchange buffers over the ranks and returns 0, or non-zero
+ * to abort the fit.  fn == NULL removes it.  Only ofb_trainer_fit_shard calls it; ofb_trainer_fit / _weighted / _forward
+ * stay local.  A reducer needs exchange buffers. */
+typedef int (*ofb_reduce_fn)(void *ctx, int stage, void *stream);
+int ofb_trainer_set_reducer(ofb_trainer *t, ofb_reduce_fn fn, void *ctx);
+
+/* One Adam step on a global batch of batch_global samples, of which this rank holds batch_local (1 <= batch_local <=
+ * max_batch, batch_local <= batch_global; batch_global != batch_local needs a reducer).  Arguments as ofb_trainer_fit;
+ * sample_weight_dev float [batch_local] may be NULL (unweighted) or the local samples' weights (ofb_trainer_fit_weighted).
+ * batch_global replaces B in the BN statistics (mean, variance, the n / (n - 1) of bn_unbiased_moving_var), in the BN
+ * backward, in the 2 / n of the losses' gradients and in the reported losses.  Each BN layer's gamma / beta gradients are
+ * written from the LOCAL backward sums, before the BWD_BN reduce, so that the GRADS reduce counts each rank's share once.
+ * loss_dev receives the global batch's losses on every rank.  With W = 1 and no reducer this is ofb_trainer_fit[_weighted]
+ * (same kernels, same arguments).  If the reducer fails the call returns OFB_E_STATE and the trainer's state is undefined:
+ * the moving statistics, the gradients or the exchange buffers may already have changed. */
+int ofb_trainer_fit_shard(ofb_trainer *t, const uint32_t *maps_bits_dev, const float *vec_dev, const float *target_act_dev,
+                          const float *target_ptr_dev, const float *sample_weight_dev, int batch_local, int batch_global,
+                          float *loss_dev, void *stream);
+
+/* Flat copies to HOST (synchronise `stream` first): current weights / gradients of the last fit (the exchange gradients
+ * when exchange buffers are set: after a sharded fit, the reduced ones). */
 int ofb_trainer_get_weights(ofb_trainer *t, float *weights_flat_host, void *stream);
 int ofb_trainer_get_grads(ofb_trainer *t, float *grads_flat_host, void *stream);
 int64_t ofb_trainer_steps(const ofb_trainer *t);   /* optimiser steps taken (Adam's t) */

@@ -67,6 +67,12 @@ class OfbError(RuntimeError):
     pass
 
 
+# include/ofb_train.h: the data-parallel fit's reduce hook and the layout of its fp64 exchange buffer
+REDUCE_FN = C.CFUNCTYPE(C.c_int, C.c_void_p, C.c_int, C.c_void_p)
+TRAIN_N_BN, TRAIN_STATS_FWD, TRAIN_STATS_LOSS, TRAIN_STATS_BWD, TRAIN_STATS_LEN = 7, 0, 112, 114, 226
+STAGE_FWD_BN, STAGE_LOSS, STAGE_BWD_BN, STAGE_GRADS = 0, 7, 8, 15
+
+
 _lib = None
 
 
@@ -153,6 +159,9 @@ def load():
     lib.ofb_trainer_td_targets_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.ofb_trainer_td_errors_discounted.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp]
     lib.ofb_trainer_td_targets_double.argtypes = [vp] * 10 + [C.c_float, vp, i32] + [vp] * 5
+    lib.ofb_trainer_fit_shard.argtypes = [vp, vp, vp, vp, vp, vp, i32, i32, vp, vp]
+    lib.ofb_trainer_set_exchange.argtypes = [vp, vp, vp]
+    lib.ofb_trainer_set_reducer.argtypes = [vp, REDUCE_FN, vp]
     lib.ofb_trainer_get_weights.argtypes = [vp, vp, vp]
     lib.ofb_trainer_get_grads.argtypes = [vp, vp, vp]
     lib.ofb_trainer_steps.argtypes = [vp]
@@ -172,13 +181,17 @@ def load():
     lib.ofb_replay_sample_prioritized.argtypes = [vp, i32, C.c_float, vp, vp, vp, vp]
     lib.ofb_replay_update_priorities.argtypes = [vp, vp, vp, vp, i32, vp]
     lib.ofb_replay_read_priorities.argtypes = [vp, vp, vp, vp, vp]
+    lib.ofb_replay_sample_stats.argtypes = [vp, vp, vp]
+    lib.ofb_replay_rescale_weights.argtypes = [vp, i32, C.c_float, vp, vp, vp]
     for name in ("ofb_replay_create", "ofb_replay_destroy", "ofb_replay_push", "ofb_replay_index", "ofb_replay_gather",
                  "ofb_replay_enable_priorities", "ofb_replay_sample_prioritized", "ofb_replay_update_priorities",
-                 "ofb_replay_read_priorities", "ofb_replay_set_n_step", "ofb_replay_gather_nstep"):
+                 "ofb_replay_read_priorities", "ofb_replay_set_n_step", "ofb_replay_gather_nstep", "ofb_replay_sample_stats",
+                 "ofb_replay_rescale_weights"):
         getattr(lib, name).restype = i32
     for name in ("ofb_trainer_create", "ofb_trainer_destroy", "ofb_trainer_fit", "ofb_trainer_forward",
                  "ofb_trainer_td_targets", "ofb_trainer_fit_weighted", "ofb_trainer_td_errors", "ofb_trainer_get_weights", "ofb_trainer_get_grads",
-                 "ofb_trainer_td_targets_discounted", "ofb_trainer_td_errors_discounted", "ofb_trainer_td_targets_double"):
+                 "ofb_trainer_td_targets_discounted", "ofb_trainer_td_errors_discounted", "ofb_trainer_td_targets_double",
+                 "ofb_trainer_fit_shard", "ofb_trainer_set_exchange", "ofb_trainer_set_reducer"):
         getattr(lib, name).restype = i32
     for name in ("ofb_policy_create", "ofb_policy_destroy", "ofb_policy_set_engine", "ofb_policy_forward",
                  "ofb_policy_write_actions", "ofb_policy_pack_image", "ofb_policy_debug_tap"):

@@ -774,3 +774,41 @@ extern "C" int ofb_replay_read_priorities(const ofb_replay *r, float *mass_dev, 
     if (last_total_dev) OFB_CUDA_CHECK(cudaMemcpyAsync(last_total_dev, &r->stats->total, sizeof(double), cudaMemcpyDeviceToDevice, st));
     return OFB_OK;
 }
+
+// ---------------------------------------------------------------- prioritized replay sharded over ranks
+__global__ void k_prio_sample_stats(const PrioStats *__restrict__ stats, double *__restrict__ out) {
+    out[0] = stats->total;
+    out[1] = (double)stats->mass_min;
+}
+
+// w[b] *= ((m_min / M) / g)^(-beta): Schaul's weight over the union of the ranks' memories (include/ofb_replay.h)
+__global__ void k_prio_rescale(float *__restrict__ w, int B, float beta, const double *__restrict__ local,
+                               const double *__restrict__ g) {
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    const double total = local[0], gr = g[0];
+    if (!(total > 0.0) || !(gr > 0.0)) return;
+    const double f = pow((local[1] / total) / gr, -(double)beta);
+    w[b] = (float)((double)w[b] * f);
+}
+
+extern "C" int ofb_replay_sample_stats(const ofb_replay *r, double *out_dev, void *stream) {
+    if (!r || !out_dev) { ofb_set_error("ofb_replay_sample_stats: null argument"); return OFB_E_ARG; }
+    if (!r->mass) { ofb_set_error("ofb_replay_sample_stats: priorities are not enabled"); return OFB_E_ARG; }
+    OFB_CUDA_CHECK(cudaSetDevice(r->device));
+    k_prio_sample_stats<<<1, 1, 0, (cudaStream_t)stream>>>(r->stats, out_dev);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}
+
+extern "C" int ofb_replay_rescale_weights(float *weight_dev, int32_t batch, float beta, const double *local_stats_dev,
+                                          const double *global_ratio_dev, void *stream) {
+    if (!weight_dev || !local_stats_dev || !global_ratio_dev || batch < 1 || !(beta >= 0.0f && beta <= 3.402823466e38f)) {
+        ofb_set_error("ofb_replay_rescale_weights: bad argument (need buffers, batch >= 1 and a finite beta >= 0)");
+        return OFB_E_ARG;
+    }
+    k_prio_rescale<<<(unsigned)((batch + 127) / 128), 128, 0, (cudaStream_t)stream>>>(weight_dev, batch, beta, local_stats_dev,
+                                                                                    global_ratio_dev);
+    OFB_CUDA_CHECK(cudaGetLastError());
+    return OFB_OK;
+}

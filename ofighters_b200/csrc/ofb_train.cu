@@ -70,6 +70,12 @@ struct ofb_trainer {
     double *loss_acc;                            // [2]
     float *g0, *g1;                              // [B,400,400,8] gradient ping-pong
     float *gu, *dh1, *dd2, *dact, *dcat;         // [B,625] [B,100] [B,50] [B,2] [B,5008]
+    // the buffers every entry point uses: the handle's own (fs = bs = sums, la = loss_acc, gr = grads) or, after
+    // ofb_trainer_set_exchange, the caller's exchange buffers (forward sums, loss accumulators, backward sums, gradients)
+    double *fs, *la, *bs;
+    float *gr;
+    ofb_reduce_fn reducer;
+    void *reducer_ctx;
 };
 
 // ---------------------------------------------------------------------------------------------- small helpers
@@ -291,16 +297,17 @@ __global__ void k_tr_upsample(const float *__restrict__ src, const float *__rest
     }
 }
 
-// y[b, o] = act(sum_i x[b, i] * W[i, o] + bias[o]);  one thread per (b, o)
+// y[b, o] = act(sum_i x[b, i] * W[i, o] + bias[o]);  one thread per (b, o).  Like every element-wise kernel here it strides
+// over the grid: blocks_for caps the grid, so a thread may own several elements at large B.
 __global__ void k_tr_dense_fwd(const float *__restrict__ x, const float *__restrict__ W, const float *__restrict__ bias,
                                float *__restrict__ y, int B, int fin, int fout, int relu) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= B * fout) return;
-    const int b = i / fout, o = i % fout;
-    float acc = bias[o];
-    const float *xp = x + (long long)b * fin;
-    for (int k = 0; k < fin; k++) acc = fmaf(xp[k], W[(long long)k * fout + o], acc);
-    y[i] = relu ? fmaxf(acc, 0.0f) : acc;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * fout; i += (long long)gridDim.x * blockDim.x) {
+        const int b = (int)(i / fout), o = (int)(i % fout);
+        float acc = bias[o];
+        const float *xp = x + (long long)b * fin;
+        for (int k = 0; k < fin; k++) acc = fmaf(xp[k], W[(long long)k * fout + o], acc);
+        y[i] = relu ? fmaxf(acc, 0.0f) : acc;
+    }
 }
 // the same for a long reduction (dense1: 5008 inputs): grid (slices, B), thread o sums its slice of k and adds it to y, which
 // k_tr_bias_fill initialised with the bias; k_tr_relu applies the activation afterwards
@@ -314,29 +321,30 @@ __global__ void k_tr_dense_fwd_splitk(const float *__restrict__ x, const float *
     atomicAdd(&y[b * fout + o], acc);
 }
 __global__ void k_tr_bias_fill(const float *__restrict__ bias, float *__restrict__ y, int B, int fout) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < B * fout) y[i] = bias[i % fout];
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * fout; i += (long long)gridDim.x * blockDim.x)
+        y[i] = bias[i % fout];
 }
 __global__ void k_tr_relu(float *__restrict__ y, int n) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) y[i] = fmaxf(y[i], 0.0f);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        y[i] = fmaxf(y[i], 0.0f);
 }
 __global__ void k_tr_set_vec(const float *__restrict__ vec, float *__restrict__ cat, int B) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < B * 8) cat[(long long)(i / 8) * 5008 + (i % 8)] = vec[i];
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * 8; i += (long long)gridDim.x * blockDim.x)
+        cat[(i / 8) * 5008 + (i % 8)] = vec[i];
 }
 // the 25x25x8 pooled map of sample b lands in cat[b, 8:5008] (Flatten on NHWC, vector first: qlearnIA_V2.py:150-154)
 __global__ void k_tr_flat_to_cat(const float *__restrict__ p4, float *__restrict__ cat, int B) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < B * 5000) cat[(long long)(i / 5000) * 5008 + 8 + (i % 5000)] = p4[i];
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * 5000; i += (long long)gridDim.x * blockDim.x)
+        cat[(i / 5000) * 5008 + 8 + (i % 5000)] = p4[i];
 }
 
 // ---------------------------------------------------------------------------------------------- backward kernels
-// dpred = 2 (pred - target) / n, loss_acc += sum (pred - target)^2
-__global__ void k_tr_mse(const float *__restrict__ pred, const float *__restrict__ target, long long n, float *__restrict__ dpred,
-                         double *__restrict__ loss_acc) {
+// dpred = 2 (pred - target) / n_norm, loss_acc += sum (pred - target)^2 over the n local elements (n_norm: the elements of
+// the global batch; n for a single fit)
+__global__ void k_tr_mse(const float *__restrict__ pred, const float *__restrict__ target, long long n, long long n_norm,
+                         float *__restrict__ dpred, double *__restrict__ loss_acc) {
     double v[1] = {0.0};
-    const float scale = 2.0f / (float)n;
+    const float scale = 2.0f / (float)n_norm;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         const float d = pred[i] - target[i];
         dpred[i] = d * scale;
@@ -346,10 +354,10 @@ __global__ void k_tr_mse(const float *__restrict__ pred, const float *__restrict
 }
 // the same with per-sample weights w[b] over `per` elements each: dpred = 2 w_b (pred - target) / n,
 // loss_acc += sum w_b (pred - target)^2  (so loss_acc / n = (1/B) sum_b w_b mse_b)
-__global__ void k_tr_mse_weighted(const float *__restrict__ pred, const float *__restrict__ target, long long n, long long per,
-                                  const float *__restrict__ w, float *__restrict__ dpred, double *__restrict__ loss_acc) {
+__global__ void k_tr_mse_weighted(const float *__restrict__ pred, const float *__restrict__ target, long long n, long long n_norm,
+                                  long long per, const float *__restrict__ w, float *__restrict__ dpred, double *__restrict__ loss_acc) {
     double v[1] = {0.0};
-    const float scale = 2.0f / (float)n;
+    const float scale = 2.0f / (float)n_norm;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
         const float d = pred[i] - target[i], wb = w[i / per];
         dpred[i] = (d * scale) * wb;
@@ -515,15 +523,16 @@ __global__ void k_tr_bnpool_bwd_reduce(const float *__restrict__ y, const float 
     }
     block_accumulate<16>(v, sums, 16);
 }
-// pass 2: dy[b, y, x, c] = gamma * rstd * (dz - s1 / N - xhat * s2 / N).  One thread per 2x2 window and all 8 channels (the
-// trunk's convolutions all have 8): the window's 4 pixels are read and written as float4 pairs.
+// pass 2: dy[b, y, x, c] = gamma * rstd * (dz - s1 / N - xhat * s2 / N), N = n_norm (the global batch's pixels; B * H * W for
+// a single fit).  One thread per 2x2 window and all 8 channels (the trunk's convolutions all have 8): the window's 4 pixels
+// are read and written as float4 pairs.
 __global__ void k_tr_bnpool_bwd_apply(const float *__restrict__ y, const float *__restrict__ mean, const float *__restrict__ var,
                                       const float *__restrict__ gamma, const float *__restrict__ beta, float eps,
                                       const float *__restrict__ dp, long long dp_stride, const double *__restrict__ sums,
-                                      float *__restrict__ dy, int B, int H, int W) {
+                                      float *__restrict__ dy, int B, int H, int W, long long n_norm) {
     constexpr int C = 8;
     __shared__ float cm[C], cr[C], cg[C], cb[C], c1[C], c2[C];
-    const double inv_n = 1.0 / (double)((long long)B * H * W);
+    const double inv_n = 1.0 / (double)n_norm;
     if (threadIdx.x < C) {
         const int c = threadIdx.x;
         cm[c] = mean[c]; cr[c] = rsqrtf(var[c] + eps); cg[c] = gamma[c]; cb[c] = beta[c];
@@ -586,8 +595,8 @@ __global__ void k_tr_bn_bwd_reduce(const float *__restrict__ y, const float *__r
 }
 __global__ void k_tr_bn_bwd_apply(const float *__restrict__ y, const float *__restrict__ mean, const float *__restrict__ var,
                                   const float *__restrict__ gamma, const float *__restrict__ beta, float eps, float *__restrict__ dz,
-                                  const double *__restrict__ sums, long long n_px, int C) {
-    const double inv_n = 1.0 / (double)n_px;
+                                  const double *__restrict__ sums, long long n_px, int C, long long n_norm) {
+    const double inv_n = 1.0 / (double)n_norm;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n_px * C; i += (long long)gridDim.x * blockDim.x) {
         const int c = (int)(i % C);
         const float m = mean[c], r = rsqrtf(var[c] + eps);
@@ -660,17 +669,17 @@ __global__ void k_tr_dense_bwd_w(const float *__restrict__ x, const float *__res
 // dx[b, i] (+)= sum_o dy[b, o] * W[i, o]
 __global__ void k_tr_dense_bwd_x(const float *__restrict__ dy, const float *__restrict__ W, float *__restrict__ dx, int B, int fin,
                                  int fout, int accumulate) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= (long long)B * fin) return;
-    const int b = (int)(i / fin), k = (int)(i % fin);
-    float s = 0.0f;
-    for (int o = 0; o < fout; o++) s = fmaf(dy[b * fout + o], W[(long long)k * fout + o], s);
-    dx[i] = accumulate ? dx[i] + s : s;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < (long long)B * fin; i += (long long)gridDim.x * blockDim.x) {
+        const int b = (int)(i / fin), k = (int)(i % fin);
+        float s = 0.0f;
+        for (int o = 0; o < fout; o++) s = fmaf(dy[b * fout + o], W[(long long)k * fout + o], s);
+        dx[i] = accumulate ? dx[i] + s : s;
+    }
 }
 // g[i] = (a[i] > 0) ? g[i] : 0     (ReLU backward through the stored activation)
 __global__ void k_tr_relu_mask(const float *__restrict__ a, float *__restrict__ g, long long n) {
-    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && !(a[i] > 0.0f)) g[i] = 0.0f;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x)
+        if (!(a[i] > 0.0f)) g[i] = 0.0f;
 }
 
 // Keras Adam: m = b1 m + (1 - b1) g; v = b2 v + (1 - b2) g^2; p -= lr_t m / (sqrt(v) + eps)
@@ -938,6 +947,9 @@ extern "C" int ofb_trainer_create(const float *w_host, int64_t n_params, const o
         ofb_trainer_destroy(t);
         return OFB_E_CUDA;
     }
+    t->fs = t->bs = t->sums;
+    t->la = t->loss_acc;
+    t->gr = t->grads;
     *out = t;
     return OFB_OK;
 }
@@ -955,12 +967,28 @@ static void conv_bwd(const float *x, const float *dy, const float *w, float *dw,
     if (dx) k_tr_conv_bwd_data<CIN, COUT><<<blocks_for((long long)B * H * W, 256), 256, 0, st>>>(dy, w, dx, B, H, W);
 }
 
-// training-mode forward; update_moving: BatchNormalization's moving averages follow the batch statistics
-static int forward_train(ofb_trainer *t, const uint32_t *maps, const float *vec, int B, int update_moving, cudaStream_t st) {
+// The reducer's call for one stage of a sharded fit (no-op for a local fit).
+static int reduce_stage(ofb_trainer *t, int shard, int stage, cudaStream_t st) {
+    if (!shard || !t->reducer) return OFB_OK;
+    const int r = t->reducer(t->reducer_ctx, stage, (void *)st);
+    if (r != 0) {
+        ofb_set_error("ofb_trainer_fit_shard: the reducer failed at stage %d (returned %d); the trainer's state is undefined",
+                      stage, r);
+        return OFB_E_STATE;
+    }
+    return OFB_OK;
+}
+
+// training-mode forward on the B local samples; update_moving: BatchNormalization's moving averages follow the batch
+// statistics.  Bn: the samples the statistics are over (B for a local forward); shard: the forward of a sharded fit, whose
+// per-layer sums the reducer sums over the ranks (stage FWD_BN + layer) before they are consumed.
+static int forward_train(ofb_trainer *t, const uint32_t *maps, const float *vec, int B, int Bn, int shard, int update_moving,
+                         cudaStream_t st) {
     const Table &T = t->tab;
     float *P = t->params;
     const float eps = t->cfg.bn_eps;
-    TR_CHECK(cudaMemsetAsync(t->sums, 0, 7 * 16 * sizeof(double), st));
+    int rc;
+    TR_CHECK(cudaMemsetAsync(t->fs, 0, 7 * 16 * sizeof(double), st));
     k_tr_unpack<<<blocks_for((long long)B * IMG * IMG, 256), 256, 0, st>>>(maps, t->x0, (long long)B * IMG * IMG);
     const int Hs[4] = {400, 200, 100, 50};
     for (int i = 0; i < 4; i++) {
@@ -970,9 +998,10 @@ static int forward_train(ofb_trainer *t, const uint32_t *maps, const float *vec,
         if (i == 0) conv_fwd<2, 8>(in, P + c.k.off, P + c.b.off, t->y[i], B, H, H, st);
         else conv_fwd<8, 8>(in, P + c.k.off, P + c.b.off, t->y[i], B, H, H, st);
         const long long npx = (long long)B * H * H;
-        k_tr_chan_sums<<<blocks_for(npx, 256, 148 * 4), 256, 0, st>>>(t->y[i], npx, 8, t->sums + i * 16);
-        k_tr_bn_finalize<<<1, 32, 0, st>>>(t->sums + i * 16, npx, 8, t->bn_mean + i * 8, t->bn_var + i * 8, P + c.m.off, P + c.v.off,
-                                         t->cfg.bn_momentum, t->cfg.bn_unbiased_moving_var, update_moving);
+        k_tr_chan_sums<<<blocks_for(npx, 256, 148 * 4), 256, 0, st>>>(t->y[i], npx, 8, t->fs + i * 16);
+        if ((rc = reduce_stage(t, shard, OFB_STAGE_FWD_BN + i, st)) != OFB_OK) return rc;
+        k_tr_bn_finalize<<<1, 32, 0, st>>>(t->fs + i * 16, (long long)Bn * H * H, 8, t->bn_mean + i * 8, t->bn_var + i * 8, P + c.m.off,
+                                         P + c.v.off, t->cfg.bn_momentum, t->cfg.bn_unbiased_moving_var, update_moving);
         k_tr_bn_relu_pool<<<blocks_for(npx * 2, 256), 256, 0, st>>>(t->y[i], t->bn_mean + i * 8, t->bn_var + i * 8, P + c.g.off,
                                                                     P + c.be.off, eps, t->p[i], B, H, H, 8);
     }
@@ -1005,9 +1034,11 @@ static int forward_train(ofb_trainer *t, const uint32_t *maps, const float *vec,
         else conv_fwd<8, 1>(t->a[j], P + c.k.off, P + c.b.off, t->yu[j], B, H, H, st);
         if (c.bn) {
             const long long npx = (long long)B * H * H;
-            k_tr_chan_sums<<<blocks_for(npx, 256, 148 * 4), 256, 0, st>>>(t->yu[j], npx, c.cout, t->sums + (4 + j) * 16);
-            k_tr_bn_finalize<<<1, 32, 0, st>>>(t->sums + (4 + j) * 16, npx, c.cout, t->bn_mean + (4 + j) * 8, t->bn_var + (4 + j) * 8,
-                                             P + c.m.off, P + c.v.off, t->cfg.bn_momentum, t->cfg.bn_unbiased_moving_var, update_moving);
+            k_tr_chan_sums<<<blocks_for(npx, 256, 148 * 4), 256, 0, st>>>(t->yu[j], npx, c.cout, t->fs + (4 + j) * 16);
+            if ((rc = reduce_stage(t, shard, OFB_STAGE_FWD_BN + 4 + j, st)) != OFB_OK) return rc;
+            k_tr_bn_finalize<<<1, 32, 0, st>>>(t->fs + (4 + j) * 16, (long long)Bn * H * H, c.cout, t->bn_mean + (4 + j) * 8,
+                                             t->bn_var + (4 + j) * 8, P + c.m.off, P + c.v.off, t->cfg.bn_momentum,
+                                             t->cfg.bn_unbiased_moving_var, update_moving);
         }
     }
     TR_CHECK(cudaGetLastError());
@@ -1031,39 +1062,43 @@ extern "C" int ofb_trainer_forward(ofb_trainer *t, const uint32_t *maps, const f
     if (!maps || !vec) { ofb_set_error("ofb_trainer_forward: null input"); return OFB_E_ARG; }
     TR_CHECK(cudaSetDevice(t->device));
     cudaStream_t st = (cudaStream_t)stream;
-    rc = forward_train(t, maps, vec, B, 0, st);
+    rc = forward_train(t, maps, vec, B, B, 0, 0, st);
     if (rc != OFB_OK) return rc;
     if (act_dev) TR_CHECK(cudaMemcpyAsync(act_dev, t->act, (size_t)B * 2 * sizeof(float), cudaMemcpyDeviceToDevice, st));
     if (ptr_dev) TR_CHECK(cudaMemcpyAsync(ptr_dev, t->yu[3], (size_t)B * IMG * IMG * sizeof(float), cudaMemcpyDeviceToDevice, st));
     return OFB_OK;
 }
 
-// one Adam step; sample_weight == NULL: today's unweighted loss, with the kernels of ofb_trainer_fit unchanged
+// one Adam step on the B local samples of a batch of Bn; sample_weight == NULL: today's unweighted loss, with the kernels of
+// ofb_trainer_fit unchanged.  shard: a sharded fit (ofb_trainer_fit_shard): the reducer sums every accumulated slice over
+// the ranks before it is consumed, and each BN layer's gamma / beta gradients are taken from the local backward sums.
 static int fit_impl(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act, const float *target_ptr,
-                    const float *sample_weight, int B, float *loss_dev, void *stream) {
+                    const float *sample_weight, int B, int Bn, int shard, float *loss_dev, void *stream) {
     int rc;
     TR_CHECK(cudaSetDevice(t->device));
     cudaStream_t st = (cudaStream_t)stream;
     const Table &T = t->tab;
-    float *P = t->params, *G = t->grads;
+    float *P = t->params, *G = t->gr;
     const float eps = t->cfg.bn_eps;
-    rc = forward_train(t, maps, vec, B, 1, st);
+    rc = forward_train(t, maps, vec, B, Bn, shard, 1, st);
     if (rc != OFB_OK) return rc;
     TR_CHECK(cudaMemsetAsync(G, 0, (size_t)T.total * sizeof(float), st));
-    TR_CHECK(cudaMemsetAsync(t->sums, 0, 7 * 16 * sizeof(double), st));
-    TR_CHECK(cudaMemsetAsync(t->loss_acc, 0, 2 * sizeof(double), st));
+    TR_CHECK(cudaMemsetAsync(t->bs, 0, 7 * 16 * sizeof(double), st));
+    TR_CHECK(cudaMemsetAsync(t->la, 0, 2 * sizeof(double), st));
 
-    // ---- losses: mse(output1) + mse(output2), each a mean over all of its elements
+    // ---- losses: mse(output1) + mse(output2), each a mean over all of its elements (of the global batch)
     const long long n_act = (long long)B * 2, n_ptr = (long long)B * IMG * IMG;
+    const long long N_act = (long long)Bn * 2, N_ptr = (long long)Bn * IMG * IMG;
     if (!sample_weight) {
-        k_tr_mse<<<1, 64, 0, st>>>(t->act, target_act, n_act, t->dact, t->loss_acc);
-        k_tr_mse<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, t->g0, t->loss_acc + 1);
+        k_tr_mse<<<1, 64, 0, st>>>(t->act, target_act, n_act, N_act, t->dact, t->la);
+        k_tr_mse<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, N_ptr, t->g0, t->la + 1);
     } else {
-        k_tr_mse_weighted<<<1, 64, 0, st>>>(t->act, target_act, n_act, 2, sample_weight, t->dact, t->loss_acc);
-        k_tr_mse_weighted<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, IMG * IMG, sample_weight, t->g0,
-                                                                          t->loss_acc + 1);
+        k_tr_mse_weighted<<<1, 64, 0, st>>>(t->act, target_act, n_act, N_act, 2, sample_weight, t->dact, t->la);
+        k_tr_mse_weighted<<<blocks_for(n_ptr, 256, 148 * 4), 256, 0, st>>>(t->yu[3], target_ptr, n_ptr, N_ptr, IMG * IMG, sample_weight,
+                                                                          t->g0, t->la + 1);
     }
-    if (loss_dev) k_tr_loss_out<<<1, 1, 0, st>>>(t->loss_acc, n_act, n_ptr, loss_dev);
+    if ((rc = reduce_stage(t, shard, OFB_STAGE_LOSS, st)) != OFB_OK) return rc;
+    if (loss_dev) k_tr_loss_out<<<1, 1, 0, st>>>(t->la, N_act, N_ptr, loss_dev);
 
     // ---- pointer head, top down.  g0 holds the gradient w.r.t. the stage's conv output, g1 w.r.t. its (upsampled) input.
     const int hs[4] = {25, 50, 100, 200}, cin[4] = {1, 2, 4, 8};
@@ -1072,13 +1107,17 @@ static int fit_impl(ofb_trainer *t, const uint32_t *maps, const float *vec, cons
         const int h = hs[j], H = 2 * h;
         const long long npx = (long long)B * H * H;
         if (c.bn) {       // g0 = d relu(bn(yu[j])) -> d yu[j]
-            double *s = t->sums + (4 + j) * 16;
+            double *s = t->bs + (4 + j) * 16;
             const float *mean = t->bn_mean + (4 + j) * 8, *var = t->bn_var + (4 + j) * 8;
             k_tr_bn_bwd_reduce<<<blocks_for(npx, 256, 148 * 4), 256, 0, st>>>(t->yu[j], mean, var, P + c.g.off, P + c.be.off, eps, t->g0, npx,
                                                                               c.cout, s);
+            if (shard) {  // local gamma / beta gradients, before the sums become global
+                k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, c.cout, G + c.g.off, G + c.be.off);
+                if ((rc = reduce_stage(t, shard, OFB_STAGE_BWD_BN + 4 + j, st)) != OFB_OK) return rc;
+            }
             k_tr_bn_bwd_apply<<<blocks_for(npx * c.cout, 256), 256, 0, st>>>(t->yu[j], mean, var, P + c.g.off, P + c.be.off, eps, t->g0, s,
-                                                                             npx, c.cout);
-            k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, c.cout, G + c.g.off, G + c.be.off);
+                                                                             npx, c.cout, (long long)Bn * H * H);
+            if (!shard) k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, c.cout, G + c.g.off, G + c.be.off);
         }
         if (j == 3) conv_bwd<8, 1>(t->a[j], t->g0, P + c.k.off, G + c.k.off, G + c.b.off, t->g1, B, H, H, st);
         else if (j == 2) conv_bwd<4, 8>(t->a[j], t->g0, P + c.k.off, G + c.k.off, G + c.b.off, t->g1, B, H, H, st);
@@ -1112,19 +1151,24 @@ static int fit_impl(ofb_trainer *t, const uint32_t *maps, const float *vec, cons
         const ConvP &c = T.conv[i];
         const int H = Hs[i];
         const long long npx = (long long)B * H * H;
-        double *s = t->sums + i * 16;
+        double *s = t->bs + i * 16;
         const float *mean = t->bn_mean + i * 8, *var = t->bn_var + i * 8;
         k_tr_bnpool_bwd_reduce<<<blocks_for(npx / 4, 256, 148 * 4), 256, 0, st>>>(t->y[i], mean, var, P + c.g.off, P + c.be.off, eps, dp,
                                                                                   dp_stride, B, H, H, 8, s);
+        if (shard) {
+            k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, 8, G + c.g.off, G + c.be.off);
+            if ((rc = reduce_stage(t, shard, OFB_STAGE_BWD_BN + i, st)) != OFB_OK) return rc;
+        }
         k_tr_bnpool_bwd_apply<<<blocks_for(npx / 4, 128), 128, 0, st>>>(t->y[i], mean, var, P + c.g.off, P + c.be.off, eps, dp, dp_stride, s,
-                                                                        t->g1, B, H, H);
-        k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, 8, G + c.g.off, G + c.be.off);
+                                                                        t->g1, B, H, H, (long long)Bn * H * H);
+        if (!shard) k_tr_bn_param_grads<<<1, 32, 0, st>>>(s, 8, G + c.g.off, G + c.be.off);
         if (i == 0) conv_bwd<2, 8>(t->x0, t->g1, P + c.k.off, G + c.k.off, G + c.b.off, nullptr, B, H, H, st);
         else conv_bwd<8, 8>(t->p[i - 1], t->g1, P + c.k.off, G + c.k.off, G + c.b.off, t->g0, B, H, H, st);
         dp = t->g0;                                      // d p[i-1]: [B, H, H, 8] = the pooled output of layer i - 1
         dp_stride = (long long)H * H * 8;
     }
-    // ---- Adam
+    // ---- Adam, on the gradients of the global batch
+    if ((rc = reduce_stage(t, shard, OFB_STAGE_GRADS, st)) != OFB_OK) return rc;
     t->steps += 1;
     const double b1 = t->cfg.beta1, b2 = t->cfg.beta2;
     const float lr_t = (float)((double)t->cfg.lr * sqrt(1.0 - pow(b2, (double)t->steps)) / (1.0 - pow(b1, (double)t->steps)));
@@ -1139,7 +1183,7 @@ extern "C" int ofb_trainer_fit(ofb_trainer *t, const uint32_t *maps, const float
     int rc = check_batch(t, B, "ofb_trainer_fit");
     if (rc != OFB_OK) return rc;
     if (!maps || !vec || !target_act || !target_ptr) { ofb_set_error("ofb_trainer_fit: null argument"); return OFB_E_ARG; }
-    return fit_impl(t, maps, vec, target_act, target_ptr, nullptr, B, loss_dev, stream);
+    return fit_impl(t, maps, vec, target_act, target_ptr, nullptr, B, B, 0, loss_dev, stream);
 }
 
 extern "C" int ofb_trainer_fit_weighted(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act,
@@ -1150,7 +1194,61 @@ extern "C" int ofb_trainer_fit_weighted(ofb_trainer *t, const uint32_t *maps, co
         ofb_set_error("ofb_trainer_fit_weighted: null argument");
         return OFB_E_ARG;
     }
-    return fit_impl(t, maps, vec, target_act, target_ptr, sample_weight, B, loss_dev, stream);
+    return fit_impl(t, maps, vec, target_act, target_ptr, sample_weight, B, B, 0, loss_dev, stream);
+}
+
+extern "C" int ofb_trainer_fit_shard(ofb_trainer *t, const uint32_t *maps, const float *vec, const float *target_act,
+                                     const float *target_ptr, const float *sample_weight, int B, int Bn, float *loss_dev, void *stream) {
+    int rc = check_batch(t, B, "ofb_trainer_fit_shard");
+    if (rc != OFB_OK) return rc;
+    if (!maps || !vec || !target_act || !target_ptr) { ofb_set_error("ofb_trainer_fit_shard: null argument"); return OFB_E_ARG; }
+    if (Bn < B) {
+        ofb_set_error("ofb_trainer_fit_shard: batch_global %d is smaller than batch_local %d", Bn, B);
+        return OFB_E_ARG;
+    }
+    if (Bn != B && !t->reducer) {
+        ofb_set_error("ofb_trainer_fit_shard: batch_global %d != batch_local %d needs a reducer (ofb_trainer_set_reducer)", Bn, B);
+        return OFB_E_ARG;
+    }
+    if (t->reducer && t->fs == t->sums) {
+        ofb_set_error("ofb_trainer_fit_shard: a reducer needs exchange buffers (ofb_trainer_set_exchange)");
+        return OFB_E_ARG;
+    }
+    return fit_impl(t, maps, vec, target_act, target_ptr, sample_weight, B, Bn, 1, loss_dev, stream);
+}
+
+extern "C" int ofb_trainer_set_exchange(ofb_trainer *t, double *stats_dev, float *grads_dev) {
+    if (!t) { ofb_set_error("ofb_trainer_set_exchange: null handle"); return OFB_E_ARG; }
+    if (!stats_dev != !grads_dev) {
+        ofb_set_error("ofb_trainer_set_exchange: stats_dev and grads_dev are both given or both NULL");
+        return OFB_E_ARG;
+    }
+    if (!stats_dev && t->reducer) {
+        ofb_set_error("ofb_trainer_set_exchange: remove the reducer before the exchange buffers");
+        return OFB_E_ARG;
+    }
+    if (stats_dev) {
+        t->fs = stats_dev + OFB_TRAIN_STATS_FWD;
+        t->la = stats_dev + OFB_TRAIN_STATS_LOSS;
+        t->bs = stats_dev + OFB_TRAIN_STATS_BWD;
+        t->gr = grads_dev;
+    } else {
+        t->fs = t->bs = t->sums;
+        t->la = t->loss_acc;
+        t->gr = t->grads;
+    }
+    return OFB_OK;
+}
+
+extern "C" int ofb_trainer_set_reducer(ofb_trainer *t, ofb_reduce_fn fn, void *ctx) {
+    if (!t) { ofb_set_error("ofb_trainer_set_reducer: null handle"); return OFB_E_ARG; }
+    if (fn && t->fs == t->sums) {
+        ofb_set_error("ofb_trainer_set_reducer: a reducer needs exchange buffers (ofb_trainer_set_exchange)");
+        return OFB_E_ARG;
+    }
+    t->reducer = fn;
+    t->reducer_ctx = fn ? ctx : nullptr;
+    return OFB_OK;
 }
 
 static int td_errors_impl(const float *act_obs, const float *ptr_obs, const float *act_next, const float *ptr_next,
@@ -1247,6 +1345,6 @@ extern "C" int ofb_trainer_get_weights(ofb_trainer *t, float *out_host, void *st
     return copy_out(t, t ? t->params : nullptr, out_host, stream, "ofb_trainer_get_weights");
 }
 extern "C" int ofb_trainer_get_grads(ofb_trainer *t, float *out_host, void *stream) {
-    return copy_out(t, t ? t->grads : nullptr, out_host, stream, "ofb_trainer_get_grads");
+    return copy_out(t, t ? t->gr : nullptr, out_host, stream, "ofb_trainer_get_grads");
 }
 extern "C" int64_t ofb_trainer_steps(const ofb_trainer *t) { return t ? t->steps : -1; }

@@ -188,12 +188,14 @@ class DeviceReplayMemory:
         self.launch_count += 1
         return out
 
-    def sample(self, batch_size):
-        """``random.sample(range(len(self)), batch_size)`` -- the draw ``Trainer.replay`` makes on its deque -- gathered."""
+    def sample(self, batch_size, rng=None):
+        """``random.sample(range(len(self)), batch_size)`` -- the draw ``Trainer.replay`` makes on its deque -- gathered.
+        ``rng``: a ``random.Random`` to draw with instead of the module's shared state (each rank of a data-parallel trainer
+        keeps its own)."""
         n = len(self)
         if n < 1:
             raise Exception("sample on an empty replay memory")
-        return self.gather(random.sample(range(n), batch_size))
+        return self.gather((random if rng is None else rng).sample(range(n), batch_size))
 
 
 class EmptyReplayMemory(Exception):
@@ -281,6 +283,28 @@ class PrioritizedReplayMemory(DeviceReplayMemory):
         out = torch.empty((1,), dtype=torch.float32, device=self.device)
         _lib.check(self._lib.ofb_replay_read_priorities(self._h, None, _ptr(out), None, self._stream()))
         return out
+
+    def sample_stats(self):
+        """Device copy of (total mass, smallest non-zero mass) of the last ``sample_prioritized`` (float64 [2]), what the
+        ranks of a data-parallel replay combine into Schaul's weights over all their memories.  No host synchronisation."""
+        out = torch.empty((2,), dtype=torch.float64, device=self.device)
+        _lib.check(self._lib.ofb_replay_sample_stats(self._h, _ptr(out), self._stream()))
+        self.launch_count += 1
+        return out
+
+    def rescale_weights(self, weight, beta, local_stats, global_ratio):
+        """In place on ``weight`` (float32 [B] from ``sample_prioritized`` with the same ``beta``): the factor
+        ((m_min / M) / g) ** -beta that turns this memory's importance weights into those over the union of the ranks'
+        memories (include/ofb_replay.h).  ``local_stats``: ``sample_stats()``; ``global_ratio``: float64 [1], g = the
+        minimum over the ranks of m_min / M.  Device only."""
+        for name, t, dt, n in (("weight", weight, torch.float32, None), ("local_stats", local_stats, torch.float64, 2),
+                               ("global_ratio", global_ratio, torch.float64, 1)):
+            if not isinstance(t, torch.Tensor) or t.dtype != dt or t.device != self.device or not t.is_contiguous() or \
+                    t.dim() != 1 or (n is not None and t.numel() != n):
+                raise Exception("Invalid {} : expected a contiguous 1-d {} tensor on {}.".format(name, dt, self.device))
+        _lib.check(self._lib.ofb_replay_rescale_weights(_ptr(weight), weight.numel(), float(beta), _ptr(local_stats),
+                                                        _ptr(global_ratio), self._stream()))
+        self.launch_count += 1
 
     def last_total(self):
         """Device copy of the fp64 total mass the last ``sample_prioritized`` drew from (float64 [1])."""

@@ -54,6 +54,37 @@ def broadcast_weights(flat, src=0, group=None):
     return dist.broadcast(flat, src=src, group=group)
 
 
+class DistReducer:
+    """The reducer of a data-parallel ``TrainerB200`` (``reducer=``) over a ``torch.distributed`` process group: every rank
+    of ``group`` builds its trainer with one.  ``all_reduce`` sums (or takes the minimum / maximum) in place, ordered after
+    the work queued on the current stream -- what the trainer's reduce hook needs, since the fit's kernels run on that
+    stream.  NCCL gives every rank the same bits.  Create the group with a ``timeout``, so that a rank that stops calling
+    fails the others instead of hanging them.
+
+        dist.init_process_group("nccl", timeout=datetime.timedelta(seconds=120))
+        trainer = TrainerB200(weights, batch_size=8, reducer=DistReducer())
+    """
+
+    _OPS = {"sum": "SUM", "min": "MIN", "max": "MAX"}
+
+    def __init__(self, group=None):
+        if not (dist.is_available() and dist.is_initialized()):
+            raise Exception("DistReducer needs an initialised torch.distributed process group.")
+        self.group = group
+        self.rank = dist.get_rank(group)
+        self.world = dist.get_world_size(group)
+
+    def all_reduce(self, tensor, op="sum"):
+        if op not in self._OPS:
+            raise Exception("Invalid op {} : expected one of {}.".format(op, sorted(self._OPS)))
+        dist.all_reduce(tensor, op=getattr(dist.ReduceOp, self._OPS[op]), group=self.group)
+
+    def broadcast(self, tensor, src=0):
+        """``tensor`` of group rank ``src`` to every rank, in place."""
+        g_src = src if self.group is None else dist.get_global_rank(self.group, src)
+        dist.broadcast(tensor, src=g_src, group=self.group)
+
+
 def stats_dict(stats):
     v = stats.detach().cpu().tolist()
     return dict(zip(STAT_NAMES, v))

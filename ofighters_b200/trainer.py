@@ -28,7 +28,7 @@ import torch
 from . import _lib
 from .epsilon import Epsilon_cos, Epsilon_decay, EpsilonSchedule  # noqa: F401  (re-exported: Trainer(epsilon=Epsilon_cos(...)))
 from .policy import WEIGHT_SPEC, PolicyB200, keras_default_weights
-from .replay import EmptyReplayMemory, PrioritizedReplayMemory
+from .replay import DeviceReplayMemory, EmptyReplayMemory, PrioritizedReplayMemory
 
 
 def flatten_weights(weights):
@@ -71,7 +71,7 @@ def blend_weights(weights, target, tau):
 class TrainerB200:
     def __init__(self, weights=None, name=None, learning_rate=0.001, epsilon=None, batch_size=30, memory_size=400,
                  device=None, seed=0, max_ships=64, bn_unbiased_moving_var=False, target_update=None, target_tau=1.0,
-                 double_dqn=False):
+                 double_dqn=False, reducer=None):
         """Defaults are the reference constructor's (qlearnIA_V2.py:48); the module-level TRAINER is built with
         ``learning_rate=0.0001, epsilon=Epsilon_cos(period=110*400), batch_size=8`` (:304-310).
 
@@ -80,7 +80,15 @@ class TrainerB200:
         ``steps % C == 0``, become ``tau * theta + (1 - tau) * theta-`` (``target_tau``, 0 < tau <= 1; BN moving statistics
         included).  ``replay`` then bootstraps from the target's predictions on the next observations.  ``double_dqn=True``
         (needs ``target_update``) lets the online network choose the action and the pointer and the target score them
-        (``ofb_trainer_td_targets_double``).  With ``target_update=None`` every path launches what it launched before."""
+        (``ofb_trainer_td_targets_double``).  With ``target_update=None`` every path launches what it launched before.
+
+        Data-parallel learning (the reference has one trainer on one machine; opt-in): ``reducer`` is an object with
+        ``rank``, ``world``, ``all_reduce(tensor, op="sum")`` (in place, in the current stream's order; ops "sum" and "min") and
+        ``broadcast(tensor, src=0)`` -- ``sharding.DistReducer`` over ``torch.distributed``.  Every rank then builds its trainer
+        with the same arguments; rank 0's initial weights are broadcast, ``fit`` is one Adam step on the union of the ranks'
+        batches (``ofb_trainer_fit_shard``: BatchNormalization statistics, losses and gradients summed over the ranks, so the
+        replicas stay identical) and ``replay`` with a ``DeviceReplayMemory`` draws ``batch_size`` transitions from each rank's
+        own memory.  Both are collective: every rank must call them at the same point."""
         if target_update is not None:
             if isinstance(target_update, bool) or int(target_update) != target_update or int(target_update) < 1:
                 raise Exception("Invalid target_update {} : expected an int >= 1 (optimiser steps between refreshes) or None."
@@ -108,6 +116,17 @@ class TrainerB200:
         self.launch_count = 0
         weights = weights if weights is not None else keras_default_weights(seed)
         flat = flatten_weights(weights)
+        self.reducer = reducer
+        self.rank = int(reducer.rank) if reducer is not None else 0
+        self.world = int(reducer.world) if reducer is not None else 1
+        if reducer is not None:                           # one set of initial weights: rank 0's
+            flat_dev = flat.to(self.device)
+            reducer.broadcast(flat_dev, src=0)
+            flat = flat_dev.cpu()
+            weights = unflatten_weights(flat)
+        # per-rank stream of the uniform draws of a sharded replay (ranks drawing the same positions would draw the same
+        # frame, arena and ship of their own memories)
+        self._rng = random.Random("ofighters-dp-replay:%d:%d" % (int(seed), self.rank))
         cfg = _lib.OfbTrainConfig()
         self._lib.ofb_train_default_config(C.byref(cfg))
         cfg.lr = float(learning_rate)
@@ -118,6 +137,13 @@ class TrainerB200:
                                                 self.device.index or 0, C.byref(h)))
         self._h = h
         self.max_batch = cfg.max_batch
+        self._reduce_error = None
+        if reducer is not None:                           # caller-owned exchange buffers, summed by the reducer's callback
+            self._xstats = torch.zeros(_lib.TRAIN_STATS_LEN, dtype=torch.float64, device=self.device)
+            self._xgrads = torch.zeros(flat.numel(), dtype=torch.float32, device=self.device)
+            _lib.check(self._lib.ofb_trainer_set_exchange(h, _ptr(self._xstats), _ptr(self._xgrads)))
+            self._reduce_cb = _lib.REDUCE_FN(self._on_reduce)      # kept alive as long as the handle
+            _lib.check(self._lib.ofb_trainer_set_reducer(h, self._reduce_cb, None))
         self.model = PolicyB200(weights, device=self.device, max_ships=max_ships)   # the predict() side
         self._loss = torch.zeros(3, dtype=torch.float32, device=self.device)
         self.target_update = None if target_update is None else int(target_update)
@@ -140,6 +166,36 @@ class TrainerB200:
 
     def _stream(self):
         return C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+
+    def _exchange_slice(self, stage):
+        """The slice of the exchange buffers a reduce stage sums (include/ofb_train.h)."""
+        if _lib.STAGE_FWD_BN <= stage < _lib.STAGE_FWD_BN + _lib.TRAIN_N_BN:
+            o = _lib.TRAIN_STATS_FWD + 16 * (stage - _lib.STAGE_FWD_BN)
+            return self._xstats[o:o + 16]
+        if stage == _lib.STAGE_LOSS:
+            return self._xstats[_lib.TRAIN_STATS_LOSS:_lib.TRAIN_STATS_LOSS + 2]
+        if _lib.STAGE_BWD_BN <= stage < _lib.STAGE_BWD_BN + _lib.TRAIN_N_BN:
+            o = _lib.TRAIN_STATS_BWD + 16 * (stage - _lib.STAGE_BWD_BN)
+            return self._xstats[o:o + 16]
+        if stage == _lib.STAGE_GRADS:
+            return self._xgrads
+        raise Exception("unknown reduce stage {}".format(stage))
+
+    def _on_reduce(self, ctx, stage, stream):
+        """The C hook of a sharded fit, called on the thread (and current stream) of ``fit``.  An exception must not
+        unwind through C: it is kept for ``fit`` to raise and the fit is aborted with a non-zero return."""
+        try:
+            self.reducer.all_reduce(self._exchange_slice(int(stage)))
+            return 0
+        except BaseException as e:                       # noqa: B902 -- KeyboardInterrupt included: C cannot unwind it
+            self._reduce_error = e
+            return 1
+
+    def _all_ranks(self, flag):
+        """True when ``flag`` holds on every rank (an all-reduce MIN; one host synchronisation)."""
+        t = torch.tensor([1 if flag else 0], dtype=torch.int32, device=self.device)
+        self.reducer.all_reduce(t, op="min")
+        return bool(int(t.item()))
 
     # ------------------------------------------------------------------ weights
     def get_weights(self):
@@ -201,23 +257,38 @@ class TrainerB200:
             raise Exception("Invalid vector input : expected shape {} but got shape {}.".format((B, 8), tuple(vec.shape)))
         return B, vec
 
-    def fit(self, maps_bits, vec, target_act, target_ptr, sync_model=True, sample_weight=None):
+    def fit(self, maps_bits, vec, target_act, target_ptr, sync_model=True, sample_weight=None, batch_global=None):
         """``model.fit(x=[img, vec], y=[act, ptr], epochs=1, batch_size=B)`` (:286): one Adam step.  Returns the loss
         tensor (total, mse(output1), mse(output2)) of the batch before the update (device, float32 [3]).
         ``sample_weight``: float [B] of weights >= 0 -- ``model.fit(..., sample_weight=w)``: each head's loss becomes
-        (1/B) sum_b w_b mse_b, and the returned losses are the weighted ones (include/ofb_train.h)."""
+        (1/B) sum_b w_b mse_b, and the returned losses are the weighted ones (include/ofb_train.h).
+        With a ``reducer`` the step is on the union of every rank's batch, whose size an all-reduce of the local B gives
+        (``batch_global`` overrides it), and the losses are the global batch's."""
         B, vec = self._check_batch(maps_bits, vec)
         target_act = target_act.to(device=self.device, dtype=torch.float32).contiguous()
         target_ptr = target_ptr.to(device=self.device, dtype=torch.float32).contiguous()
         if tuple(target_act.shape) != (B, 2) or target_ptr.numel() != B * 160000:
             raise Exception("Invalid targets : expected shapes {} and {}.".format((B, 2), (B, 400, 400, 1)))
-        if sample_weight is None:
-            _lib.check(self._lib.ofb_trainer_fit(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr), B,
-                                                 _ptr(self._loss), self._stream()))
-        else:
+        if sample_weight is not None:
             sample_weight = torch.as_tensor(sample_weight).to(device=self.device, dtype=torch.float32).contiguous()
             if tuple(sample_weight.shape) != (B,):
                 raise Exception("Invalid sample_weight : expected shape {} but got shape {}.".format((B,), tuple(sample_weight.shape)))
+        if self.reducer is not None or batch_global is not None:
+            if batch_global is None:                      # ranks cannot disagree on the global batch: it is their sum
+                n = torch.tensor([B], dtype=torch.int32, device=self.device)
+                self.reducer.all_reduce(n)
+                batch_global = int(n.item())
+            self._reduce_error = None
+            rc = self._lib.ofb_trainer_fit_shard(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr),
+                                                 _ptr(sample_weight), B, int(batch_global), _ptr(self._loss), self._stream())
+            if rc < 0 and self._reduce_error is not None:
+                err, self._reduce_error = self._reduce_error, None
+                raise _lib.OfbError("libofb error %d: %s" % (rc, self._lib.ofb_last_error().decode())) from err
+            _lib.check(rc)
+        elif sample_weight is None:
+            _lib.check(self._lib.ofb_trainer_fit(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr), B,
+                                                 _ptr(self._loss), self._stream()))
+        else:
             _lib.check(self._lib.ofb_trainer_fit_weighted(self._h, _ptr(maps_bits), _ptr(vec), _ptr(target_act), _ptr(target_ptr),
                                                           _ptr(sample_weight), B, _ptr(self._loss), self._stream()))
         self.launch_count += self.KERNELS_PER_FIT
@@ -337,7 +408,10 @@ class TrainerB200:
         (``memory.n_step`` > 1, whose ``gamma`` must be the trainer's) the targets are R + gamma^k max Q(s_{t+k}) of each
         sample's window (``ofb_trainer_td_targets_discounted``).  With a target network (``target_update``) the max-bootstrap
         reads the target's predictions on the next observations; with ``double_dqn`` the online network selects and the
-        target evaluates (``ofb_trainer_td_targets_double``, which on the prioritized path also gives the TD errors)."""
+        target evaluates (``ofb_trainer_td_targets_double``, which on the prioritized path also gives the TD errors).
+        With a ``reducer`` see ``_replay_shard``: a collective call that returns None when some rank had nothing to draw."""
+        if self.reducer is not None:
+            return self._replay_shard(batch_size, memory, beta)
         if isinstance(memory, PrioritizedReplayMemory):
             return self._replay_prioritized(batch_size, memory, beta)
         dev = self.device
@@ -398,6 +472,69 @@ class TrainerB200:
         host = torch.cat([loss, (td_act.abs() + td_ptr.abs()).mean().reshape(1)]).cpu().tolist()
         return SimpleNamespace(history={"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]],
                                         "td_error": [host[3]]})
+
+
+    def _replay_shard(self, batch_size, memory, beta):
+        """``replay`` of a data-parallel trainer, collective over the ranks.  Each rank draws ``batch_size`` transitions
+        (fewer if its memory holds fewer) from its own ``DeviceReplayMemory``, so the global batch is the sum over the ranks
+        (the DDP convention); the targets come from the rank's replica and the fit is ``ofb_trainer_fit_shard``.
+          * Whether to replay is decided together: an all-reduce MIN of "this rank can draw"; when some rank cannot, every
+            rank skips (returns None), so all ranks make the same collective calls.
+          * Uniform draws use the rank's own ``random.Random``, seeded from (seed, rank).
+          * Prioritized draws are stratified by shard: rank r draws in proportion to its masses, P(i) = m_i / (W M_r), and
+            the importance weights are rescaled to Schaul's weights over the union of the memories, with g = the minimum
+            over ranks of m_min,r / M_r from one fp64 all-reduce MIN on the device (``ofb_replay_rescale_weights``).
+            Priorities are updated locally.
+        n-step returns, the target network and Double DQN are per-rank and need nothing more."""
+        if not isinstance(memory, DeviceReplayMemory):
+            raise Exception("Invalid memory : a data-parallel replay draws from a replay.DeviceReplayMemory on every rank.")
+        self._check_memory(memory)
+        B = int(batch_size)
+        if B < 1 or B > self.max_batch:
+            raise Exception("Invalid batch : {} samples but the trainer was sized for {}.".format(B, self.max_batch))
+        prioritized = isinstance(memory, PrioritizedReplayMemory)
+        if prioritized:
+            try:
+                mb = memory.sample_prioritized(B, beta)
+            except EmptyReplayMemory:
+                mb = None
+            have = mb is not None
+        else:
+            n = len(memory)
+            have = n > 0
+        if not self._all_ranks(have):
+            return None
+        if prioritized:
+            stats = memory.sample_stats()
+            ratio = (stats[1:2] / stats[0:1]).contiguous()
+            self.reducer.all_reduce(ratio, op="min")
+            memory.rescale_weights(mb.weight, beta, stats, ratio)
+            weight = mb.weight
+        else:
+            B = min(B, n)
+            mb = memory.sample(B, rng=self._rng)
+            weight = None
+        discount = mb.discount if memory.n_step > 1 else None
+        act_o, ptr_o = self.predict(mb.maps_obs, mb.vec_obs)
+        td_act = td_ptr = None
+        if self.double_dqn:
+            td_act, td_ptr = self._td_targets_double(act_o, ptr_o, mb.maps_next, mb.vec_next, mb.iaction, mb.pointer, mb.reward,
+                                                     mb.done, discount, B, want_td=prioritized)
+        else:
+            act_n, ptr_n = self._predict_next(mb.maps_next, mb.vec_next)
+            fields = (act_o, ptr_o, act_n, ptr_n, mb.iaction, mb.pointer, mb.reward, mb.done)
+            if prioritized:
+                td_act, td_ptr = self.td_errors(*fields, discount=discount)
+            self._td_targets(*fields, discount, B)
+        if prioritized:
+            memory.update_priorities(mb.ids, td_act, td_ptr)
+        loss = self.fit(mb.maps_next, mb.vec_next, act_o, ptr_o, sample_weight=weight)
+        parts = [loss] if not prioritized else [loss, (td_act.abs() + td_ptr.abs()).mean().reshape(1)]
+        host = torch.cat(parts).cpu().tolist()
+        hist = {"loss": [host[0]], "output1_loss": [host[1]], "output2_loss": [host[2]], "batch": [B]}
+        if prioritized:
+            hist["td_error"] = [host[3]]
+        return SimpleNamespace(history=hist)
 
 
 def len_flat():
@@ -528,7 +665,12 @@ class BatchedQLearner:
 
     With a ``replay.PrioritizedReplayMemory`` each replay is prioritized, with the importance-sampling exponent annealed
     linearly from ``beta0`` to 1 over ``beta_frames`` frames: beta = min(1, beta0 + (1 - beta0) * total_steps / beta_frames)
-    (``betas`` logs the value of every replay).  With a uniform memory ``beta0`` and ``beta_frames`` play no part."""
+    (``betas`` logs the value of every replay).  With a uniform memory ``beta0`` and ``beta_frames`` play no part.
+
+    Data-parallel (a trainer built with a ``reducer``; every rank runs its own learner on its own shard of the arenas,
+    ``sharding.make_sharded_battleground``): at a replay frame every rank calls the collective ``trainer.replay``, which
+    skips on every rank when some rank holds no transition yet, and fits one global batch of ``world * batch_size``
+    samples.  Snapshots are saved by rank 0 only."""
 
     def __init__(self, trainer, memory, replay_every=50, collecting_steps=20, snapshot=50, actor=None, snapshot_folder="networks",
                  beta0=0.4, beta_frames=100_000):
@@ -581,7 +723,14 @@ class BatchedQLearner:
         if not collecting:
             self.trainer.decay_epsilon()
         replayed = False
-        if self.total_steps % self.replay_every == 0 and self.prioritized:
+        if self.total_steps % self.replay_every == 0 and self.trainer.reducer is not None:
+            h = self.trainer.replay(self.trainer.batch_size, memory=self.memory, beta=self.beta)   # collective
+            if h is not None:
+                self.losses.append(h.history["loss"][0])
+                if self.prioritized:
+                    self.betas.append(self.beta)
+                replayed = True
+        elif self.total_steps % self.replay_every == 0 and self.prioritized:
             try:                                          # the sample reads whether there is a transition to draw
                 h = self.trainer.replay(self.trainer.batch_size, memory=self.memory, beta=self.beta)
             except EmptyReplayMemory:
@@ -594,6 +743,6 @@ class BatchedQLearner:
             h = self.trainer.replay(self.trainer.batch_size, memory=self.memory)
             self.losses.append(h.history["loss"][0])
             replayed = True
-        if self.snapshot > 0 and self.episode > 0 and self.episode % self.snapshot == 0 and self.steps < 2:
+        if self.snapshot > 0 and self.episode > 0 and self.episode % self.snapshot == 0 and self.steps < 2 and self.trainer.rank == 0:
             self.saved.append(self.trainer.save(id="iteration-%s" % self.episode, overwrite=True, folder=self.snapshot_folder))
         return iact, xy, replayed
