@@ -471,8 +471,20 @@ k_prio_draw(const uint8_t *__restrict__ valid, const float *__restrict__ mass, l
         const long long c = s_first != 0x7fffffff ? s_first : s_last;
         const long long id = replay_id(c, cP, oldest, depth);
         ids_out[b] = (int32_t)id;
-        // fp32 pow (the fp64 one spills), within a few ulp; mass >= mass_min makes w <= 1, kept so under that rounding
-        weight_out[b] = fminf(powf((float)((double)mass[id] / (double)st.mass_min), -beta), 1.0f);
+        // fp32 pow (the fp64 one spills), within a few ulp; mass >= mass_min makes w <= 1, kept so under that rounding.
+        // A ratio r past FLT_MAX (a mass clamped to FLT_MAX over a small m_min) would cast to inf and give w = 0: there
+        // r = f * 2^e with f in [1, 2), and r^-beta = f^-beta * 2^phi * 2^n with n + phi = -beta * e, n an integer.
+        // Below FLT_MAX, e = 0 and scale = 1 exactly, so w is the plain powf.  mass_min is read again here: st.mass_min,
+        // kept live across the fp64 division's slow-path calls, spills.
+        const double r = (double)mass[id] / (double)stats->mass_min;
+        const long long bits = __double_as_longlong(r);
+        const bool big = !(r <= 3.402823466e38);
+        const int e = big ? (int)(bits >> 52) - 1023 : 0;
+        const float base = big ? (float)__longlong_as_double((bits & 0x000fffffffffffffll) | 0x3ff0000000000000ll) : (float)r;
+        const double x = -(double)beta * e, n = fmax(floor(x), -250.0);   // 2^x below 2^-250 is 0 in fp32 anyway
+        const int n0 = (int)n / 2, n1 = (int)n - n0;                    // 2^n as two normal factors
+        const float scale = exp2f((float)(x - n)) * __int_as_float((127 + n0) << 23) * __int_as_float((127 + n1) << 23);
+        weight_out[b] = fminf(powf(base, -beta) * scale, 1.0f);
     }
 }
 
